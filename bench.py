@@ -25,6 +25,8 @@ translated-texture 4288x2848 uint8 frames.  One "step" = one whole ``track`` of 
               host core on a bounded sub-sample of the same workload (full N, fewer points and frames).
 * ``--impl reference`` times that CPU port with every host core (fork pool over points, the reference's
               own parallel axis) and prints the same JSON line with ``"impl": "reference"``.
+* ``--dump-outputs DIR`` writes what the last timed ``gb_track`` computed (``dump_outputs``), so that two builds can be
+              compared output for output: the inputs are seeded, the same arguments give the same inputs.
 """
 import argparse
 import datetime
@@ -183,6 +185,24 @@ class ClockSampler:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["unsampled"]}
         return {"sm_mhz": float(np.median(self.sm)), "sm_max_mhz": float(max(self.smax)), "reasons": sorted(self.reasons),
                 "samples": len(self.sm)}
+
+
+def dump_outputs(directory, result, limit=64 * 10 ** 6):
+    """Write the arrays ``Session.fetch`` returns (means, sigmas, status, status_time, obs_flags) as ``directory/<name>.npy``,
+    float64 (obs_flags: float32, exact for its uint8 values), and the point each row belongs to as ``points.npy``.  When all
+    points would take more than ``limit`` bytes, a fixed seeded sample of the points is written."""
+    arrays = {k: np.asarray(result[k], dtype=np.float32 if k == "obs_flags" else np.float64)
+              for k in ("means", "sigmas", "status", "status_time", "obs_flags")}
+    P = len(arrays["means"])
+    per_point = 8 + sum(a[0].nbytes for a in arrays.values())
+    budget = limit - 1024 * (len(arrays) + 1)  # (.npy headers)
+    points = np.arange(P)
+    if P * per_point > budget:
+        points = np.sort(np.random.default_rng(0).choice(P, budget // per_point, replace=False))
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "points.npy"), points.astype(np.float64))
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), np.ascontiguousarray(a[points]))
 
 
 def build_scene(n_points, n_frames, pinned=False):
@@ -384,6 +404,8 @@ def run_gpu_arm(args):
     if not args.per_step_events:
         kernel_ms /= (T - 1)  # gb_track = init + templates + (T - 1) updates; the updates are > 99 % of it
     status = session.buf["status"].cpu().numpy()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, session.fetch())  # (rank 0's points; the untimed tracks below reuse the buffers)
     # per-kernel durations of one more (untimed) track: CUDA events around every launch on its own stream
     import ctypes as C
     lib = _lib.load()
@@ -459,7 +481,7 @@ def run_gpu_arm(args):
         tracker.clear_device_cache()
         return tracker.track(models, tile_size=scene.tile_size)
 
-    e2e_steps = max(1, min(args.steps, 8))
+    e2e_steps = args.steps
     # (the warm-up calls keep ALL their results until the last one is done: a call needs a fresh set of pinned result buffers
     #  whenever every cached set is still referenced, and a first cudaHostAlloc of that set — 2 x 38 MB at 8 GPUs, 8 processes
     #  at once — costs ~50 ms (tools/e2e_steps.py: host_alloc 2 in exactly the slow calls).  Three sets cached here cover the
@@ -650,7 +672,12 @@ def main():
     ap.add_argument("--per-step-events", action="store_true", help="drive the updates one gb_track_step at a time with CUDA events around each")
     ap.add_argument("--points", type=int, default=0, help="override points per GPU (profiling only; not a bench value)")
     ap.add_argument("--frames", type=int, default=0, help="override frame count (profiling only; not a bench value)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the results of the GPU arm")
     select_config(args.config)
     if args.impl == "reference":
         run_reference_arm(args)

@@ -70,6 +70,93 @@ def reference_draws(seed, n_points, n_particles, n_steps_per_point, tangent=Fals
     return init, step, unif
 
 
+def lowering_scene(kind):
+    """The scene whose objects ``lowered_tables`` lowers: four points of one motion kind, three jittered frames far from the
+    origin of the world, a gridded DEM for the tangent models."""
+    import scenes
+    from glimpse_b200 import synthetic
+
+    scene = synthetic.nadir_scene(seed=5, n_points=4, n_particles=64, n_frames=3, imgsz=(320, 240), margin_px=90, kind=kind,
+                                  jitter_deg=0.05, world_offset=(4.99e5, 6.77e6))
+    if kind.startswith("tangent"):
+        scenes.add_gridded_dem(scene)
+    return scene
+
+
+def _struct_rows(structs):
+    return np.array([np.frombuffer(bytes(s), dtype=np.uint8) for s in structs])
+
+
+def lowered_tables(scene, api):
+    """The host side of the C ABI for ``scene`` built with ``api`` (this package or the reference): the gb_camera of every
+    image (one with curvature / refraction corrections), the gb_motion table, the gb_surface table with the cell values of
+    its gridded surfaces, and the index of a viewshed raster among the surfaces.  Structs are rows of their bytes."""
+    from glimpse_b200 import synthetic
+    from glimpse_b200.camera import lower_camera
+    from glimpse_b200.session import lower_models
+
+    observers, models = synthetic.build(scene, api)
+    observers[0].images[1].cam.correction = {"radius": 6.3781e6, "refraction": 0.13}
+    view = api.Raster(np.ones((6, 8)), x=(4.98e5, 5.0e5), y=(6.78e6, 6.76e6))
+    table_m, surfaces, vi = lower_models(models, view)
+    out = {"cameras": _struct_rows([lower_camera(img.cam) for obs in observers for img in obs.images]),
+           "motion": np.frombuffer(table_m.tobytes(), dtype=np.uint8), "surfaces": _struct_rows([s for s, _ in surfaces]),
+           "viewshed": np.array(vi)}
+    for i, (_, z) in enumerate(surfaces):
+        if z is not None:
+            out[f"cells{i}"] = np.asarray(z)
+    return out
+
+
+def raster_frames_scene():
+    from glimpse_b200 import synthetic
+
+    return synthetic.as_raster_frames(synthetic.nadir_scene(seed=5, n_points=4, n_particles=64, n_frames=3, imgsz=(320, 240),
+                                                            margin_px=90, world_offset=(4.99e5, 6.77e6)))
+
+
+def raster_frame_results(scene, api):
+    """An Observer of orthoimages built with ``api``: every frame's affine gb_camera (a row of its bytes) and its answers to
+    xyz_to_uv / uv_to_xyz / inbounds at seven fixed points, d, size and read of a fixed box, stacked over the frames."""
+    from glimpse_b200 import synthetic
+    from glimpse_b200.session import lower_grid_camera
+
+    xyz = np.column_stack((4.99e5 + np.linspace(-40, 40, 7), 6.77e6 + np.linspace(-30, 30, 7), np.zeros(7)))
+    out = {k: [] for k in ("camera", "xyz_to_uv", "uv_to_xyz", "inbounds", "d", "size", "read")}
+    for img in synthetic.build(scene, api)[0][0].images:
+        uv = img.xyz_to_uv(xyz)
+        for key, value in (("camera", np.frombuffer(bytes(lower_grid_camera(img)), dtype=np.uint8)), ("xyz_to_uv", uv),
+                           ("uv_to_xyz", img.uv_to_xyz(uv)), ("inbounds", img.inbounds(uv - 150)), ("d", img.d),
+                           ("size", img.size), ("read", img.read(box=(3, 4, 30, 20)))):
+            out[key].append(np.asarray(value))
+    return {k: np.stack(v) for k, v in out.items()}
+
+
+def assert_tables_close(got, want):
+    """``lowered_tables`` / ``raster_frame_results`` against stored ones: the same arrays, integers and struct fields of
+    integer type equal, floating-point values equal to 1e-12 (relative, or absolute near zero): the stored values come
+    from another host, whose libm may round the sines and cosines of a rotation differently in the last bit."""
+    from glimpse_b200 import _lib
+    from glimpse_b200.session import MOTION_DTYPE
+
+    structs = {"cameras": np.dtype(_lib.gb_camera), "camera": np.dtype(_lib.gb_camera), "surfaces": np.dtype(_lib.gb_surface),
+               "motion": MOTION_DTYPE}
+    assert sorted(got) == sorted(want), (sorted(got), sorted(want))
+    for key, value in got.items():
+        ref = np.asarray(want[key])
+        assert value.shape == ref.shape, key
+        if key in structs:
+            value, ref = value.reshape(-1).view(structs[key]), ref.reshape(-1).view(structs[key])
+            fields = [(f"{key}.{name}", value[name], ref[name]) for name in structs[key].names]
+        else:
+            fields = [(key, value, ref)]
+        for name, a, b in fields:
+            if np.issubdtype(a.dtype, np.floating):
+                np.testing.assert_allclose(a, b, rtol=1e-12, atol=1e-12, err_msg=name)
+            else:
+                np.testing.assert_array_equal(a, b, err_msg=name)
+
+
 def shape_scene(name):
     import scenes
     from glimpse_b200 import synthetic

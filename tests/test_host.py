@@ -440,67 +440,57 @@ def test_observer_subset_split_and_select_datetimes():
         obs.sample_tile(np.zeros((1, 2)), np.zeros((5, 5)), (0, 0, 5, 5), kx=6)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src"), reason="needs the reference checkout (build container only)")
+def _reference_results(lower, scene):
+    """``lower(scene, api)`` with the unmodified reference (``oracle/ref_shim.py``), or None where it cannot be imported."""
+    from oracle import ref_shim
+
+    return lower(scene, ref_shim.import_reference()) if ref_shim.available() else None
+
+
 @pytest.mark.parametrize("kind", ["cartesian", "cylindrical", "tangent_cartesian", "tangent_cylindrical"])
 def test_reference_objects_lower_to_the_same_tables(kind):
     """INTEGRATION.md §1: the reference's own Observer / Image / Camera / motion-model / Raster objects are accepted as they
-    are.  Built from one scene with both packages, they must lower to byte-identical gb_camera / gb_motion / gb_surface tables
-    (host side of the C ABI), including gridded DEMs, a viewshed raster and cameras with curvature / refraction corrections."""
-    import scenes
-    from glimpse_b200 import synthetic
-    from glimpse_b200.camera import lower_camera
-    from glimpse_b200.session import lower_models
-    from oracle.ref_shim import import_reference
+    are.  Built from one scene, this package's objects lower to the gb_camera / gb_motion / gb_surface tables (host side of
+    the C ABI) stored in tests/golden/lowering.npz, including gridded DEMs, a viewshed raster and cameras with curvature /
+    refraction corrections; where the reference can be imported, its objects must lower to byte-identical tables."""
+    import helpers
 
     import glimpse_b200 as gb
 
-    glimpse = import_reference()
-    scene = synthetic.nadir_scene(seed=5, n_points=4, n_particles=64, n_frames=3, imgsz=(320, 240), margin_px=90, kind=kind,
-                                  jitter_deg=0.05, world_offset=(4.99e5, 6.77e6))
-    if kind.startswith("tangent"):
-        scenes.add_gridded_dem(scene)
-    tables = []
-    for api in (glimpse, gb):
-        observers, models = synthetic.build(scene, api)
-        observers[0].images[1].cam.correction = {"radius": 6.3781e6, "refraction": 0.13}
-        cams = [bytes(lower_camera(img.cam)) for obs in observers for img in obs.images]
-        view = api.Raster(np.ones((6, 8)), x=(4.98e5, 5.0e5), y=(6.78e6, 6.76e6))
-        table_m, surfaces, vi = lower_models(models, view)
-        surf = [(bytes(s), None if z is None else z.tobytes()) for s, z in surfaces]
-        tables.append((cams, table_m.tobytes(), surf, vi))
-    assert tables[0][0] == tables[1][0]  # gb_camera of every image
-    assert tables[0][1] == tables[1][1]  # gb_motion of every point
-    assert tables[0][2] == tables[1][2] and tables[0][3] == tables[1][3]  # gb_surface table (structs and cell values), viewshed index
-    assert len(tables[0][2]) >= (3 if kind.startswith("tangent") else 2)
+    scene = helpers.lowering_scene(kind)
+    mine = helpers.lowered_tables(scene, gb)
+    golden = helpers.load_golden("lowering")
+    helpers.assert_tables_close(mine, {k.split(".", 1)[1]: golden[k] for k in golden.files if k.split(".", 1)[0] == kind})
+    assert len(mine["surfaces"]) >= (3 if kind.startswith("tangent") else 2)
+    theirs = _reference_results(helpers.lowered_tables, scene)
+    if theirs is not None:
+        assert sorted(theirs) == sorted(mine)
+        for key in mine:
+            np.testing.assert_array_equal(theirs[key], mine[key], err_msg=key)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src"), reason="needs the reference checkout (build container only)")
 def test_reference_raster_frames_lower_to_the_same_affine_camera():
-    """An Observer of orthoimages: the reference's Raster frames and this package's lower to the same affine gb_camera, and
-    both packages' Raster agree on xyz_to_uv / uv_to_xyz / inbounds / read / d / size (raster.py:119-122, 339-341, 423-459, 763-836)."""
-    import scenes
+    """An Observer of orthoimages: this package's Raster frames lower to the affine gb_camera and answer xyz_to_uv /
+    uv_to_xyz / inbounds / read / d / size (raster.py:119-122, 339-341, 423-459, 763-836) as stored in
+    tests/golden/lowering.npz; where the reference can be imported, its Raster frames must give exactly the same."""
+    import helpers
     from glimpse_b200 import synthetic
     from glimpse_b200.session import lower_grid_camera
-    from oracle.ref_shim import import_reference
 
     import glimpse_b200 as gb
 
-    glimpse = import_reference()
-    scene = synthetic.as_raster_frames(synthetic.nadir_scene(seed=5, n_points=4, n_particles=64, n_frames=3, imgsz=(320, 240), margin_px=90,
-                                                             world_offset=(4.99e5, 6.77e6)))
-    built = [synthetic.build(scene, api)[0][0] for api in (glimpse, gb)]
-    for a, b in zip(built[0].images, built[1].images):
-        ca, cb = lower_grid_camera(a), lower_grid_camera(b)
-        assert bytes(ca) == bytes(cb) and cb.affine == 1 and tuple(cb.imgsz) == (320, 240)
+    scene = helpers.raster_frames_scene()
+    mine = helpers.raster_frame_results(scene, gb)
+    golden = helpers.load_golden("lowering")
+    helpers.assert_tables_close(mine, {k.split(".", 1)[1]: golden[k] for k in golden.files if k.split(".", 1)[0] == "raster"})
+    theirs = _reference_results(helpers.raster_frame_results, scene)
+    if theirs is not None:
+        for key in mine:
+            np.testing.assert_array_equal(theirs[key], mine[key], err_msg=key)
+    for b in synthetic.build(scene, gb)[0][0].images:
+        cb = lower_grid_camera(b)
+        assert cb.affine == 1 and tuple(cb.imgsz) == (320, 240)
         assert cb.f[0] > 0 > cb.f[1]  # north-up: y decreases with the row
-        xyz = np.column_stack((4.99e5 + np.linspace(-40, 40, 7), 6.77e6 + np.linspace(-30, 30, 7), np.zeros(7)))
-        np.testing.assert_array_equal(a.xyz_to_uv(xyz), b.xyz_to_uv(xyz))
-        uv = a.xyz_to_uv(xyz)
-        np.testing.assert_array_equal(a.uv_to_xyz(uv), b.uv_to_xyz(uv))
-        np.testing.assert_array_equal(a.inbounds(uv - 150), b.inbounds(uv - 150))
-        np.testing.assert_array_equal(a.d, b.d)
-        np.testing.assert_array_equal(a.size, b.size)
-        np.testing.assert_array_equal(a.read(box=(3, 4, 30, 20)), b.read(box=(3, 4, 30, 20)))
         assert b.read().dtype == np.uint8
         with pytest.raises(ValueError):
             b.read(box=(-1, 0, 5, 5))
