@@ -25,6 +25,7 @@ GB_OBS_OUT_OF_FRAME = 2
 GB_ST_WINDOW_TOO_LARGE = 6
 GB_WINDOW_MARGIN, GB_WINDOW_MARGIN_MAX = 191, 1000  # default / retry capacity of the search windows beyond the template, px
 GB_RNG_SUPPLIED, GB_RNG_PHILOX = 0, 1
+GB_DRAW_WORDS, GB_DRAW_NORMALS, GB_DRAW_UNIFORM, GB_DRAW_UNIFORM_PARTICLE = 0, 1, 2, 3  # what gb_philox_draws writes
 GB_RESAMPLE = {"systematic": 0, "stratified": 1, "choice": 2, "residual": 3}
 GB_MODE_STREAM = 1
 GB_PIX = {"uint8": 0, "uint16": 1, "float32": 2, "float64": 3}
@@ -139,6 +140,8 @@ SIGNATURES = {
     "gb_init_particles": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "gb_motion_log_likelihoods": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "gb_moments": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "gb_philox_draws": (C.c_int, [C.c_uint64, C.c_uint64, C.c_uint32, C.c_uint32, C.c_int64, C.c_int32, C.c_int32, C.c_void_p,
+                                  C.c_void_p]),
 }
 
 _lib = None

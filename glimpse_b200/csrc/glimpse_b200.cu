@@ -405,6 +405,30 @@ __global__ void __launch_bounds__(GB_THREADS) k_moments(const double* __restrict
   }
 }
 
+// The device draws of gb_track's philox mode, read back through the very functions the step kernels call (stand-alone
+// entry point gb_philox_draws; element i is particle first + i, or time `time + i` for the systematic uniform).
+__global__ void k_philox_draws(uint64_t seed, uint64_t point, uint32_t time, uint32_t first, int64_t n, int kind, uint32_t rng_stream,
+                               void* out) {
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    const uint32_t particle = first + (uint32_t)i;
+    if (kind == GB_DRAW_WORDS) {
+      uint32_t r[4];
+      Philox{(uint32_t)seed, (uint32_t)(seed >> 32)}.generate(particle, time, (uint32_t)point,
+                                                             ((uint32_t)(point >> 32) << 8) | rng_stream, r);
+      uint32_t* dst = static_cast<uint32_t*>(out) + 4 * i;
+#pragma unroll
+      for (int c = 0; c < 4; ++c) dst[c] = r[c];
+    } else if (kind == GB_DRAW_NORMALS) {
+      double* dst = static_cast<double*>(out) + 3 * i;
+      philox_normals3(seed, point, time, particle, rng_stream, dst[0], dst[1], dst[2]);
+    } else if (kind == GB_DRAW_UNIFORM) {
+      static_cast<double*>(out)[i] = philox_uniform(seed, point, time + (uint32_t)i);
+    } else {
+      static_cast<double*>(out)[i] = philox_uniform_particle(seed, point, time, particle);
+    }
+  }
+}
+
 // ---------------------------------------------------------------------------------------------
 // First frame: initialize_particles + test_particles + unit weights + moments
 // (motion.py:149-163, 260-283; tracker.py:327-330, 350-357).  One CTA per point.
@@ -1944,6 +1968,17 @@ int gb_moments(const double* particles, const double* weights, int64_t n, double
                void* stream) {
   if (!particles || !weights || !mean || n <= 0) return fail(GB_E_INVALID, "bad arguments%s");
   k_moments<<<1, GB_THREADS, kHeaderBytes, (cudaStream_t)stream>>>(particles, weights, n, mean, sigma, cov);
+  GB_CUDA(cudaGetLastError());
+  return GB_OK;
+}
+
+int gb_philox_draws(uint64_t seed, uint64_t point, uint32_t time, uint32_t first_particle, int64_t n, int32_t kind, int32_t rng_stream,
+                    void* out, void* stream) {
+  if (!out || n <= 0 || n > ((int64_t)1 << 32) || kind < GB_DRAW_WORDS || kind > GB_DRAW_UNIFORM_PARTICLE || rng_stream < 0 ||
+      rng_stream > 255)
+    return fail(GB_E_INVALID, "bad arguments%s");
+  k_philox_draws<<<grid_for(n, 256), 256, 0, (cudaStream_t)stream>>>(seed, point, time, first_particle, n, kind, (uint32_t)rng_stream,
+                                                                     out);
   GB_CUDA(cudaGetLastError());
   return GB_OK;
 }

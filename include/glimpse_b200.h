@@ -62,6 +62,12 @@ extern "C" {
 #define GB_RNG_SUPPLIED 0 /* normals / uniforms provided in the reference's draw order */
 #define GB_RNG_PHILOX 1   /* counter-based Philox4x32-10 on device */
 
+/* What gb_philox_draws writes */
+#define GB_DRAW_WORDS 0              /* uint32 [n][4]: the four Philox4x32-10 output words */
+#define GB_DRAW_NORMALS 1            /* double [n][3]: the three float32 Box-Muller normals of those words */
+#define GB_DRAW_UNIFORM 2            /* double [n]: the systematic resampler's uniform (stream 3) */
+#define GB_DRAW_UNIFORM_PARTICLE 3   /* double [n]: the per-particle uniform of the other resamplers (stream 4) */
+
 /* Camera of one image, already lowered from the reference's 20-vector
  * [xyz, viewdir, imgsz, f, c, k1..k6, p1, p2] (camera.py:101,127-198): R is `Camera.R`
  * (camera.py:239-280), cc = imgsz / 2 + c (camera.py:1507).  corr_* implement
@@ -406,6 +412,14 @@ int gb_sample_surface(const double* tile, int32_t rows, int32_t cols, int32_t kx
  * row-major particles[n][6], weights[n]: mean[6], sigma[6] (or NULL), cov[36] (or NULL). */
 int gb_moments(const double* particles, const double* weights, int64_t n, double* mean, double* sigma, double* cov,
                void* stream);
+/* The draws of rng_mode = GB_RNG_PHILOX as a stand-alone call, computed by the device functions the track kernels call.
+ * Philox4x32-10 with key (seed & 0xffffffff, seed >> 32) and counter (particle, time, point & 0xffffffff,
+ * (point >> 32) << 8 | rng_stream); streams: 0 and 1 = the six normals of initialisation, 2 = the normals of every later step,
+ * 3 = the systematic resampler's uniform (particle word 0xffffffff), 4 = the per-particle uniform of the stratified, choice and
+ * residual resamplers.  Element i of `out` (device memory) is particle first_particle + i (GB_DRAW_WORDS, GB_DRAW_NORMALS with
+ * `rng_stream`, GB_DRAW_UNIFORM_PARTICLE) or time `time` + i (GB_DRAW_UNIFORM); 1 <= n <= 2^32. */
+int gb_philox_draws(uint64_t seed, uint64_t point, uint32_t time, uint32_t first_particle, int64_t n, int32_t kind, int32_t rng_stream,
+                    void* out, void* stream);
 
 #ifdef __cplusplus
 }

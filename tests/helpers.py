@@ -157,11 +157,12 @@ def assert_tables_close(got, want):
                 np.testing.assert_array_equal(a, b, err_msg=name)
 
 
-def shape_scene(name):
+def case_scene(name):
+    """(scene, case) of a case of ``scenes.track_cases()`` or ``scenes.shape_cases()``."""
     import scenes
     from glimpse_b200 import synthetic
 
-    case = scenes.shape_cases()[name]
+    case = {**scenes.track_cases(), **scenes.shape_cases()}[name]
     scene = synthetic.nadir_scene(**case["scene_kwargs"])
     if case.get("post"):
         scene = case["post"](scene)
@@ -180,7 +181,7 @@ def shape_golden(name):
 
     if name in _SHAPE_CACHE:
         return _SHAPE_CACHE[name]
-    scene, case = shape_scene(name)
+    scene, case = case_scene(name)
     small = load_golden(name)
     crc = np.array([int(np.asarray(f, dtype=np.int64).sum()) for o in scene.observers for f in o.frames])
     np.testing.assert_array_equal(crc, small["frame_crc"])
