@@ -30,6 +30,8 @@ GB_RESAMPLE = {"systematic": 0, "stratified": 1, "choice": 2, "residual": 3}
 GB_MODE_STREAM = 1
 GB_PIX = {"uint8": 0, "uint16": 1, "float32": 2, "float64": 3}
 GB_PLAN_RANKED_FRAMES = 1
+GB_PLAN_LARGE_TEMPLATES = 2  # templates above 1024 pixels, up to 128 a side
+GB_MAX_TEMPLATE, GB_MAX_TEMPLATE_SIDE = 1024, 128  # template pixels without that flag / largest side with it
 GB_HP_MODES = {"reflect": 0, "grid-mirror": 0, "constant": 1, "grid-constant": 1, "nearest": 2, "mirror": 3, "wrap": 4, "grid-wrap": 4}
 GB_MOTION_CARTESIAN, GB_MOTION_CYLINDRICAL, GB_MOTION_TANGENT_CARTESIAN, GB_MOTION_TANGENT_CYLINDRICAL = 0, 1, 2, 3
 

@@ -9,6 +9,10 @@
 #define GB_MAX_OBS 8
 #define GB_XCH 36 /* doubles per slot of a block reduction (28 moment sums at most) */
 #define GB_MAX_BINS 1024
+// Templates up to this many pixels keep their high-passed copy and CDF tables in shared memory next to the search window;
+// larger ones (GB_PLAN_LARGE_TEMPLATES, up to GB_MAX_TEMPLATE_SIDE a side) are read from global memory.
+#define GB_SMEM_TEMPLATE 1024
+#define GB_MAX_TEMPLATE_SIDE 128
 
 // particle flag bits, in the order the reference would raise (tracker.py:106-119, observer.py:201,
 // raster.py:961-973)

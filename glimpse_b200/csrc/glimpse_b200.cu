@@ -21,7 +21,7 @@
 #include "tile.cuh"
 
 #define GB_THREADS 512
-#define GB_MAX_TEMPLATE 1024 /* template pixels handled by k_template */
+#define GB_MAX_TEMPLATE 1024 /* template pixels a plan admits without GB_PLAN_LARGE_TEMPLATES */
 #define GB_MAX_HIGHPASS 31   /* rows / columns of the median high-pass */
 
 namespace gb {
@@ -112,6 +112,7 @@ struct StepParams {
   int tmpl_from_ev;  // k_template: staggered templates read the evolved particles from s_ev (pipelined flow)
   int resample_method;  // GB_RESAMPLE_*
   int s2_budget;        // shared-memory bytes k_s2_surface may use for one window (negative: planar path forced, tests)
+  int s2_smem;          // dynamic shared memory k_s2_surface is launched with (s2_smem_bytes)
   int64_t p0, pb;    // batch of points handled by this launch
   int interp_rows, interp_cols;  // spline degree along the rows (kx) / columns (ky) of the SSE surface: 3 or 1 (Tracker.interpolation)
 };
@@ -509,18 +510,45 @@ __global__ void __launch_bounds__(GB_THREADS) k_init(const __grid_constant__ Ste
 
 // ---------------------------------------------------------------------------------------------
 // Template construction (tracker.py:536-561, 494-534): one CTA per (point, observer) due at t.
+// LARGE: templates above GB_SMEM_TEMPLATE pixels (GB_PLAN_LARGE_TEMPLATES).  Their levels, histogram and representatives
+// live in dynamic shared memory (template_smem_bytes), the grey values of ranked frames in the (point, observer)'s surface
+// region, which no kernel uses while templates are cut.  Otherwise the two variants run the same code.
 // ---------------------------------------------------------------------------------------------
+// histogram bins: one per rank of a ranked template, one per band sum of a uint8 frame of up to 8 bands
+__host__ __device__ inline int template_bins(int area) { return area > 255 * 8 + 1 ? area : 255 * 8 + 1; }
+__host__ __device__ inline int template_smem_bytes(int area) {
+  return (int)(align16((int64_t)template_bins(area) * 4) + 2 * align16((int64_t)area * 2));
+}
+
+template <bool LARGE>
 __global__ void __launch_bounds__(256) k_template(const __grid_constant__ StepParams prm) {
   __shared__ double s_red[8][8];
   __shared__ int s_box[4];
   __shared__ int s_ok;
   __shared__ double s_stats[2];
-  __shared__ uint16_t s_raw[GB_MAX_TEMPLATE];
-  __shared__ uint32_t s_hist[GB_MAX_BINS];
-  __shared__ double s_vals[GB_MAX_TEMPLATE];  // frames other than uint8: the tile's grey values ...
-  __shared__ uint16_t s_rep[GB_MAX_TEMPLATE]; // ... and one pixel of every level
   const int64_t p = blockIdx.x / prm.O;
   const int o = (int)(blockIdx.x - p * prm.O);
+  uint16_t* s_raw;   // grey level of every pixel
+  uint32_t* s_hist;  // pixels per level
+  double* s_vals;    // frames other than uint8: the tile's grey values ...
+  uint16_t* s_rep;   // ... and one pixel of every level
+  if constexpr (LARGE) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int a = prm.tile_w * prm.tile_h;
+    s_hist = reinterpret_cast<uint32_t*>(smem_raw);
+    s_raw = reinterpret_cast<uint16_t*>(smem_raw + align16((int64_t)template_bins(a) * 4));
+    s_rep = reinterpret_cast<uint16_t*>(smem_raw + align16((int64_t)template_bins(a) * 4) + align16((int64_t)a * 2));
+    s_vals = reinterpret_cast<double*>(prm.s_surf + (p * prm.O + o) * prm.surf_bytes);
+  } else {
+    __shared__ uint16_t a_raw[GB_SMEM_TEMPLATE];
+    __shared__ uint32_t a_hist[GB_MAX_BINS];
+    __shared__ double a_vals[GB_SMEM_TEMPLATE];
+    __shared__ uint16_t a_rep[GB_SMEM_TEMPLATE];
+    s_raw = a_raw;
+    s_hist = a_hist;
+    s_vals = a_vals;
+    s_rep = a_rep;
+  }
   const int t = prm.t;
   if (prm.status[p] != 0 || prm.tmpl_frame[o] != t || !prm.mask[p * prm.O + o] || prm.img[o] < 0) return;
   if (t < prm.first[p] || t > prm.last[p]) return;
@@ -961,8 +989,12 @@ static void fill_params(const gb_track_desc& d, int t, StepParams& prm) {
 static int check_desc(const gb_track_desc& d) {
   if (d.P <= 0 || d.N <= 0 || d.T < 2) return fail(GB_E_INVALID, "P, N must be positive and T >= 2%s");
   if (d.O < 1 || d.O > GB_MAX_OBS) return fail(GB_E_INVALID, "between 1 and 8 observers are supported%s");
-  if (d.tile_w < 1 || d.tile_h < 1 || (int64_t)d.tile_w * d.tile_h > GB_MAX_TEMPLATE)
-    return fail(GB_E_RESOURCE, "template larger than 1024 pixels%s");
+  if (d.tile_w < 1 || d.tile_h < 1 || (int64_t)d.tile_w * d.tile_h > GB_MAX_TEMPLATE) {
+    if (d.tile_w < 1 || d.tile_h < 1 || (int64_t)d.tile_w * d.tile_h > d.plan.max_template)
+      return fail(GB_E_RESOURCE, "template larger than 1024 pixels (or than the plan's max_template)%s");
+    if (d.tile_w > GB_MAX_TEMPLATE_SIDE || d.tile_h > GB_MAX_TEMPLATE_SIDE)
+      return fail(GB_E_RESOURCE, "template above 1024 pixels and wider or taller than 128 pixels%s");
+  }
   if (d.highpass_size != 0 && ((d.highpass_size & 0xffff) < 1 || (d.highpass_size & 0xffff) > GB_MAX_HIGHPASS ||
                                (d.highpass_size >> 16 & 0xffff) < 1 || (d.highpass_size >> 16 & 0xffff) > GB_MAX_HIGHPASS))
     return fail(GB_E_INVALID, "highpass_size: rows and columns must be between 1 and 31%s");
@@ -1005,6 +1037,14 @@ static int check_desc(const gb_track_desc& d) {
 #define GB_S2_SMEM_KB 110
 #endif
 static constexpr int kSurfaceSmem = GB_S2_SMEM_KB * 1024;
+// ... and for large templates whose usual windows (the template plus 10-40 px) would not fit that: one CTA an SM with
+// 224 KB, where a 128 x 128 template's windows up to ~165 px stay interleaved in shared memory and up to ~210 px staged
+static constexpr int kSurfaceSmemLarge = 224 * 1024;
+
+static int s2_smem_bytes(int tw, int th) {
+  if ((int64_t)tw * th <= GB_SMEM_TEMPLATE) return kSurfaceSmem;
+  return tile_bytes_needed(tw + 40, th + 40, tw, th, GB_MAX_BINS, 0) <= kSurfaceSmem ? kSurfaceSmem : kSurfaceSmemLarge;
+}
 
 struct StreamLayout {
   int64_t ev[2], uv, w, bsum, pre, pm, ibox, pflags[2], act, meta, ref, surf, total;
@@ -1062,7 +1102,8 @@ static void stream_bind(const gb_track_desc& d, StepParams& prm, int par, int64_
   prm.s_nblk = pl.stream_nblk;
   {
     const int mag = pl.tile_bytes < 0 ? -pl.tile_bytes : pl.tile_bytes;
-    prm.s2_budget = (pl.tile_bytes < 0 ? -1 : 1) * (mag < kSurfaceSmem ? mag : kSurfaceSmem);
+    prm.s2_smem = s2_smem_bytes(d.tile_w, d.tile_h);
+    prm.s2_budget = (pl.tile_bytes < 0 ? -1 : 1) * (mag < prm.s2_smem ? mag : prm.s2_smem);
   }
   prm.p0 = p0;
   prm.pb = pb;
@@ -1104,7 +1145,10 @@ static int launch_stream_batch(const StepParams& prm, cudaStream_t stream) {
   k_s1_propagate<<<nb, GB_SBLOCK_THREADS, 0, stream>>>(prm);
   FrameMaps fm;
   frame_maps(prm, fm);
-  k_s2_surface<<<(unsigned)(prm.pb * prm.O), GB_S2_THREADS, kSurfaceSmem, stream>>>(prm, fm, prm.s2_budget);
+  if (prm.tile_w * prm.tile_h > GB_SMEM_TEMPLATE)
+    k_s2_surface<true><<<(unsigned)(prm.pb * prm.O), GB_S2_THREADS, prm.s2_smem, stream>>>(prm, fm, prm.s2_budget);
+  else
+    k_s2_surface<false><<<(unsigned)(prm.pb * prm.O), GB_S2_THREADS, prm.s2_smem, stream>>>(prm, fm, prm.s2_budget);
   if (spline_is_hermite(prm.interp_cols, prm.interp_rows))
     k_s3_weights<false><<<dim3((unsigned)prm.s_nblk, (unsigned)prm.pb), s3_threads(prm.s_block), 0, stream>>>(prm);
   else
@@ -1133,7 +1177,8 @@ static int launch_stream_update(const gb_track_desc& d, StepParams& prm, cudaStr
   GB_CUDA(cudaGetDevice(&dev));
   cudaError_t aerr = cudaSuccess;
   std::call_once(attr_once[dev & 15], [&]() {
-    aerr = cudaFuncSetAttribute(k_s2_surface, cudaFuncAttributeMaxDynamicSharedMemorySize, kSurfaceSmem);
+    aerr = cudaFuncSetAttribute(k_s2_surface<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSurfaceSmem);
+    if (aerr == cudaSuccess) aerr = cudaFuncSetAttribute(k_s2_surface<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSurfaceSmemLarge);
   });
   if (aerr != cudaSuccess) return fail(GB_E_CUDA, "k_s2_surface attributes: %s", cudaGetErrorString(aerr));
   const bool cov = d.covariances != nullptr;
@@ -1172,7 +1217,7 @@ static int launch_stream_update(const gb_track_desc& d, StepParams& prm, cudaStr
 }
 
 static int launch_init(const StepParams& prm, bool cov, cudaStream_t stream);
-static int launch_template(const StepParams& prm, cudaStream_t stream);
+static int launch_template(const gb_track_desc& d, StepParams prm, cudaStream_t stream);
 
 // Optional per-kernel timing of the pipelined flow (gb_kernel_timing): every launch is bracketed by CUDA events
 // on the stream it is launched on; durations are accumulated per kernel kind when the track has finished.
@@ -1226,7 +1271,8 @@ static int track_streaming(const gb_track_desc& d, cudaStream_t stream, int64_t*
   GB_CUDA(cudaGetDevice(&dev));
   cudaError_t aerr = cudaSuccess;
   std::call_once(attr_once[dev & 15], [&]() {
-    aerr = cudaFuncSetAttribute(k_s2_surface, cudaFuncAttributeMaxDynamicSharedMemorySize, kSurfaceSmem);
+    aerr = cudaFuncSetAttribute(k_s2_surface<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSurfaceSmem);
+    if (aerr == cudaSuccess) aerr = cudaFuncSetAttribute(k_s2_surface<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSurfaceSmemLarge);
     if (aerr == cudaSuccess) aerr = cudaFuncSetAttribute(k_s4p_resample_propagate<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kS4pSmem);
     if (aerr == cudaSuccess) aerr = cudaFuncSetAttribute(k_s4p_resample_propagate<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kS4pSmem);
     if (aerr == cudaSuccess) aerr = cudaFuncSetAttribute(k_s4p_resample_propagate<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kS4pSmem);
@@ -1334,7 +1380,7 @@ static int track_streaming(const gb_track_desc& d, cudaStream_t stream, int64_t*
       }
       if (has_tmpl[t]) {
         g_ktimer.begin(GB_K_TEMPLATE, stream);
-        if ((rc = launch_template(prm, stream))) return rc;
+        if ((rc = launch_template(d, prm, stream))) return rc;
         g_ktimer.end(stream);
         if (launches) ++*launches;
       }
@@ -1363,7 +1409,10 @@ static int track_streaming(const gb_track_desc& d, cudaStream_t stream, int64_t*
       }
       if (has_update[t]) {
         kt.begin(GB_K_SURFACE, ss);
-        k_s2_surface<<<(unsigned)(pb * prm.O), GB_S2_THREADS, kSurfaceSmem, ss>>>(prm, fm, prm.s2_budget);
+        if (prm.tile_w * prm.tile_h > GB_SMEM_TEMPLATE)
+          k_s2_surface<true><<<(unsigned)(pb * prm.O), GB_S2_THREADS, prm.s2_smem, ss>>>(prm, fm, prm.s2_budget);
+        else
+          k_s2_surface<false><<<(unsigned)(pb * prm.O), GB_S2_THREADS, prm.s2_smem, ss>>>(prm, fm, prm.s2_budget);
         kt.end(ss);
         kt.begin(GB_K_WEIGHTS, ss);
         if (spline_is_hermite(prm.interp_cols, prm.interp_rows))
@@ -1421,8 +1470,25 @@ static int launch_init(const StepParams& prm, bool cov, cudaStream_t stream) {
   return GB_OK;
 }
 
-static int launch_template(const StepParams& prm, cudaStream_t stream) {
-  k_template<<<(unsigned)(prm.P * prm.O), 256, 0, stream>>>(prm);
+static int launch_template(const gb_track_desc& d, StepParams prm, cudaStream_t stream) {
+  const int area = prm.tile_w * prm.tile_h;
+  if (area <= GB_SMEM_TEMPLATE) {
+    k_template<false><<<(unsigned)(prm.P * prm.O), 256, 0, stream>>>(prm);
+  } else {
+    // the work area of ranked frames: the surface regions (plan.surf_bytes >= 8 B a template pixel)
+    prm.s_surf = reinterpret_cast<char*>(d.scratch) + stream_layout(d.P, d.N, d.O, d.plan.stream_nblk, d.plan.surf_bytes).surf;
+    prm.surf_bytes = d.plan.surf_bytes;
+    const int smem = template_smem_bytes(area);
+    static std::once_flag once[16];
+    int dev = 0;
+    GB_CUDA(cudaGetDevice(&dev));
+    cudaError_t err = cudaSuccess;
+    std::call_once(once[dev & 15], [&]() {
+      err = cudaFuncSetAttribute(k_template<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, template_smem_bytes(GB_MAX_TEMPLATE_SIDE * GB_MAX_TEMPLATE_SIDE));
+    });
+    if (err != cudaSuccess) return fail(GB_E_CUDA, "k_template attributes: %s", cudaGetErrorString(err));
+    k_template<true><<<(unsigned)(prm.P * prm.O), 256, smem, stream>>>(prm);
+  }
   GB_CUDA(cudaGetLastError());
   return GB_OK;
 }
@@ -1749,8 +1815,11 @@ int gb_step_plan_ex(int64_t n_particles, int32_t tile_w, int32_t tile_h, int64_t
                     int32_t flags, int32_t mode, int32_t window_margin, gb_plan* plan) {
   if (window_margin < 4 || window_margin > GB_MAX_SURFACE - 1) return fail(GB_E_INVALID, "window_margin must be between 4 and 1023%s");
   if (!plan || n_particles <= 0 || tile_w < 1 || tile_h < 1) return fail(GB_E_INVALID, "bad plan arguments%s");
-  if ((int64_t)tile_w * tile_h > GB_MAX_TEMPLATE) return fail(GB_E_RESOURCE, "template larger than 1024 pixels%s");
-  if (flags & ~GB_PLAN_RANKED_FRAMES) return fail(GB_E_INVALID, "unknown plan flags%s");
+  if ((int64_t)tile_w * tile_h > GB_MAX_TEMPLATE && !(flags & GB_PLAN_LARGE_TEMPLATES))
+    return fail(GB_E_RESOURCE, "template larger than 1024 pixels (GB_PLAN_LARGE_TEMPLATES admits up to 128 x 128)%s");
+  if ((int64_t)tile_w * tile_h > GB_MAX_TEMPLATE && (tile_w > GB_MAX_TEMPLATE_SIDE || tile_h > GB_MAX_TEMPLATE_SIDE))
+    return fail(GB_E_RESOURCE, "template above 1024 pixels and wider or taller than 128 pixels%s");
+  if (flags & ~(GB_PLAN_RANKED_FRAMES | GB_PLAN_LARGE_TEMPLATES)) return fail(GB_E_INVALID, "unknown plan flags%s");
   if (n_observers < 1 || n_observers > GB_MAX_OBS) return fail(GB_E_INVALID, "between 1 and 8 observers are supported%s");
   if (mode != GB_MODE_STREAM) return fail(GB_E_INVALID, "unknown mode (the cluster-per-point organisation of round 1 was removed)%s");
   memset(plan, 0, sizeof(*plan));
@@ -1764,7 +1833,7 @@ int gb_step_plan_ex(int64_t n_particles, int32_t tile_w, int32_t tile_h, int64_t
     plan->cluster = 1;
     plan->n_local = (int32_t)n_particles;
     plan->particles_in_smem = 0;
-    plan->tile_bytes = kSurfaceSmem;
+    plan->tile_bytes = s2_smem_bytes(tile_w, tile_h);
     // particles of a point are cut into equal even-sized blocks that fit k_s4p's shared memory (<= 768 parents)
     plan->stream_nblk = (int32_t)((n_particles + GB_S4P_CAP - 1) / GB_S4P_CAP);
     plan->stream_block = (int32_t)(((n_particles + plan->stream_nblk - 1) / plan->stream_nblk + 1) / 2 * 2);
@@ -1779,6 +1848,11 @@ int gb_step_plan_ex(int64_t n_particles, int32_t tile_w, int32_t tile_h, int64_t
       int64_t bytes = tile_bytes_needed((int)Su, (int)Sv, tile_w, tile_h, (int)bins, tile_w * tile_h) + 16;
       bytes += bspline_band_bytes((int)(Su - tile_w + 1), (int)(Sv - tile_h + 1), 5, 5) + 16;
       if (ranked) bytes += bins * 8 + 16;
+      const int64_t ta = (int64_t)tile_w * tile_h;
+      if (ta > GB_SMEM_TEMPLATE) {
+        bytes += ta * 4 + 16;                       // the template's column-major copy behind the window's data
+        if (bytes < ta * 8) bytes = ta * 8;         // k_template's grey values of a ranked template
+      }
       plan->surf_bytes = (bytes + 255) / 256 * 256;
     }
     // Points are independent: they are cut into `slots` batches that advance on their own side streams, so the
@@ -1815,7 +1889,7 @@ int gb_track_init(const gb_track_desc* d, int32_t t, void* stream) {
   StepParams prm;
   fill_params(*d, t, prm);
   if ((rc = launch_init(prm, d->covariances != nullptr, (cudaStream_t)stream))) return rc;
-  return launch_template(prm, (cudaStream_t)stream);
+  return launch_template(*d, prm, (cudaStream_t)stream);
 }
 
 int gb_track_step(const gb_track_desc* d, int32_t t, const gb_stage_io* io, void* stream) {
@@ -1905,7 +1979,7 @@ int gb_track(const gb_track_desc* d, void* stream_, int64_t* launches_out) {
       prm.skip_evolve = 1;
     }
     if (any_tmpl) {
-      if ((rc = launch_template(prm, stream))) return rc;
+      if ((rc = launch_template(*d, prm, stream))) return rc;
       ++launches;
     }
     if (any_step) {

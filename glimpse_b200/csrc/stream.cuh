@@ -215,6 +215,9 @@ __global__ void __launch_bounds__(GB_SBLOCK_THREADS, 4) k_s1_propagate(const __g
 #ifndef GB_S2_MINB
 #define GB_S2_MINB 2
 #endif
+// LARGE: templates above GB_SMEM_TEMPLATE pixels, read from the window's global region (TileWork::tcol); launched by template
+// size, so that smaller templates run the kernel without that path.
+template <bool LARGE>
 __global__ void __launch_bounds__(GB_S2_THREADS, GB_S2_MINB) k_s2_surface(const __grid_constant__ StepParams prm, const __grid_constant__ FrameMaps fm,
                                                                  int smem_budget) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -365,6 +368,15 @@ __global__ void __launch_bounds__(GB_S2_THREADS, GB_S2_MINB) k_s2_surface(const 
     w.vals = reinterpret_cast<double*>(region + tail);
     tail += (int64_t)w.Su * w.Sv * 8;
   }
+  const int64_t ta = (int64_t)w.tw * w.th;
+  if constexpr (LARGE) {
+    // large template: its column-major copy goes behind the tile's data and its CDF tables are read where k_template left them
+    tail = align16(tail);
+    w.tcol = reinterpret_cast<float*>(region + tail);
+    tail += ta * 4;
+    w.tq = prm.tmpl_quantiles + po * ta;
+    w.tv = prm.tmpl_values + po * ta;
+  }
   if (tail > prm.surf_bytes || w.Mu > GB_MAX_SURFACE || w.Mv > GB_MAX_SURFACE || (ranked && w.Su * w.Sv > 65535)) {
     if (tid == 0) atomicOr(&prm.s_pflags[p], (int)GB_F_WINDOW);
     return;
@@ -389,7 +401,6 @@ __global__ void __launch_bounds__(GB_S2_THREADS, GB_S2_MINB) k_s2_surface(const 
     clk[9] = smid;
     clk[10] = in_smem ? 1 : planar ? 2 : staged ? 3 : 0;
   }
-  const int64_t ta = (int64_t)w.tw * w.th;
   const int boxv[4] = {box_l, box_t, box_r, box_b};
   float* dump_search = prm.io.dump_search ? prm.io.dump_search + po * prm.io.dump_cap : nullptr;
   float* dump_sse = prm.io.dump_sse ? prm.io.dump_sse + po * prm.io.dump_cap : nullptr;

@@ -33,6 +33,8 @@ struct TileWork {
   float* hp;         // [Sv][Sp] high-passed search tile, Sp = Su rounded up to 4
   uint16_t* raw;     // [Sv][Su] raw window; aliases hp (dead before hp is written)
   float2* tmpl;      // [th][tw] high-passed template, negated and duplicated (-t, -t): the packed FP32 SSD adds it to two pixels
+  float* tcol = nullptr;  // templates above GB_SMEM_TEMPLATE pixels instead: [tw][th] negated, column by column, in the window's
+                          // global region (tmpl unused; tq / tv point at the template's global tables)
   uint32_t* hist;    // [nbins]
   int Su, Sv, Mu, Mv, Mp, Sp, Tp, nbins, nvals, tw, th;
   int dtype = 0;               // GB_PIX_* of the frame: other than uint8, the window goes through `vals` and becomes ranks
@@ -50,13 +52,19 @@ struct TileWork {
 
 __host__ __device__ inline int64_t align16(int64_t b) { return (b + 15) / 16 * 16; }
 
+// Bytes of the template copy and its CDF tables next to the window: none for templates above GB_SMEM_TEMPLATE pixels, which
+// the SSD reads from global memory (a 128 x 128 template alone would take 128 KB of the window's shared memory).
+__host__ __device__ inline int64_t tile_template_bytes(int tw, int th, int nvals) {
+  if ((int64_t)tw * th > GB_SMEM_TEMPLATE) return 0;
+  return align16((int64_t)nvals * 8) * 2 + align16((int64_t)th * tw * 8);
+}
+
 __host__ __device__ inline int64_t tile_bytes_needed(int Su, int Sv, int tw, int th, int nbins, int nvals) {
   const int64_t Mu = Su - tw + 1, Mv = Sv - th + 1, Mp = Mu | 1, Sp = (Su + 3) / 4 * 4;
   const int64_t herm = Mv * Mp * 16, packed = (int64_t)(Sv + 4) * (Su + 4) * 4;
   int64_t b = align16(herm > packed ? herm : packed);
-  b += align16((int64_t)nbins * 8) + align16((int64_t)nvals * 8) * 2;
+  b += align16((int64_t)nbins * 8) + tile_template_bytes(tw, th, nvals);
   b += align16((int64_t)Sv * Sp * 4);
-  b += align16((int64_t)th * tw * 8);
   b += align16((int64_t)nbins * 4);
   return b;
 }
@@ -72,16 +80,30 @@ __device__ inline void tile_carve(char* base, TileWork& w) {
   p += align16(herm > packed ? herm : packed);
   w.lut = reinterpret_cast<double*>(p);
   p += align16((int64_t)w.nbins * 8);
-  w.tq = reinterpret_cast<double*>(p);
-  p += align16((int64_t)w.nvals * 8);
-  w.tv = reinterpret_cast<double*>(p);
-  p += align16((int64_t)w.nvals * 8);
+  if (!w.tcol) {
+    w.tq = reinterpret_cast<double*>(p);
+    p += align16((int64_t)w.nvals * 8);
+    w.tv = reinterpret_cast<double*>(p);
+    p += align16((int64_t)w.nvals * 8);
+  }
   w.hp = reinterpret_cast<float*>(p);
   w.raw = reinterpret_cast<uint16_t*>(p);
   p += align16((int64_t)w.Sv * w.Sp * 4);
-  w.tmpl = reinterpret_cast<float2*>(p);
-  p += align16((int64_t)w.th * w.tw * 8);
+  if (!w.tcol) {
+    w.tmpl = reinterpret_cast<float2*>(p);
+    p += align16((int64_t)w.th * w.tw * 8);
+  }
   w.hist = reinterpret_cast<uint32_t*>(p);
+}
+
+// Large templates: the negated high-passed template, column by column, into the window's global region (tile_prepare, all
+// threads; the SSD reads it after the CTA's next barrier).
+__device__ __forceinline__ void tile_template_global(const TileWork& w, const double* __restrict__ g_tmpl) {
+  const int ta = w.tw * w.th;
+  for (int k = threadIdx.x; k < ta; k += blockDim.x) {
+    const int c = k / w.th, r = k - c * w.th;
+    w.tcol[k] = -(float)g_tmpl[r * w.tw + c];
+  }
 }
 
 // np.interp(q, xp, fp) for one abscissa (numpy compiled_base.c arr_interp): clamped at the ends,
@@ -466,13 +488,17 @@ __device__ inline void tile_prepare(const uint8_t* __restrict__ pixels, int pitc
       w.vals[e] = pixel_gray(pixels, pitch, nchan, w.dtype, box[1] + r, box[0] + c);
     }
     for (int i = tid; i < w.nbins; i += nthr) w.hist[i] = 0u;
-    for (int i = tid; i < ta; i += nthr) {
-      const float tv = -(float)g_tmpl[i];
-      w.tmpl[i] = make_float2(tv, tv);
-    }
-    for (int i = tid; i < w.nvals; i += nthr) {
-      w.tq[i] = g_tq[i];
-      w.tv[i] = g_tv[i];
+    if (w.tcol) {
+      tile_template_global(w, g_tmpl);
+    } else {
+      for (int i = tid; i < ta; i += nthr) {
+        const float tv = -(float)g_tmpl[i];
+        w.tmpl[i] = make_float2(tv, tv);
+      }
+      for (int i = tid; i < w.nvals; i += nthr) {
+        w.tq[i] = g_tq[i];
+        w.tv[i] = g_tv[i];
+      }
     }
     __syncthreads();
     for (int e = tid; e < area; e += nthr) {
@@ -496,13 +522,17 @@ __device__ inline void tile_prepare(const uint8_t* __restrict__ pixels, int pitc
     }
     const int ta = w.tw * w.th;
     for (int i = tid; i < w.nbins; i += nthr) w.hist[i] = 0u;
-    for (int i = tid; i < ta; i += nthr) {
-      const float tv = -(float)g_tmpl[i];
-      w.tmpl[i] = make_float2(tv, tv);
-    }
-    for (int i = tid; i < w.nvals; i += nthr) {
-      w.tq[i] = g_tq[i];
-      w.tv[i] = g_tv[i];
+    if (w.tcol) {
+      tile_template_global(w, g_tmpl);
+    } else {
+      for (int i = tid; i < ta; i += nthr) {
+        const float tv = -(float)g_tmpl[i];
+        w.tmpl[i] = make_float2(tv, tv);
+      }
+      for (int i = tid; i < w.nvals; i += nthr) {
+        w.tq[i] = g_tq[i];
+        w.tv[i] = g_tv[i];
+      }
     }
     __syncthreads();
     mbar_wait(w.bar, 0);
@@ -549,13 +579,17 @@ __device__ inline void tile_prepare(const uint8_t* __restrict__ pixels, int pitc
       }
     }
     for (int i = tid; i < w.nbins; i += nthr) w.hist[i] = 0u;
-    for (int i = tid; i < ta; i += nthr) {
-      const float tv = -(float)(i == tid ? t_first : g_tmpl[i]);
-      w.tmpl[i] = make_float2(tv, tv);
-    }
-    for (int i = tid; i < w.nvals; i += nthr) {
-      w.tq[i] = i == tid ? q_first : g_tq[i];
-      w.tv[i] = i == tid ? v_first : g_tv[i];
+    if (w.tcol) {
+      tile_template_global(w, g_tmpl);
+    } else {
+      for (int i = tid; i < ta; i += nthr) {
+        const float tv = -(float)(i == tid ? t_first : g_tmpl[i]);
+        w.tmpl[i] = make_float2(tv, tv);
+      }
+      for (int i = tid; i < w.nvals; i += nthr) {
+        w.tq[i] = i == tid ? q_first : g_tq[i];
+        w.tv[i] = i == tid ? v_first : g_tv[i];
+      }
     }
   }
   __syncthreads();
@@ -685,19 +719,35 @@ __device__ __forceinline__ float2 ssd_load(const float* p) {
   return make_float2(p[0], p[1]);
 }
 
+// One column of the template as the pairs (-t, -t), row by row: from the shared copy [th][tw] of small templates, or from the
+// column-major float copy of a large one in global memory (every lane of the warp reads the same address: one broadcast
+// load, and eight consecutive rows share a 32-byte sector).
+struct TmplShared {
+  const float2* p;
+  int tw;
+  __device__ __forceinline__ float2 operator[](int ip) const { return p[ip * tw]; }
+};
+struct TmplGlobal {
+  const float* p;
+  __device__ __forceinline__ float2 operator[](int ip) const {
+    const float t = p[ip];
+    return make_float2(t, t);
+  }
+};
+
 // SSD of one lane: output rows r0 .. r0 + kmax - 1 (kmax <= 4), output columns c (even) and c + 1, template columns
 // [jlo, jhi).  Packed FP32 arithmetic (FADD2 / FFMA2, new in sm_100): the two columns share every instruction, each half
 // an ordinary IEEE operation, so the sums are bit-identical to scalar code.  The four row outputs stay in registers
 // while the template column slides past; the template is stored negated (d = pixel + (-t)).
-template <bool ALIGNED>
-__device__ __forceinline__ void ssd_column(const TileWork& w, const float* Icol, const float2* Tcol, int kmax, float2 (&a)[4]) {
-  const int th = w.th, Sp = w.Sp, tw = w.tw;
+template <bool ALIGNED, class TC>
+__device__ __forceinline__ void ssd_column(const TileWork& w, const float* Icol, const TC Tcol, int kmax, float2 (&a)[4]) {
+  const int th = w.th, Sp = w.Sp;
   const int nrow = th + kmax - 1;
   if (th >= 4) {
     // ta, tb, tc = template rows ip-1, ip-2, ip-3; output row k pairs image row ip with template row ip-k
     float2 ta, tb, tc, d;
     {
-      const float2 t_0 = Tcol[0], t_1 = Tcol[tw], t_2 = Tcol[2 * tw];
+      const float2 t_0 = Tcol[0], t_1 = Tcol[1], t_2 = Tcol[2];
       const float2 i_0 = ssd_load<ALIGNED>(Icol), i_1 = ssd_load<ALIGNED>(Icol + Sp), i_2 = ssd_load<ALIGNED>(Icol + 2 * Sp);
       d = __fadd2_rn(i_0, t_0); a[0] = __ffma2_rn(d, d, a[0]);
       d = __fadd2_rn(i_1, t_1); a[0] = __ffma2_rn(d, d, a[0]);
@@ -709,7 +759,7 @@ __device__ __forceinline__ void ssd_column(const TileWork& w, const float* Icol,
     }
 #pragma unroll 4
     for (int ip = 3; ip < th; ++ip) {
-      const float2 tn = Tcol[ip * tw];
+      const float2 tn = Tcol[ip];
       const float2 iv = ssd_load<ALIGNED>(Icol + ip * Sp);
       d = __fadd2_rn(iv, tn); a[0] = __ffma2_rn(d, d, a[0]);
       d = __fadd2_rn(iv, ta); a[1] = __ffma2_rn(d, d, a[1]);
@@ -740,7 +790,7 @@ __device__ __forceinline__ void ssd_column(const TileWork& w, const float* Icol,
       t3 = t2;
       t2 = t1;
       t1 = t0;
-      t0 = ip < th ? Tcol[ip * tw] : zero;
+      t0 = ip < th ? Tcol[ip] : zero;
       const float2 iv = ssd_load<ALIGNED>(Icol + ip * Sp);
       if (ip < th) { const float2 d = __fadd2_rn(iv, t0); a[0] = __ffma2_rn(d, d, a[0]); }
       if (ip >= 1 && ip <= th) { const float2 d = __fadd2_rn(iv, t1); a[1] = __ffma2_rn(d, d, a[1]); }
@@ -757,11 +807,42 @@ __device__ __forceinline__ void ssd_warp_item(const TileWork& w, int r0, int c, 
   acc[0] = acc[1] = acc[2] = acc[3] = zero;
   const int rc = min(r0, w.Mv - 1), cc = min(c, (w.Mu - 1) & ~1);
   const int kmax = max(1, min(4, w.Mv - rc));
+  if (w.tcol) {
+    for (int j = jlo; j < jhi; ++j) {
+      const float* Icol = w.hp + rc * w.Sp + cc + j;
+      const TmplGlobal Tcol{w.tcol + j * w.th};
+      if (j & 1) ssd_column<false>(w, Icol, Tcol, kmax, acc);
+      else ssd_column<true>(w, Icol, Tcol, kmax, acc);
+    }
+    return;
+  }
   for (int j = jlo; j < jhi; ++j) {
     const float* Icol = w.hp + rc * w.Sp + cc + j;
-    const float2* Tcol = w.tmpl + j;
+    const TmplShared Tcol{w.tmpl + j, w.tw};
     if (j & 1) ssd_column<false>(w, Icol, Tcol, kmax, acc);  // cc is even and rows start 16-byte aligned: parity of j decides
     else ssd_column<true>(w, Icol, Tcol, kmax, acc);
+  }
+}
+
+// SSD of one lane over every template column, for the organisations that give a warp item the whole template (planar, staged).
+// A large template is summed in four column slices, added in the order tile_finish_interleaved adds its slices: one running
+// float32 sum of up to 16 384 products drifts ~1.7e-5 from the exact SSD, four slices of a quarter stay within ~4e-6.
+__device__ __forceinline__ void ssd_warp_item_all(const TileWork& w, int r0, int c, float2 (&acc)[4]) {
+  if (!w.tcol) {
+    ssd_warp_item(w, r0, c, 0, w.tw, acc);
+    return;
+  }
+  const int jper = (w.tw + 3) / 4;
+  ssd_warp_item(w, r0, c, 0, jper, acc);
+#pragma unroll 1
+  for (int jp = 1; jp < 4; ++jp) {
+    float2 part[4];
+    ssd_warp_item(w, r0, c, jp * jper, min((jp + 1) * jper, w.tw), part);
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      acc[k].x = __fadd_rn(acc[k].x, part[k].x);
+      acc[k].y = __fadd_rn(acc[k].y, part[k].y);
+    }
   }
 }
 
@@ -868,8 +949,7 @@ __host__ __device__ inline int64_t tile_bytes_needed_planar(int Su, int Sv, int 
   const int64_t r1 = align16((int64_t)Sv * Sp * 4);  // >= Mv * Mq * 4 (F_u) and >= Sv * Su * 2 (raw)
   const int64_t packed = (int64_t)(Sv + 4) * (Su + 4) * 4, planes = 2 * align16(Mv * Mq * 4);
   int64_t b = r1 + align16(packed > planes ? packed : planes);
-  b += align16((int64_t)nbins * 8) + align16((int64_t)nvals * 8) * 2;
-  b += align16((int64_t)th * tw * 8);
+  b += align16((int64_t)nbins * 8) + tile_template_bytes(tw, th, nvals);
   b += align16((int64_t)nbins * 4);
   return b;
 }
@@ -892,17 +972,19 @@ __device__ inline void tile_carve_planar(char* base, TileWork& w, TilePlanes& pl
   p += align16(packed > 2 * plane ? packed : 2 * plane);
   w.lut = reinterpret_cast<double*>(p);
   p += align16((int64_t)w.nbins * 8);
-  w.tq = reinterpret_cast<double*>(p);
-  p += align16((int64_t)w.nvals * 8);
-  w.tv = reinterpret_cast<double*>(p);
-  p += align16((int64_t)w.nvals * 8);
-  w.tmpl = reinterpret_cast<float2*>(p);
-  p += align16((int64_t)w.th * w.tw * 8);
+  if (!w.tcol) {
+    w.tq = reinterpret_cast<double*>(p);
+    p += align16((int64_t)w.nvals * 8);
+    w.tv = reinterpret_cast<double*>(p);
+    p += align16((int64_t)w.nvals * 8);
+    w.tmpl = reinterpret_cast<float2*>(p);
+    p += align16((int64_t)w.th * w.tw * 8);
+  }
   w.hist = reinterpret_cast<uint32_t*>(p);
 }
 
 // Phases 6-7 on planes; `out` = the surface's global region, float4 [Mv][Mp].  Same arithmetic as
-// tile_finish_interleaved with one template slice (JP = 1): identical results.
+// tile_finish_interleaved with one template slice (JP = 1), or four for a large template (ssd_warp_item_all).
 __device__ inline void tile_finish_planar(TileWork& w, const TilePlanes& pl, float4* __restrict__ out, float* dump_sse,
                                           int64_t dump_cap, long long* clk) {
   const int tid = threadIdx.x, nthr = blockDim.x, lane = tid & 31, warp = tid >> 5, nwarp = nthr >> 5;
@@ -914,7 +996,7 @@ __device__ inline void tile_finish_planar(TileWork& w, const TilePlanes& pl, flo
       const int rg = item / L.CB, cb = item - rg * L.CB;
       const int r0 = L.row(rg, lane), c = L.col(cb, lane);
       float2 acc[4];
-      ssd_warp_item(w, r0, c, 0, w.tw, acc);
+      ssd_warp_item_all(w, r0, c, acc);
 #pragma unroll
       for (int k = 0; k < 4; ++k)
         if (r0 + k < Mv) {
@@ -970,8 +1052,7 @@ __device__ inline void tile_finish_planar(TileWork& w, const TilePlanes& pl, flo
 // ---------------------------------------------------------------------------------------------
 __host__ __device__ inline int64_t tile_bytes_needed_staged(int Su, int Sv, int tw, int th, int nbins, int nvals) {
   int64_t b = align16((int64_t)Su * Sv * 2) + align16((int64_t)(Sv + 4) * (Su + 4) * 4);
-  b += align16((int64_t)nbins * 8) + align16((int64_t)nvals * 8) * 2;
-  b += align16((int64_t)th * tw * 8);
+  b += align16((int64_t)nbins * 8) + tile_template_bytes(tw, th, nvals);
   b += align16((int64_t)nbins * 4);
   const int64_t Mu = Su - tw + 1, Mv = Sv - th + 1, planes = 2 * align16(Mv * (Mu | 1) * 4);
   return b > planes ? b : planes;
@@ -993,12 +1074,14 @@ __device__ inline void tile_build_surface_staged(char* smem, char* region, const
   p += align16((int64_t)(w.Sv + 4) * (w.Su + 4) * 4);
   w.lut = reinterpret_cast<double*>(p);
   p += align16((int64_t)w.nbins * 8);
-  w.tq = reinterpret_cast<double*>(p);
-  p += align16((int64_t)w.nvals * 8);
-  w.tv = reinterpret_cast<double*>(p);
-  p += align16((int64_t)w.nvals * 8);
-  w.tmpl = reinterpret_cast<float2*>(p);
-  p += align16((int64_t)w.th * w.tw * 8);
+  if (!w.tcol) {
+    w.tq = reinterpret_cast<double*>(p);
+    p += align16((int64_t)w.nvals * 8);
+    w.tv = reinterpret_cast<double*>(p);
+    p += align16((int64_t)w.nvals * 8);
+    w.tmpl = reinterpret_cast<float2*>(p);
+    p += align16((int64_t)w.th * w.tw * 8);
+  }
   w.hist = reinterpret_cast<uint32_t*>(p);
   w.herm = nullptr;
   float* hp_global = reinterpret_cast<float*>(region);
@@ -1023,7 +1106,7 @@ __device__ inline void tile_build_surface_staged(char* smem, char* region, const
       const int rg = item / L.CB, cb = item - rg * L.CB;
       const int r0 = L.row(rg, lane), c = L.col(cb, lane);
       float2 acc[4];
-      ssd_warp_item(w, r0, c, 0, w.tw, acc);
+      ssd_warp_item_all(w, r0, c, acc);
 #pragma unroll
       for (int k = 0; k < 4; ++k)
         if (r0 + k < Mv) {

@@ -249,12 +249,18 @@ def lower_models(models, viewshed=None):
     return table_m, table, view
 
 
+def plan_template_flags(tw: int, th: int) -> int:
+    """The plan flag a ``tw`` x ``th`` template needs: templates above 1024 pixels are planned with their own organisation."""
+    return _lib.GB_PLAN_LARGE_TEMPLATES if tw * th > _lib.GB_MAX_TEMPLATE else 0
+
+
 def session_bytes(lib, mode: int, cluster: int, P: int, N: int, T: int, O: int, tw: int, th: int, return_covariances: bool,
                   return_particles: bool, window_margin: int = _lib.GB_WINDOW_MARGIN) -> int:
     """Device memory one :class:`Session` of ``P`` points allocates (the frames excluded): two particle-state buffers,
     the weights, the launch plan's scratch, templates and result blocks."""
     plan = _lib.gb_plan()
-    _lib.check(lib.gb_step_plan_ex(N, tw, th, P, O, int(cluster), mode, int(window_margin), C.byref(plan)))
+    flags = int(cluster) | plan_template_flags(tw, th)
+    _lib.check(lib.gb_step_plan_ex(N, tw, th, P, O, flags, mode, int(window_margin), C.byref(plan)))
     per_point = 2 * 48 * N + 8 * N                      # state_a, state_b, weight_state
     per_point += 3 * O * tw * th * 8 + O * 40           # templates
     per_point += T * ((36 if return_covariances else 6) + 6) * 8 + T * O * 9 + 16  # moments, flags, window sizes, status
@@ -308,6 +314,7 @@ class Session:
             if window_margin is None:
                 window_margin = getattr(tracker, "window_margin", _lib.GB_WINDOW_MARGIN)
             flags = _lib.GB_PLAN_RANKED_FRAMES if frames_need_ranks(tracker.observers, self.image_index) else 0
+            flags |= plan_template_flags(self.tw, self.th)
             _lib.check(self.lib.gb_step_plan_ex(N, self.tw, self.th, P, O, flags, mode, int(window_margin),
                                                 C.byref(self.plan)))
             self.h2d = 0

@@ -95,6 +95,17 @@ def highpass_size(highpass: dict):
     return highpass_params(highpass)[:2]
 
 
+def template_size(tile_size):
+    """(w, h) of ``Tracker.track(tile_size=...)``.  Templates up to 1024 pixels take any shape; larger ones have a kernel up to
+    128 pixels a side, and beyond that ``NotImplementedError`` is raised (there is no CPU fallback)."""
+    tw, th = (int(v) for v in tile_size)
+    side = _lib.GB_MAX_TEMPLATE_SIDE
+    if tw * th > _lib.GB_MAX_TEMPLATE and (tw > side or th > side):
+        raise NotImplementedError(f"tile_size: templates above {_lib.GB_MAX_TEMPLATE} pixels have a device kernel up to {side} x {side} "
+                                  f"pixels, not {tw} x {th}")
+    return tw, th
+
+
 def interpolation_degrees(interpolation: dict):
     """(kx, ky) of ``RectBivariateSpline(rows, columns, sse, **interpolation)`` (reference tracker.py:60, 584-594,
     observer.py:210): spline degree along the rows / columns of the SSE surface, 1 to 5 each (3 and 1 keep the Hermite-form
@@ -253,6 +264,7 @@ class Tracker:
             raise ValueError(f"unknown resample_method {self.resample_method!r}")
         highpass_size(self.highpass)  # raises for what has no device kernel
         interpolation_degrees(self.interpolation)
+        template_size(tile_size)
         self.reset()
         ntracks = len(motion_models)
         raise_errors = ntracks < 2

@@ -250,9 +250,13 @@ typedef struct gb_plan {
 
 /* Size a launch plan for N particles per point, a w x h template, P points and O observers.
  * `flags`: GB_PLAN_RANKED_FRAMES = some frame is not uint8 (the surface regions are sized for rank histograms of the largest window);
+ * GB_PLAN_LARGE_TEMPLATES = admit templates above 1024 pixels, up to 128 pixels a side (without it they return GB_E_RESOURCE;
+ * with it a template above 1024 pixels and above 128 pixels a side still does).  The kernels choose their path from the template
+ * size, not from the flag; gb_track* accept a template above 1024 pixels only with a plan whose max_template covers it.
  * `mode` must be GB_MODE_STREAM.
  * Plan fields that only that organisation used (cluster, particles_in_smem, n_slabs, slab_bytes, particle_scratch_bytes) are 1 / 0. */
 #define GB_PLAN_RANKED_FRAMES 1
+#define GB_PLAN_LARGE_TEMPLATES 2
 int gb_step_plan(int64_t n_particles, int32_t tile_w, int32_t tile_h, int64_t npoints, int32_t n_observers,
                  int32_t flags, int32_t mode, gb_plan* plan_host);
 /* The same with the capacity of the search windows chosen by the caller: in GB_MODE_STREAM every (point, observer) owns a surface
