@@ -8,7 +8,11 @@
 
 #define GB_MAX_OBS 8
 #define GB_XCH 36 /* doubles per slot of a block reduction (28 moment sums at most) */
+// histogram bins the 110 / 224 KB launch choice of large templates assumes (uint8 frames of up to 4 bands: 1021 bins)
 #define GB_MAX_BINS 1024
+// bands of a frame, and the grey levels of a uint8 frame with that many (its band sums 0 .. 255 * bands)
+#define GB_MAX_BANDS 8
+#define GB_MAX_U8_BINS (255 * GB_MAX_BANDS + 1)
 // Templates up to this many pixels keep their high-passed copy and CDF tables in shared memory next to the search window;
 // larger ones (GB_PLAN_LARGE_TEMPLATES, up to GB_MAX_TEMPLATE_SIDE a side) are read from global memory.
 #define GB_SMEM_TEMPLATE 1024

@@ -515,7 +515,7 @@ __global__ void __launch_bounds__(GB_THREADS) k_init(const __grid_constant__ Ste
 // region, which no kernel uses while templates are cut.  Otherwise the two variants run the same code.
 // ---------------------------------------------------------------------------------------------
 // histogram bins: one per rank of a ranked template, one per band sum of a uint8 frame of up to 8 bands
-__host__ __device__ inline int template_bins(int area) { return area > 255 * 8 + 1 ? area : 255 * 8 + 1; }
+__host__ __device__ inline int template_bins(int area) { return area > GB_MAX_U8_BINS ? area : GB_MAX_U8_BINS; }
 __host__ __device__ inline int template_smem_bytes(int area) {
   return (int)(align16((int64_t)template_bins(area) * 4) + 2 * align16((int64_t)area * 2));
 }
@@ -541,7 +541,7 @@ __global__ void __launch_bounds__(256) k_template(const __grid_constant__ StepPa
     s_vals = reinterpret_cast<double*>(prm.s_surf + (p * prm.O + o) * prm.surf_bytes);
   } else {
     __shared__ uint16_t a_raw[GB_SMEM_TEMPLATE];
-    __shared__ uint32_t a_hist[GB_MAX_BINS];
+    __shared__ uint32_t a_hist[GB_MAX_U8_BINS];
     __shared__ double a_vals[GB_SMEM_TEMPLATE];
     __shared__ uint16_t a_rep[GB_SMEM_TEMPLATE];
     s_raw = a_raw;
@@ -1015,6 +1015,14 @@ static int check_desc(const gb_track_desc& d) {
     return fail(GB_E_INVALID, "interp_rows / interp_cols: spline degrees 1 to 5 (0 = the default 3)%s");
   if (!d.sigmas == !d.covariances) return fail(GB_E_INVALID, "exactly one of sigmas / covariances must be given%s");
   if (!d.images_host) return fail(GB_E_INVALID, "images_host is required%s");
+  if (!d.image_offset_host || !d.image_index_host) return fail(GB_E_INVALID, "image_offset_host and image_index_host are required%s");
+  // the tile kernels size their grey-level histograms for 1 to GB_MAX_BANDS bands (frames no time references are not read)
+  for (int64_t k = 0; k < (int64_t)d.T * d.O; ++k) {
+    const int idx = d.image_index_host[k];
+    if (idx < 0) continue;
+    const int nchan = d.images_host[d.image_offset_host[k % d.O] + idx].nchan;
+    if (nchan < 1 || nchan > GB_MAX_BANDS) return fail(GB_E_INVALID, "frames must have 1 to 8 bands (gb_image.nchan)%s");
+  }
   if (!d.images || !d.mask || !d.first || !d.last || !d.motion || !d.surfaces || !d.state_a || !d.state_b || !d.means ||
       !d.status || !d.status_time || !d.obs_flags || !d.tmpl_tile || !d.tmpl_values || !d.tmpl_quantiles ||
       !d.tmpl_nvalues || !d.tmpl_box || !d.tmpl_duv)
@@ -1844,7 +1852,9 @@ int gb_step_plan_ex(int64_t n_particles, int32_t tile_w, int32_t tile_h, int64_t
       // the collocation factors of spline degrees 2 / 4 / 5
       const int64_t Su = tile_w + window_margin, Sv = tile_h + window_margin;
       const bool ranked = (flags & GB_PLAN_RANKED_FRAMES) != 0;
-      const int64_t bins = ranked ? (Su * Sv < 65535 ? Su * Sv : 65535) : GB_MAX_BINS;
+      // (uint8 frames: one bin per band sum, 255 * bands + 1 for up to GB_MAX_BANDS bands; a ranked plan may hold them too)
+      const int64_t ranks = Su * Sv < 65535 ? Su * Sv : 65535;
+      const int64_t bins = ranked && ranks > GB_MAX_U8_BINS ? ranks : GB_MAX_U8_BINS;
       int64_t bytes = tile_bytes_needed((int)Su, (int)Sv, tile_w, tile_h, (int)bins, tile_w * tile_h) + 16;
       bytes += bspline_band_bytes((int)(Su - tile_w + 1), (int)(Sv - tile_h + 1), 5, 5) + 16;
       if (ranked) bytes += bins * 8 + 16;

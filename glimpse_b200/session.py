@@ -487,7 +487,7 @@ class Session:
 
     # ---------------------------------------------------------------- uploads
     def _upload_frames(self):
-        """Copy every frame ``image_index`` references to the device as it is (uint8, 1-4 bands; reference
+        """Copy every frame ``image_index`` references to the device as it is (``device_frame``: 1-8 bands; reference
         ``Observer.cache_images`` / ``Image.read``, tracker.py:295-299).  Copies go to a side stream in
         time order, each followed by an event that ``gb_track`` waits on before the first kernel that reads
         the frame, so the upload of later frames overlaps the tracking of earlier ones."""

@@ -92,6 +92,41 @@ def test_plan_sizes():
     assert b"removed" in lib.gb_last_error()
 
 
+def test_track_entry_points_refuse_frames_without_1_to_8_bands():
+    """gb_track, gb_track_step and gb_track_init check every frame a time references for 1-8 bands before any device work
+    (the tile kernels size their grey-level histograms for 255 * 8 + 1 levels); frames no time references are not read."""
+    from glimpse_b200 import _lib
+
+    lib = _lib.load()
+    d = _lib.gb_track_desc()
+    d.P, d.N, d.T, d.O, d.tile_w, d.tile_h = 1, 4, 2, 1, 15, 15
+    assert lib.gb_step_plan(4, 15, 15, 1, 1, 0, _lib.GB_MODE_STREAM, C.byref(d.plan)) == 0
+    fake = 1 << 20  # device pointers are not dereferenced by the argument checks
+    for name in ("images", "mask", "first", "last", "motion", "surfaces", "state_a", "state_b", "means", "sigmas", "status",
+                 "status_time", "obs_flags", "tmpl_tile", "tmpl_values", "tmpl_quantiles", "tmpl_nvalues", "tmpl_box", "tmpl_duv",
+                 "scratch", "init_normals", "step_normals", "uniforms"):
+        setattr(d, name, fake)
+    images = (_lib.gb_image * 2)()
+    offsets = np.array([0, 2], dtype=np.int32)
+    index = np.zeros((2, 1), dtype=np.int32)  # image 1 is never referenced
+    d.images_host, d.image_offset_host, d.image_index_host = C.addressof(images), offsets.ctypes.data, index.ctypes.data
+    calls = {"gb_track": lambda: lib.gb_track(C.byref(d), None, None),
+             "gb_track_step": lambda: lib.gb_track_step(C.byref(d), 1, None, None),
+             "gb_track_init": lambda: lib.gb_track_init(C.byref(d), 0, None)}
+    for name, call in calls.items():
+        for nchan in (0, 9, -1, 255):
+            images[0].nchan, images[1].nchan = nchan, 1
+            assert call() == -1, (name, nchan)
+            assert b"1 to 8 bands" in lib.gb_last_error(), (name, nchan)
+        # 1-8 bands pass this check (the next one, a missing buffer, fails instead), whatever an unreferenced frame holds
+        d.means = None
+        for nchan in (1, 5, 8):
+            images[0].nchan, images[1].nchan = nchan, 0
+            assert call() == -1, (name, nchan)
+            assert b"missing required buffer" in lib.gb_last_error(), (name, nchan)
+        d.means = fake
+
+
 def test_point_span_and_shards():
     from glimpse_b200.session import point_span
     from glimpse_b200.tracker import shard_bounds
