@@ -11,7 +11,7 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libglimpse_b200.so")
 
-GB_MAX_OBS = 8
+GB_MAX_OBS = 8  # observers with a frame at the same time (GB_MAX_OBSERVERS); a call may have any number of observers
 GB_ST_MESSAGES = {
     1: (ValueError, "Some particles are on non-visible viewshed cells"),
     2: (ValueError, "Some particles have missing (NaN) values"),
@@ -21,7 +21,7 @@ GB_ST_MESSAGES = {
     6: (MemoryError, "Search window larger than the launch plan's surface capacity (template + 191 px per axis in mode='stream'; "
                      "the particle cloud has dispersed)"),
 }
-GB_OBS_OUT_OF_FRAME = 2
+GB_OBS_NO_IMAGE, GB_OBS_OUT_OF_FRAME = 1, 2
 GB_ST_WINDOW_TOO_LARGE = 6
 GB_WINDOW_MARGIN, GB_WINDOW_MARGIN_MAX = 191, 1000  # default / retry capacity of the search windows beyond the template, px
 GB_RNG_SUPPLIED, GB_RNG_PHILOX = 0, 1

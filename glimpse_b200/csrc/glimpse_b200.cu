@@ -56,11 +56,16 @@ struct StepParams {
   uint64_t seed;
   int64_t point_offset;
   double tau, tau2;
-  int img[GB_MAX_OBS];       // global image index of each observer at time t, -1 = none
+  // Slots of time t: what a time step uses once and discards (the arrays below, the scratch regions, the grids of k_s2_surface
+  // and k_template) is indexed by slot; templates, masks and outputs by observer obs[s].  A call of up to GB_MAX_OBS observers
+  // has the identity table (n_slots = O, obs[s] = s); a larger one lists the observers with a frame at t in ascending order.
+  int n_slots, slot_stride;  // slots in use at t; slots per point in the scratch layout (plan.n_observers)
+  int obs[GB_MAX_OBS];       // observer of each slot
+  int img[GB_MAX_OBS];       // global image index of each slot's observer at time t, -1 = none
   CamK cam[GB_MAX_OBS];      // that image's camera (constant bank: operands without loads)
   const uint8_t* pixels[GB_MAX_OBS];
   int pitch[GB_MAX_OBS], nchan[GB_MAX_OBS], pixdtype[GB_MAX_OBS];
-  int tmpl_frame[GB_MAX_OBS]; // time index at which each observer's template is cut
+  int tmpl_frame[GB_MAX_OBS]; // time index at which each slot's observer's template is cut
   double obs_scale[GB_MAX_OBS];
   const gb_image* images;
   const uint8_t* mask;
@@ -97,16 +102,16 @@ struct StepParams {
   double* s_ev_next; // [P][6][N]   pipelined flow: particles advanced to the next time (other parity)
   double* s_ref;     // [P][6]      pipelined flow: fixed origin of the moment sums
   int* s_pflags_next; // [P]        pipelined flow: flags of the next time
-  double* s_uv;      // [P][O][2][N] projected particles
+  double* s_uv;      // [P][slot][2][N] projected particles
   double* s_w;       // [P][N]      weights
   double* s_bsum;    // [P][nblk]   per-CTA weight totals
   double* s_pm;      // [P][nblk][28] per-CTA moment sums
   double* s_pre;     // [P][nblk + 4] prefix of the CTA totals (0 .. total), 1 / total, uniform draw, 1 / N (written by k_s3b_publish)
-  int* s_ibox;       // [P][O][5]   integer cloud box (left, top, -right, -bottom, -(any NaN))
+  int* s_ibox;       // [P][slot][5] integer cloud box (left, top, -right, -bottom, -(any NaN))
   int* s_pflags;     // [P]         GB_F_* raised during this update
   uint8_t* s_act;    // [P]         GB_ACT_* bits of this update
-  int* s_meta;       // [P][O][8]   surface meta: box[4], Mu, Mv, Mp, ok
-  char* s_surf;      // [P][O] surface regions of surf_bytes each (Hermite array first)
+  int* s_meta;       // [P][slot][8] surface meta: box[4], Mu, Mv, Mp, ok
+  char* s_surf;      // [P][slot] surface regions of surf_bytes each (Hermite array first)
   int64_t surf_bytes;
   int s_block, s_nblk;
   int tmpl_from_ev;  // k_template: staggered templates read the evolved particles from s_ev (pipelined flow)
@@ -120,13 +125,15 @@ struct StepParams {
 // What k_s4p needs to know about the NEXT time to advance the particles to it.
 struct NextParams {
   double tau, tau2;
-  int spec_update, pad_;  // no point starts at this time: every active point is resampled, k_s4p may request its parents early
+  int spec_update;  // no point starts at this time: every active point is resampled, k_s4p may request its parents early
+  int n_slots;      // the slot table of the next time (see StepParams)
+  int obs[GB_MAX_OBS];
   int img[GB_MAX_OBS];
   CamK cam[GB_MAX_OBS];
 };
 
-// Tensor maps (TMA descriptors) of the frames the observers show at time t: a kernel parameter of k_s2_surface, so the
-// descriptors live in the constant bank of the launch.  ok[o] = 0: that frame is read with ordinary loads.
+// Tensor maps (TMA descriptors) of the frames the slots show at time t: a kernel parameter of k_s2_surface, so the
+// descriptors live in the constant bank of the launch.  ok[s] = 0: that frame is read with ordinary loads.
 struct alignas(64) FrameMaps {
   CUtensorMap map[GB_MAX_OBS];
   int ok[GB_MAX_OBS];
@@ -509,9 +516,10 @@ __global__ void __launch_bounds__(GB_THREADS) k_init(const __grid_constant__ Ste
 }
 
 // ---------------------------------------------------------------------------------------------
-// Template construction (tracker.py:536-561, 494-534): one CTA per (point, observer) due at t.
+// Template construction (tracker.py:536-561, 494-534): one CTA per (point, slot) of time t; the template of the slot's
+// observer is cut when t is its template frame.
 // LARGE: templates above GB_SMEM_TEMPLATE pixels (GB_PLAN_LARGE_TEMPLATES).  Their levels, histogram and representatives
-// live in dynamic shared memory (template_smem_bytes), the grey values of ranked frames in the (point, observer)'s surface
+// live in dynamic shared memory (template_smem_bytes), the grey values of ranked frames in the (point, slot)'s surface
 // region, which no kernel uses while templates are cut.  Otherwise the two variants run the same code.
 // ---------------------------------------------------------------------------------------------
 // histogram bins: one per rank of a ranked template, one per band sum of a uint8 frame of up to 8 bands
@@ -526,8 +534,9 @@ __global__ void __launch_bounds__(256) k_template(const __grid_constant__ StepPa
   __shared__ int s_box[4];
   __shared__ int s_ok;
   __shared__ double s_stats[2];
-  const int64_t p = blockIdx.x / prm.O;
-  const int o = (int)(blockIdx.x - p * prm.O);
+  const int64_t p = blockIdx.x / prm.n_slots;
+  const int slot = (int)(blockIdx.x - p * prm.n_slots), o = prm.obs[slot];
+  const int64_t po = p * prm.O + o;
   uint16_t* s_raw;   // grey level of every pixel
   uint32_t* s_hist;  // pixels per level
   double* s_vals;    // frames other than uint8: the tile's grey values ...
@@ -538,7 +547,7 @@ __global__ void __launch_bounds__(256) k_template(const __grid_constant__ StepPa
     s_hist = reinterpret_cast<uint32_t*>(smem_raw);
     s_raw = reinterpret_cast<uint16_t*>(smem_raw + align16((int64_t)template_bins(a) * 4));
     s_rep = reinterpret_cast<uint16_t*>(smem_raw + align16((int64_t)template_bins(a) * 4) + align16((int64_t)a * 2));
-    s_vals = reinterpret_cast<double*>(prm.s_surf + (p * prm.O + o) * prm.surf_bytes);
+    s_vals = reinterpret_cast<double*>(prm.s_surf + (p * prm.slot_stride + slot) * prm.surf_bytes);
   } else {
     __shared__ uint16_t a_raw[GB_SMEM_TEMPLATE];
     __shared__ uint32_t a_hist[GB_MAX_U8_BINS];
@@ -550,7 +559,7 @@ __global__ void __launch_bounds__(256) k_template(const __grid_constant__ StepPa
     s_rep = a_rep;
   }
   const int t = prm.t;
-  if (prm.status[p] != 0 || prm.tmpl_frame[o] != t || !prm.mask[p * prm.O + o] || prm.img[o] < 0) return;
+  if (prm.status[p] != 0 || prm.tmpl_frame[slot] != t || !prm.mask[po] || prm.img[slot] < 0) return;
   if (t < prm.first[p] || t > prm.last[p]) return;
   const int64_t N = prm.N;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -572,7 +581,7 @@ __global__ void __launch_bounds__(256) k_template(const __grid_constant__ StepPa
     if (lane == 0) s_red[warp][k] = x;
   }
   __syncthreads();
-  const gb_image* img = prm.images + prm.img[o];
+  const gb_image* img = prm.images + prm.img[slot];
   const int tw = prm.tile_w, th = prm.tile_h;
   if (tid == 0) {
     double tot[4] = {0, 0, 0, 0};
@@ -592,9 +601,9 @@ __global__ void __launch_bounds__(256) k_template(const __grid_constant__ StepPa
       s_box[1] = (int)floor(tp + 0.5);
       s_box[2] = (int)floor(r + 0.5);
       s_box[3] = (int)floor(b + 0.5);
-      int32_t* gbox = prm.tmpl_box + (p * prm.O + o) * 4;
+      int32_t* gbox = prm.tmpl_box + po * 4;
       for (int k = 0; k < 4; ++k) gbox[k] = s_box[k];
-      double* duv = prm.tmpl_duv + (p * prm.O + o) * 2;
+      double* duv = prm.tmpl_duv + po * 2;
       duv[0] = sub(u, (double)(s_box[0] + s_box[2]) / 2.0);
       duv[1] = sub(v, (double)(s_box[1] + s_box[3]) / 2.0);
     } else {
@@ -677,8 +686,8 @@ __global__ void __launch_bounds__(256) k_template(const __grid_constant__ StepPa
   // CDF over occupied grey levels (helpers.py:433-464): levels are visited in increasing order, and
   // the normalised value is an increasing function of the level, so this is np.unique's order.
   if (tid == 0) {
-    double* vals = prm.tmpl_values + (p * prm.O + o) * (int64_t)(tw * th);
-    double* qs = prm.tmpl_quantiles + (p * prm.O + o) * (int64_t)(tw * th);
+    double* vals = prm.tmpl_values + po * (int64_t)(tw * th);
+    double* qs = prm.tmpl_quantiles + po * (int64_t)(tw * th);
     int n = 0;
     uint32_t run = 0;
     for (int b = 0; b < nbins; ++b) {
@@ -688,11 +697,11 @@ __global__ void __launch_bounds__(256) k_template(const __grid_constant__ StepPa
       qs[n] = quo((double)run, (double)area);
       ++n;
     }
-    prm.tmpl_nvalues[p * prm.O + o] = n;
+    prm.tmpl_nvalues[po] = n;
   }
   // high-pass (tracker.py:530-531): value minus the reflected median (5x5 unless Tracker.highpass says otherwise), taken
   // on grey levels
-  double* tile = prm.tmpl_tile + (p * prm.O + o) * (int64_t)(tw * th);
+  double* tile = prm.tmpl_tile + po * (int64_t)(tw * th);
   const bool hp_plain = prm.hp_mode == GB_HP_REFLECT && prm.hp_org_r == 0 && prm.hp_org_c == 0 && !prm.hp_has_fp;
   const bool hp5 = prm.hp_rows == 5 && prm.hp_cols == 5 && hp_plain;
   // (general border mode: the constant beyond the border takes its place among the grey levels through the normalised values)
@@ -889,13 +898,31 @@ static int ensure_tensor_maps(const gb_track_desc& d) {
 static void frame_maps(const StepParams& prm, FrameMaps& fm) {
   memset(&fm, 0, sizeof(fm));
   if (!g_tmaps_on) return;
-  for (int o = 0; o < prm.O; ++o) {
-    const int image = prm.img[o];
+  for (int s = 0; s < prm.n_slots; ++s) {
+    const int image = prm.img[s];
     if (image >= 0 && (size_t)image < g_tmaps.ok.size() && g_tmaps.ok[image]) {
-      fm.map[o] = g_tmaps.host[image];
-      fm.ok[o] = 1;
+      fm.map[s] = g_tmaps.host[image];
+      fm.ok[s] = 1;
     }
   }
+}
+
+// Time index at which observer o's template is cut: its first frame (-1: none).
+static int template_frame(const gb_track_desc& d, int o) {
+  for (int t = 0; t < d.T; ++t)
+    if (d.image_index_host[(int64_t)t * d.O + o] >= 0) return t;
+  return -1;
+}
+
+// Most observers with a frame at one time (image_index_host >= 0).
+static int max_active_observers(const gb_track_desc& d) {
+  int most = 0;
+  for (int t = 0; t < d.T; ++t) {
+    int n = 0;
+    for (int o = 0; o < d.O; ++o) n += d.image_index_host[(int64_t)t * d.O + o] >= 0;
+    if (n > most) most = n;
+  }
+  return most;
 }
 
 static void fill_params(const gb_track_desc& d, int t, StepParams& prm) {
@@ -934,26 +961,33 @@ static void fill_params(const gb_track_desc& d, int t, StepParams& prm) {
     prm.tau = d.tau_host[t - 1];
     prm.tau2 = d.tau2_host[t - 1];
   }
+  // the slot table (check_desc has bounded the observers with a frame at t by the plan's slots)
+  prm.slot_stride = d.plan.n_observers;
+  int n = 0;
   for (int o = 0; o < d.O; ++o) {
     const int idx = d.image_index_host[(int64_t)t * d.O + o];
-    prm.img[o] = idx >= 0 ? d.image_offset_host[o] + idx : -1;
+    if (d.O > GB_MAX_OBS && idx < 0) continue;
+    const int s = n++;
+    prm.obs[s] = o;
+    prm.img[s] = idx >= 0 ? d.image_offset_host[o] + idx : -1;
     if (idx >= 0 && d.images_host) {
-      const gb_image& im = d.images_host[prm.img[o]];
-      camk_from(im.cam, prm.cam[o]);
-      prm.pixels[o] = im.pixels;
-      prm.pitch[o] = im.pitch;
-      prm.nchan[o] = im.nchan;
-      prm.pixdtype[o] = im.dtype;
+      const gb_image& im = d.images_host[prm.img[s]];
+      camk_from(im.cam, prm.cam[s]);
+      prm.pixels[s] = im.pixels;
+      prm.pitch[s] = im.pitch;
+      prm.nchan[s] = im.nchan;
+      prm.pixdtype[s] = im.dtype;
     }
-    prm.obs_scale[o] = d.obs_scale_host[o];
-    int tf = -1;
-    for (int tt = 0; tt < d.T; ++tt)
-      if (d.image_index_host[(int64_t)tt * d.O + o] >= 0) {
-        tf = tt;
-        break;
-      }
-    prm.tmpl_frame[o] = tf;
+    prm.obs_scale[s] = d.obs_scale_host[o];
+    prm.tmpl_frame[s] = template_frame(d, o);
   }
+  if (n == 0) {  // no frame at t: one empty slot keeps the grids non-empty (it flags its observer GB_OBS_NO_IMAGE, as it has no frame)
+    prm.obs[0] = 0;
+    prm.img[0] = -1;
+    prm.tmpl_frame[0] = -1;
+    n = 1;
+  }
+  prm.n_slots = n;
   prm.images = d.images;
   prm.mask = d.mask;
   prm.first = d.first;
@@ -988,7 +1022,7 @@ static void fill_params(const gb_track_desc& d, int t, StepParams& prm) {
 
 static int check_desc(const gb_track_desc& d) {
   if (d.P <= 0 || d.N <= 0 || d.T < 2) return fail(GB_E_INVALID, "P, N must be positive and T >= 2%s");
-  if (d.O < 1 || d.O > GB_MAX_OBS) return fail(GB_E_INVALID, "between 1 and 8 observers are supported%s");
+  if (d.O < 1) return fail(GB_E_INVALID, "at least one observer is required%s");
   if (d.tile_w < 1 || d.tile_h < 1 || (int64_t)d.tile_w * d.tile_h > GB_MAX_TEMPLATE) {
     if (d.tile_w < 1 || d.tile_h < 1 || (int64_t)d.tile_w * d.tile_h > d.plan.max_template)
       return fail(GB_E_RESOURCE, "template larger than 1024 pixels (or than the plan's max_template)%s");
@@ -1031,7 +1065,16 @@ static int check_desc(const gb_track_desc& d) {
     return fail(GB_E_INVALID, "supplied-draw mode needs init_normals, step_normals and uniforms%s");
   if (d.plan.mode != GB_MODE_STREAM || d.plan.threads != GB_THREADS || d.plan.n_local < 1)
     return fail(GB_E_INVALID, "invalid launch plan (use gb_step_plan)%s");
-  if ((d.plan.n_observers != d.O || d.plan.stream_nblk < 1 || d.plan.surf_bytes <= 0 ||
+  // up to GB_MAX_OBS observers: one slot each; more: one slot per observer with a frame at the same time, up to GB_MAX_OBS
+  if (d.O > GB_MAX_OBS) {
+    const int active = max_active_observers(d);
+    if (active > GB_MAX_OBS) return fail(GB_E_RESOURCE, "more than 8 observers have a frame at the same time%s");
+    if (d.plan.n_observers < (active > 1 ? active : 1) || d.plan.n_observers > GB_MAX_OBS)
+      return fail(GB_E_INVALID, "plan.n_observers must cover the observers with a frame at the same time (use gb_step_plan)%s");
+  } else if (d.plan.n_observers != d.O) {
+    return fail(GB_E_INVALID, "streaming plan does not match the descriptor (use gb_step_plan)%s");
+  }
+  if ((d.plan.stream_nblk < 1 || d.plan.surf_bytes <= 0 ||
                                         d.plan.stream_batch < 1 || d.plan.stream_slots < 1 || d.plan.stream_slots > kMaxSlots))
     return fail(GB_E_INVALID, "streaming plan does not match the descriptor (use gb_step_plan)%s");
   if (d.plan.scratch_bytes > 0 && !d.scratch) return fail(GB_E_INVALID, "plan needs a scratch buffer%s");
@@ -1089,7 +1132,7 @@ static StreamLayout stream_layout(int64_t B, int64_t N, int64_t O, int64_t nblk,
 // the batch of points [p0, p0 + pb).
 static void stream_bind(const gb_track_desc& d, StepParams& prm, int par, int64_t p0, int64_t pb) {
   const gb_plan& pl = d.plan;
-  const StreamLayout L = stream_layout(d.P, d.N, d.O, pl.stream_nblk, pl.surf_bytes);
+  const StreamLayout L = stream_layout(d.P, d.N, pl.n_observers, pl.stream_nblk, pl.surf_bytes);
   char* base = reinterpret_cast<char*>(d.scratch);
   prm.s_ev = reinterpret_cast<double*>(base + L.ev[par & 1]);
   prm.s_ev_next = reinterpret_cast<double*>(base + L.ev[(par + 1) & 1]);
@@ -1149,14 +1192,14 @@ static int get_pool(StreamPool** out) {
 template <bool COV>
 static int launch_stream_batch(const StepParams& prm, cudaStream_t stream) {
   const unsigned nb = (unsigned)(prm.pb * prm.s_nblk);
-  k_s0_reset<<<grid_for(prm.pb * prm.O * 5, 256), 256, 0, stream>>>(prm);
+  k_s0_reset<<<grid_for(prm.pb * prm.slot_stride * 5, 256), 256, 0, stream>>>(prm);
   k_s1_propagate<<<nb, GB_SBLOCK_THREADS, 0, stream>>>(prm);
   FrameMaps fm;
   frame_maps(prm, fm);
   if (prm.tile_w * prm.tile_h > GB_SMEM_TEMPLATE)
-    k_s2_surface<true><<<(unsigned)(prm.pb * prm.O), GB_S2_THREADS, prm.s2_smem, stream>>>(prm, fm, prm.s2_budget);
+    k_s2_surface<true><<<(unsigned)(prm.pb * prm.n_slots), GB_S2_THREADS, prm.s2_smem, stream>>>(prm, fm, prm.s2_budget);
   else
-    k_s2_surface<false><<<(unsigned)(prm.pb * prm.O), GB_S2_THREADS, prm.s2_smem, stream>>>(prm, fm, prm.s2_budget);
+    k_s2_surface<false><<<(unsigned)(prm.pb * prm.n_slots), GB_S2_THREADS, prm.s2_smem, stream>>>(prm, fm, prm.s2_budget);
   if (spline_is_hermite(prm.interp_cols, prm.interp_rows))
     k_s3_weights<false><<<dim3((unsigned)prm.s_nblk, (unsigned)prm.pb), s3_threads(prm.s_block), 0, stream>>>(prm);
   else
@@ -1203,10 +1246,10 @@ static int launch_stream_update(const gb_track_desc& d, StepParams& prm, cudaStr
     for (int k = 0; k < used; ++k) GB_CUDA(cudaStreamWaitEvent(pool->side[k], pool->fork, 0));
   }
   if (d.image_events_host)
-    for (int o = 0; o < d.O; ++o)
-      if (prm.img[o] >= 0 && d.image_events_host[prm.img[o]])
+    for (int s = 0; s < prm.n_slots; ++s)
+      if (prm.img[s] >= 0 && d.image_events_host[prm.img[s]])
         for (int k = 0; k < used; ++k)
-          GB_CUDA(cudaStreamWaitEvent(pool->side[k], (cudaEvent_t)d.image_events_host[prm.img[o]], 0));
+          GB_CUDA(cudaStreamWaitEvent(pool->side[k], (cudaEvent_t)d.image_events_host[prm.img[s]], 0));
   for (int64_t b = 0; b < nbatch; ++b) {
     const int slot = (int)(b % slots);
     const int64_t p0 = b * batch, pb = (p0 + batch <= d.P) ? batch : d.P - p0;
@@ -1300,8 +1343,8 @@ static int track_streaming(const gb_track_desc& d, cudaStream_t stream, int64_t*
   int rc = get_pool(&pool);
   if (rc) return rc;
   std::lock_guard<std::mutex> guard(pool->busy);
-  StepParams probe;
-  fill_params(d, 0, probe);
+  std::vector<int> tmpl_frame(d.O);
+  for (int o = 0; o < d.O; ++o) tmpl_frame[o] = template_frame(d, o);
   // what happens at each time (host copies of first / last / mask)
   const int T = d.T;
   std::vector<uint8_t> has_init(T, 0), has_tmpl(T, 0), has_update(T, 0), has_prop(T, 0);
@@ -1315,7 +1358,7 @@ static int track_streaming(const gb_track_desc& d, cudaStream_t stream, int64_t*
       if (t < l) has_prop[t] = 1;
     }
     for (int o = 0; o < d.O; ++o) {
-      const int tf = probe.tmpl_frame[o];
+      const int tf = tmpl_frame[o];
       if (tf >= f && tf <= l && d.mask_host[p * d.O + o]) {
         has_tmpl[tf] = 1;
         if (tf > f) staggered_any = true;
@@ -1326,9 +1369,9 @@ static int track_streaming(const gb_track_desc& d, cudaStream_t stream, int64_t*
     return fail(GB_E_INVALID, "weight_state is required when a template starts after a point's first frame%s");
   auto wait_images = [&](cudaStream_t s, const StepParams& prm) -> int {
     if (!d.image_events_host) return GB_OK;
-    for (int o = 0; o < d.O; ++o)
-      if (prm.img[o] >= 0 && d.image_events_host[prm.img[o]])
-        GB_CUDA(cudaStreamWaitEvent(s, (cudaEvent_t)d.image_events_host[prm.img[o]], 0));
+    for (int k = 0; k < prm.n_slots; ++k)
+      if (prm.img[k] >= 0 && d.image_events_host[prm.img[k]])
+        GB_CUDA(cudaStreamWaitEvent(s, (cudaEvent_t)d.image_events_host[prm.img[k]], 0));
     return GB_OK;
   };
   bool forked = false, need_fork = true;
@@ -1346,7 +1389,7 @@ static int track_streaming(const gb_track_desc& d, cudaStream_t stream, int64_t*
     StepParams prm;
     fill_params(d, 0, prm);
     stream_bind(d, prm, 0, 0, d.P);
-    k_s0p_reset<<<grid_for(d.P * d.O * 5, 256), 256, 0, stream>>>(prm);
+    k_s0p_reset<<<grid_for(d.P * prm.slot_stride * 5, 256), 256, 0, stream>>>(prm);
     GB_CUDA(cudaGetLastError());
     if (launches) ++*launches;
   }
@@ -1368,9 +1411,11 @@ static int track_streaming(const gb_track_desc& d, cudaStream_t stream, int64_t*
       fill_params(d, t + 1, pn);
       nxt.tau = pn.tau;
       nxt.tau2 = pn.tau2;
-      for (int o = 0; o < d.O; ++o) {
-        nxt.img[o] = pn.img[o];
-        nxt.cam[o] = pn.cam[o];
+      nxt.n_slots = pn.n_slots;
+      for (int s = 0; s < pn.n_slots; ++s) {
+        nxt.obs[s] = pn.obs[s];
+        nxt.img[s] = pn.img[s];
+        nxt.cam[s] = pn.cam[s];
       }
     }
     FrameMaps fm;
@@ -1418,9 +1463,9 @@ static int track_streaming(const gb_track_desc& d, cudaStream_t stream, int64_t*
       if (has_update[t]) {
         kt.begin(GB_K_SURFACE, ss);
         if (prm.tile_w * prm.tile_h > GB_SMEM_TEMPLATE)
-          k_s2_surface<true><<<(unsigned)(pb * prm.O), GB_S2_THREADS, prm.s2_smem, ss>>>(prm, fm, prm.s2_budget);
+          k_s2_surface<true><<<(unsigned)(pb * prm.n_slots), GB_S2_THREADS, prm.s2_smem, ss>>>(prm, fm, prm.s2_budget);
         else
-          k_s2_surface<false><<<(unsigned)(pb * prm.O), GB_S2_THREADS, prm.s2_smem, ss>>>(prm, fm, prm.s2_budget);
+          k_s2_surface<false><<<(unsigned)(pb * prm.n_slots), GB_S2_THREADS, prm.s2_smem, ss>>>(prm, fm, prm.s2_budget);
         kt.end(ss);
         kt.begin(GB_K_WEIGHTS, ss);
         if (spline_is_hermite(prm.interp_cols, prm.interp_rows))
@@ -1481,10 +1526,10 @@ static int launch_init(const StepParams& prm, bool cov, cudaStream_t stream) {
 static int launch_template(const gb_track_desc& d, StepParams prm, cudaStream_t stream) {
   const int area = prm.tile_w * prm.tile_h;
   if (area <= GB_SMEM_TEMPLATE) {
-    k_template<false><<<(unsigned)(prm.P * prm.O), 256, 0, stream>>>(prm);
+    k_template<false><<<(unsigned)(prm.P * prm.n_slots), 256, 0, stream>>>(prm);
   } else {
     // the work area of ranked frames: the surface regions (plan.surf_bytes >= 8 B a template pixel)
-    prm.s_surf = reinterpret_cast<char*>(d.scratch) + stream_layout(d.P, d.N, d.O, d.plan.stream_nblk, d.plan.surf_bytes).surf;
+    prm.s_surf = reinterpret_cast<char*>(d.scratch) + stream_layout(d.P, d.N, d.plan.n_observers, d.plan.stream_nblk, d.plan.surf_bytes).surf;
     prm.surf_bytes = d.plan.surf_bytes;
     const int smem = template_smem_bytes(area);
     static std::once_flag once[16];
@@ -1495,7 +1540,7 @@ static int launch_template(const gb_track_desc& d, StepParams prm, cudaStream_t 
       err = cudaFuncSetAttribute(k_template<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, template_smem_bytes(GB_MAX_TEMPLATE_SIDE * GB_MAX_TEMPLATE_SIDE));
     });
     if (err != cudaSuccess) return fail(GB_E_CUDA, "k_template attributes: %s", cudaGetErrorString(err));
-    k_template<true><<<(unsigned)(prm.P * prm.O), 256, smem, stream>>>(prm);
+    k_template<true><<<(unsigned)(prm.P * prm.n_slots), 256, smem, stream>>>(prm);
   }
   GB_CUDA(cudaGetLastError());
   return GB_OK;
@@ -1931,8 +1976,8 @@ int gb_track(const gb_track_desc* d, void* stream_, int64_t* launches_out) {
     return GB_OK;
   }
   // per-time work flags from the host copies (tracker.py:321-347)
-  StepParams probe;
-  fill_params(*d, 0, probe);
+  std::vector<int> tmpl_frame(d->O);
+  for (int o = 0; o < d->O; ++o) tmpl_frame[o] = template_frame(*d, o);
   // In GB_MODE_STREAM the updates run on side streams that advance batch by batch without meeting; the
   // caller's stream forks them after its own kernels (init, templates, in-place evolve) and joins them
   // before the next such kernel and at the end.
@@ -1959,7 +2004,7 @@ int gb_track(const gb_track_desc* d, void* stream_, int64_t* launches_out) {
       if (f < t && t <= l) any_step = true;
       if (f <= t && t <= l)
         for (int o = 0; o < d->O; ++o)
-          if (probe.tmpl_frame[o] == t && d->mask_host[p * d->O + o]) {
+          if (tmpl_frame[o] == t && d->mask_host[p * d->O + o]) {
             any_tmpl = true;
             if (f < t) staggered = true;
           }
@@ -1970,9 +2015,9 @@ int gb_track(const gb_track_desc* d, void* stream_, int64_t* launches_out) {
     if (any_init || staggered || any_tmpl) {
       if ((rc = join_sides())) return rc;
       if (d->image_events_host)
-        for (int o = 0; o < d->O; ++o)
-          if (prm.img[o] >= 0 && d->image_events_host[prm.img[o]])
-            GB_CUDA(cudaStreamWaitEvent(stream, (cudaEvent_t)d->image_events_host[prm.img[o]], 0));
+        for (int s = 0; s < prm.n_slots; ++s)
+          if (prm.img[s] >= 0 && d->image_events_host[prm.img[s]])
+            GB_CUDA(cudaStreamWaitEvent(stream, (cudaEvent_t)d->image_events_host[prm.img[s]], 0));
     }
     if (any_init) {
       if ((rc = launch_init(prm, cov, stream))) return rc;
@@ -1994,9 +2039,9 @@ int gb_track(const gb_track_desc* d, void* stream_, int64_t* launches_out) {
     }
     if (any_step) {
       if (!streaming && d->image_events_host)
-        for (int o = 0; o < d->O; ++o)
-          if (prm.img[o] >= 0 && d->image_events_host[prm.img[o]])
-            GB_CUDA(cudaStreamWaitEvent(stream, (cudaEvent_t)d->image_events_host[prm.img[o]], 0));
+        for (int s = 0; s < prm.n_slots; ++s)
+          if (prm.img[s] >= 0 && d->image_events_host[prm.img[s]])
+            GB_CUDA(cudaStreamWaitEvent(stream, (cudaEvent_t)d->image_events_host[prm.img[s]], 0));
       if ((rc = launch_update(*d, prm, stream, need_fork, false, &launches))) return rc;
       forked = true;
       need_fork = false;

@@ -28,7 +28,7 @@ __device__ __forceinline__ bool stream_point_active(const StepParams& prm, int64
 __global__ void k_s0_reset(const __grid_constant__ StepParams prm) {
   // scratch arrays are indexed by the global point number; the host pre-shifts their base pointers so
   // that the batch [p0, p0 + pb) lands in the batch's slot
-  const int64_t lo5 = prm.p0 * prm.O * 5, n = prm.pb * prm.O * 5;
+  const int64_t lo5 = prm.p0 * prm.slot_stride * 5, n = prm.pb * prm.slot_stride * 5;
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
     prm.s_ibox[lo5 + i] = (i % 5 == 4) ? 0 : 0x7fffffff;
   for (int64_t i = prm.p0 + blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < prm.p0 + prm.pb; i += (int64_t)gridDim.x * blockDim.x) {
@@ -71,7 +71,7 @@ __global__ void __launch_bounds__(GB_SBLOCK_THREADS, 4) k_s1_propagate(const __g
   const int b = (int)(blockIdx.x % prm.s_nblk);
   if (!stream_point_active(prm, p)) return;
   const int tid = threadIdx.x, lane = tid & 31;
-  const int N = (int)prm.N, O = prm.O, t = prm.t;
+  const int N = (int)prm.N, ns = prm.n_slots, t = prm.t;
   {
     const uint32_t* src = reinterpret_cast<const uint32_t*>(prm.motion + p);
     uint32_t* dst = reinterpret_cast<uint32_t*>(&s_motion);
@@ -144,13 +144,13 @@ __global__ void __launch_bounds__(GB_SBLOCK_THREADS, 4) k_s1_propagate(const __g
       }
     }
     if (use_obs) {
-      for (int o = 0; o < O; ++o) {
-        const int64_t po = p * O + o;
-        if (prm.img[o] < 0 || !prm.mask[po]) continue;  // block-uniform
-        double* uv = prm.s_uv + po * 2 * (int64_t)N;
+      for (int sl = 0; sl < ns; ++sl) {
+        const int64_t po = p * prm.O + prm.obs[sl];
+        if (prm.img[sl] < 0 || !prm.mask[po]) continue;  // block-uniform
+        double* uv = prm.s_uv + (p * prm.slot_stride + sl) * 2 * (int64_t)N;
         double u[2], v[2];
 #pragma unroll
-        for (int q = 0; q < 2; ++q) project_fast(prm.cam[o], s[q][0], s[q][1], s[q][2], u[q], v[q]);
+        for (int q = 0; q < 2; ++q) project_fast(prm.cam[sl], s[q][0], s[q][1], s[q][2], u[q], v[q]);
         if (!vb) {
           u[1] = u[0];
           v[1] = v[0];
@@ -181,10 +181,10 @@ __global__ void __launch_bounds__(GB_SBLOCK_THREADS, 4) k_s1_propagate(const __g
         }
         // lanes 0..4 of a warp publish one value each; a tail warp without them lets its first lane do all five
         if ((mask & 0x1fu) == 0x1fu) {
-          if (lane < 5) atomicMin(&s_box[o][lane], mine);
+          if (lane < 5) atomicMin(&s_box[sl][lane], mine);
         } else if (lane == (__ffs(mask) - 1)) {
 #pragma unroll
-          for (int k = 0; k < 5; ++k) atomicMin(&s_box[o][k], red[k]);
+          for (int k = 0; k < 5; ++k) atomicMin(&s_box[sl][k], red[k]);
         }
         if (prm.io.dump_uv) {
           double* d = prm.io.dump_uv + (po * N + ia) * 2;
@@ -202,10 +202,9 @@ __global__ void __launch_bounds__(GB_SBLOCK_THREADS, 4) k_s1_propagate(const __g
   __shared__ unsigned s_or;
   const int any = (int)block_or(flags, &s_or);
   if (any && tid == 0) atomicOr(&prm.s_pflags[p], any);
-  if (use_obs && tid < O * 5) {
-    const int o = tid / 5, k = tid - o * 5;
-    const int64_t po = p * O + o;
-    if (prm.img[o] >= 0 && prm.mask[po]) atomicMin(&prm.s_ibox[po * 5 + k], s_box[o][k]);
+  if (use_obs && tid < ns * 5) {
+    const int sl = tid / 5, k = tid - sl * 5;
+    if (prm.img[sl] >= 0 && prm.mask[p * prm.O + prm.obs[sl]]) atomicMin(&prm.s_ibox[(p * prm.slot_stride + sl) * 5 + k], s_box[sl][k]);
   }
 }
 
@@ -224,25 +223,33 @@ __global__ void __launch_bounds__(GB_S2_THREADS, GB_S2_MINB) k_s2_surface(const 
   __shared__ double s_mm[GB_S2_THREADS / 32][4];
   __shared__ int s_box[4];
   __shared__ __align__(8) uint64_t s_tma_bar;
-  const int64_t po = prm.p0 * prm.O + blockIdx.x;
-  const int64_t p = po / prm.O;
-  const int o = (int)(po - p * prm.O);
+  const int64_t p = prm.p0 + blockIdx.x / prm.n_slots;
+  const int slot = (int)(blockIdx.x % prm.n_slots), o = prm.obs[slot];
+  const int64_t ps = p * prm.slot_stride + slot;  // the slot's scratch: cloud box, meta, projections, surface region
+  const int64_t po = p * prm.O + o;               // the observer's template, mask and outputs
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, t = prm.t;
-  int* meta = prm.s_meta + po * 8;
+  int* meta = prm.s_meta + ps * 8;
   // profiling aid (gb_track_step only): clock64() of thread 0 at the phase boundaries, window size, SM id
   long long* clk = prm.io.dump_clocks ? reinterpret_cast<long long*>(prm.io.dump_clocks) + po * 16 : nullptr;
   if (clk && tid == 0) clk[0] = clock64();
   if (tid == 0) meta[7] = 0;
   // every scalar the CTA branches on is requested before the first branch: one memory round trip instead of five
-  int* gib = prm.s_ibox + po * 5;
+  int* gib = prm.s_ibox + ps * 5;
   const int act = prm.s_act[p];
   const int seen = prm.mask[po];
   const int failed = prm.s_pflags[p];
   const int n_values = prm.tmpl_nvalues[po];
   const int my_ib = tid < 5 ? gib[tid] : 0;
   if (!(act & GB_ACT_ACTIVE) || prm.io.force_weights) return;
-  uint8_t* oflag = prm.obs_flags + ((int64_t)p * prm.T + t) * prm.O + o;
-  if (prm.img[o] < 0 || !seen) {
+  uint8_t* oflags = prm.obs_flags + ((int64_t)p * prm.T + t) * prm.O;
+  if (prm.n_slots < prm.O && slot == 0)  // observers without a slot have no frame at t: the first slot's CTA flags them
+    for (int k = tid; k < prm.O; k += blockDim.x) {
+      bool slotted = false;
+      for (int q = 0; q < prm.n_slots; ++q) slotted |= prm.obs[q] == k;
+      if (!slotted) oflags[k] = GB_OBS_NO_IMAGE;
+    }
+  uint8_t* oflag = oflags + o;
+  if (prm.img[slot] < 0 || !seen) {
     if (tid == 0) *oflag = GB_OBS_NO_IMAGE;
     return;
   }
@@ -265,7 +272,7 @@ __global__ void __launch_bounds__(GB_S2_THREADS, GB_S2_MINB) k_s2_surface(const 
   if (!nan_any && ((box_r - box_l) - prm.tile_w < prm.interp_cols + 2 || (box_b - box_t) - prm.tile_h < prm.interp_rows + 2)) {
     // cloud narrower than the spline degree (the integer box is at most 2 px wider than the exact extents): the reference
     // widens the box from the exact extents (tracker.py:584-594)
-    const double* uv = prm.s_uv + po * 2 * (int64_t)N;
+    const double* uv = prm.s_uv + ps * 2 * (int64_t)N;
     double mm[4] = {CUDART_INF, CUDART_INF, CUDART_INF, CUDART_INF};
     for (int i = tid; i < N; i += blockDim.x) {
       const double u = uv[i], v = uv[(int64_t)N + i];
@@ -310,7 +317,7 @@ __global__ void __launch_bounds__(GB_S2_THREADS, GB_S2_MINB) k_s2_surface(const 
     box_r = s_box[2];
     box_b = s_box[3];
   }
-  const int W = prm.cam[o].c.imgsz[0], H = prm.cam[o].c.imgsz[1];
+  const int W = prm.cam[slot].c.imgsz[0], H = prm.cam[slot].c.imgsz[1];
   const bool inframe = !nan_any && box_l >= 0 && box_l <= W && box_t >= 0 && box_t <= H && box_r >= 0 && box_r <= W &&
                        box_b >= 0 && box_b <= H;
   if (!inframe) {
@@ -335,10 +342,10 @@ __global__ void __launch_bounds__(GB_S2_THREADS, GB_S2_MINB) k_s2_surface(const 
   w.th = prm.tile_h;
   w.Mu = w.Su - w.tw + 1;
   w.Mv = w.Sv - w.th + 1;
-  w.dtype = prm.pixdtype[o];
-  w.nbins = w.dtype == GB_PIX_U8 ? 255 * prm.nchan[o] + 1 : w.Su * w.Sv;  // grey levels, or ranks of the window's pixels
+  w.dtype = prm.pixdtype[slot];
+  w.nbins = w.dtype == GB_PIX_U8 ? 255 * prm.nchan[slot] + 1 : w.Su * w.Sv;  // grey levels, or ranks of the window's pixels
   w.nvals = n_values;
-  w.tmap = fm.ok[o] ? &fm.map[o] : nullptr;
+  w.tmap = fm.ok[slot] ? &fm.map[slot] : nullptr;
   w.bar = &s_tma_bar;
   if (tid == 0) {
     *oflag = GB_OBS_USED;
@@ -355,7 +362,7 @@ __global__ void __launch_bounds__(GB_S2_THREADS, GB_S2_MINB) k_s2_surface(const 
       d[3] = box_b;
     }
   }
-  char* region = prm.s_surf + po * prm.surf_bytes;
+  char* region = prm.s_surf + ps * prm.surf_bytes;
   const int64_t need = tile_bytes_needed(w.Su, w.Sv, w.tw, w.th, w.nbins, w.nvals);
   const bool gen = !spline_is_hermite(w.ku, w.kv);  // degrees 2 / 4 / 5: coefficients solved with a work area behind the tile's data
   const bool ranked = w.dtype != GB_PIX_U8;          // frames other than uint8: the window's grey values, likewise
@@ -407,18 +414,18 @@ __global__ void __launch_bounds__(GB_S2_THREADS, GB_S2_MINB) k_s2_surface(const 
   if (planar) {
     TilePlanes pl;
     tile_carve_planar(reinterpret_cast<char*>(smem_raw), w, pl);
-    tile_prepare(prm.pixels[o], prm.pitch[o], prm.nchan[o], boxv, prm.tmpl_tile + po * ta, prm.tmpl_quantiles + po * ta,
+    tile_prepare(prm.pixels[slot], prm.pitch[slot], prm.nchan[slot], boxv, prm.tmpl_tile + po * ta, prm.tmpl_quantiles + po * ta,
                  prm.tmpl_values + po * ta, w, dump_search, prm.io.dump_cap, clk ? clk + 2 : nullptr);
     tile_finish_planar(w, pl, reinterpret_cast<float4*>(region), dump_sse, prm.io.dump_cap, clk ? clk + 2 : nullptr);
     if (clk && tid == 0) clk[5] = clock64();
   } else if (staged) {
-    tile_build_surface_staged(reinterpret_cast<char*>(smem_raw), region, prm.pixels[o], prm.pitch[o], prm.nchan[o], boxv,
+    tile_build_surface_staged(reinterpret_cast<char*>(smem_raw), region, prm.pixels[slot], prm.pitch[slot], prm.nchan[slot], boxv,
                               prm.tmpl_tile + po * ta, prm.tmpl_quantiles + po * ta, prm.tmpl_values + po * ta, w, dump_search, dump_sse,
                               prm.io.dump_cap, clk ? clk + 2 : nullptr);
     if (clk && tid == 0) clk[5] = clock64();
   } else {
     tile_carve(in_smem ? reinterpret_cast<char*>(smem_raw) : region, w);
-    tile_build_surface(prm.pixels[o], prm.pitch[o], prm.nchan[o], boxv, prm.tmpl_tile + po * ta, prm.tmpl_quantiles + po * ta,
+    tile_build_surface(prm.pixels[slot], prm.pitch[slot], prm.nchan[slot], boxv, prm.tmpl_tile + po * ta, prm.tmpl_quantiles + po * ta,
                        prm.tmpl_values + po * ta, w, dump_search, dump_sse, prm.io.dump_cap, clk ? clk + 2 : nullptr);
     if (clk && tid == 0) clk[5] = clock64();
     if (in_smem) {
@@ -506,6 +513,7 @@ __device__ __forceinline__ int count_positions_le_fast(double c, double u, doubl
 struct SurfaceRef {
   double sl, st, sr, sb, cu0, cv0, cu1, cv1, scale;
   const float4* herm;
+  double* sampled;  // gb_stage_io.dump_sampled row of the slot's observer
   int Mu, Mv, Mp, ok;
 };
 
@@ -555,15 +563,15 @@ __global__ void __launch_bounds__(GB_S3_MAX_THREADS, GB_S3_MINB) k_s3_weights(co
   const int64_t p = prm.p0 + blockIdx.y;
   const int b = (int)blockIdx.x;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int N = (int)prm.N, O = prm.O;
+  const int N = (int)prm.N, ns = prm.n_slots;
   const int act = prm.s_act[p];
   const int failed_at_t = prm.s_pflags[p];
   // every scalar of the prologue is requested before the first branch: one memory round trip instead of two
   int meta[8] = {0, 0, 0, 0, 0, 0, 0, 0};
   double du_t = 0.0, dv_t = 0.0, obs_scale = 0.0;
-  if (tid < O) {
-    const int64_t po = p * O + tid;
-    const int4 m0 = *reinterpret_cast<const int4*>(prm.s_meta + po * 8), m1 = *reinterpret_cast<const int4*>(prm.s_meta + po * 8 + 4);
+  if (tid < ns) {
+    const int64_t ps = p * prm.slot_stride + tid, po = p * prm.O + prm.obs[tid];
+    const int4 m0 = *reinterpret_cast<const int4*>(prm.s_meta + ps * 8), m1 = *reinterpret_cast<const int4*>(prm.s_meta + ps * 8 + 4);
     meta[0] = m0.x; meta[1] = m0.y; meta[2] = m0.z; meta[3] = m0.w;
     meta[4] = m1.x; meta[5] = m1.y; meta[6] = m1.z; meta[7] = m1.w;
     du_t = prm.tmpl_duv[po * 2];
@@ -578,9 +586,8 @@ __global__ void __launch_bounds__(GB_S3_MAX_THREADS, GB_S3_MINB) k_s3_weights(co
       uint32_t* dst = reinterpret_cast<uint32_t*>(&s_motion);
       for (int k = tid; k < (int)(sizeof(gb_motion) / 4); k += blockDim.x) dst[k] = src[k];
     }
-    if (tid < O) {
-      const int o = tid;
-      const int64_t po = p * O + o;
+    if (tid < ns) {
+      const int sl = tid;
       SurfaceRef r;
       r.ok = meta[7];
       r.Mu = meta[4];
@@ -596,8 +603,9 @@ __global__ void __launch_bounds__(GB_S3_MAX_THREADS, GB_S3_MINB) k_s3_weights(co
       r.cu1 = add(r.cu0, (double)(r.Mu - 1));
       r.cv1 = add(r.cv0, (double)(r.Mv - 1));
       r.scale = obs_scale;
-      r.herm = reinterpret_cast<const float4*>(prm.s_surf + po * prm.surf_bytes);
-      s_ref[o] = r;
+      r.herm = reinterpret_cast<const float4*>(prm.s_surf + (p * prm.slot_stride + sl) * prm.surf_bytes);
+      r.sampled = prm.io.dump_sampled ? prm.io.dump_sampled + (p * prm.O + prm.obs[sl]) * N : nullptr;
+      s_ref[sl] = r;
     }
   }
   __syncthreads();
@@ -607,7 +615,7 @@ __global__ void __launch_bounds__(GB_S3_MAX_THREADS, GB_S3_MINB) k_s3_weights(co
     // no image likelihood at this time and a motion model without one: the reference leaves the weights of the last
     // resampling in place (tracker.py:146-149); they live in weight_state (ones after initialisation)
     bool any_ok = false;
-    for (int o = 0; o < O; ++o) any_ok |= s_ref[o].ok != 0;
+    for (int sl = 0; sl < ns; ++sl) any_ok |= s_ref[sl].ok != 0;
     if (!any_ok && prm.weight_state) fw = prm.weight_state + (int64_t)p * N;
   }
   const bool vec = (N & 1) == 0;
@@ -626,10 +634,11 @@ __global__ void __launch_bounds__(GB_S3_MAX_THREADS, GB_S3_MINB) k_s3_weights(co
       w[1] = vb ? fw[ia + 1] : 0.0;
     } else {
       double ll[2] = {0.0, 0.0};
-      for (int o = 0; o < O; ++o) {
-        const SurfaceRef& r = s_ref[o];
+      // observers in slot order, which is ascending observer order: the reference's order of the sum
+      for (int sl = 0; sl < ns; ++sl) {
+        const SurfaceRef& r = s_ref[sl];
         if (!r.ok) continue;
-        const double* uv = prm.s_uv + (p * O + o) * 2 * (int64_t)N;
+        const double* uv = prm.s_uv + (p * prm.slot_stride + sl) * 2 * (int64_t)N;
         double u[2], v[2];
         if (vec) {
           const double2 a = *reinterpret_cast<const double2*>(uv + ia), c = *reinterpret_cast<const double2*>(uv + (int64_t)N + ia);
@@ -650,7 +659,7 @@ __global__ void __launch_bounds__(GB_S3_MAX_THREADS, GB_S3_MINB) k_s3_weights(co
           const double val = gen ? (double)bspline_eval(r.herm, r.Mp, r.Mu, r.Mv, u[q] - r.cu0, v[q] - r.cv0, prm.interp_cols, prm.interp_rows)
                                  : (double)hermite_eval_sat(r.herm, r.Mp, r.Mu, r.Mv, u[q] - r.cu0, v[q] - r.cv0, lin_u, lin_v);
           ll[q] = add(ll[q], mul(val, r.scale));
-          if (prm.io.dump_sampled && (q == 0 || vb)) prm.io.dump_sampled[(p * O + o) * N + ia + q] = val;
+          if (prm.io.dump_sampled && (q == 0 || vb)) r.sampled[ia + q] = val;
         }
       }
 #pragma unroll
@@ -863,7 +872,7 @@ __global__ void __launch_bounds__(GB_SBLOCK_THREADS, 4) k_s4c_scan(const __grid_
   }
   const double off = block_exclusive_offset(tsum, s_warp);
   const double prefix = s_pref[0], total = s_pref[1];
-  double* cdf = prm.s_uv + p * prm.O * 2 * (int64_t)N;
+  double* cdf = prm.s_uv + p * prm.slot_stride * 2 * (int64_t)N;
 #pragma unroll
   for (int q = 0; q < PPT; ++q) {
     const int k = k0 + q;
@@ -949,7 +958,7 @@ __global__ void __launch_bounds__(GB_SBLOCK_THREADS) k_s4r_residual(const __grid
   if (!stream_point_active(prm, p) || prm.s_pflags[p] != 0) return;
   const int tid = threadIdx.x, N = (int)prm.N, t = prm.t;
   const double* w = prm.s_w + (int64_t)p * N;
-  double* cs = prm.s_uv + p * prm.O * 2 * (int64_t)N;    // [N] normalised weights, then residuals, then their cumulative sum
+  double* cs = prm.s_uv + p * prm.slot_stride * 2 * (int64_t)N;    // [N] normalised weights, then residuals, then their cumulative sum
   int* ridx = reinterpret_cast<int*>(cs + N);           // [N] parent of every child
   int* cum = ridx + N;                                  // [N] inclusive prefix of the repetitions
   if (tid == 0) s_tot[0] = numpy_pairwise_sum([w](int64_t i) { return w[i]; }, 0, N);
@@ -1030,7 +1039,7 @@ __global__ void __launch_bounds__(GB_SBLOCK_THREADS, 4) k_s4c_gather(const __gri
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, t = prm.t;
   const int N = (int)prm.N;
   const int base = b * prm.s_block, end = min(N, base + prm.s_block);
-  const double* cdf = prm.s_uv + p * prm.O * 2 * (int64_t)N;
+  const double* cdf = prm.s_uv + p * prm.slot_stride * 2 * (int64_t)N;
   const double* ev = prm.s_ev + p * 6 * (int64_t)N;
   const double* wsrc = prm.s_w + (int64_t)p * N;
   const StratifiedDraws draws = stratified_draws(prm, p, t);  // one uniform per child, like the stratified resampler
@@ -1161,7 +1170,7 @@ __global__ void k_s0p_activity(const __grid_constant__ StepParams prm) {
 
 // Start of a gb_track: empty cloud boxes, no failure flags in either parity.
 __global__ void k_s0p_reset(const __grid_constant__ StepParams prm) {
-  const int64_t lo5 = prm.p0 * prm.O * 5, n = prm.pb * prm.O * 5;
+  const int64_t lo5 = prm.p0 * prm.slot_stride * 5, n = prm.pb * prm.slot_stride * 5;
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
     prm.s_ibox[lo5 + i] = (i % 5 == 4) ? 0 : 0x7fffffff;
   for (int64_t i = prm.p0 + blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < prm.p0 + prm.pb; i += (int64_t)gridDim.x * blockDim.x) {
@@ -1222,7 +1231,7 @@ __global__ void __launch_bounds__(GB_S4P_THREADS, GB_S4P_MINB) k_s4p_resample_pr
   const int64_t p = prm.p0 + blockIdx.y;  // grid: (blocks of a point, points of the batch)
   const int b = (int)blockIdx.x;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, t = prm.t;
-  const int N = (int)prm.N, O = prm.O;
+  const int N = (int)prm.N, ns = nxt.n_slots;  // slots of t + 1, where the children are projected
   const int base = b * prm.s_block;
   const int n_here = max(0, min(N, base + prm.s_block) - base);  // parents of this CTA (<= CAP)
   const double* wsrc = prm.s_w + (int64_t)p * N + base;
@@ -1255,7 +1264,7 @@ __global__ void __launch_bounds__(GB_S4P_THREADS, GB_S4P_MINB) k_s4p_resample_pr
   uint8_t mask_byte = 0;
   if (tid < (int)(sizeof(gb_motion) / 4)) motion_word = reinterpret_cast<const uint32_t*>(prm.motion + p)[tid];
   if (tid >= 64 && tid < 70) ref_word = prm.s_ref[p * 6 + (tid - 64)];
-  if (tid >= 96 && tid < 96 + O) mask_byte = prm.mask[p * O + (tid - 96)];
+  if (tid >= 96 && tid < 96 + ns) mask_byte = prm.mask[p * prm.O + nxt.obs[tid - 96]];
   if (tid >= 128 && tid < 134) {
     // written by k_s3b_publish: prefix of this and the next CTA, total, 1 / total, the uniform draw, 1 / N
     const int k = tid - 128;
@@ -1276,7 +1285,7 @@ __global__ void __launch_bounds__(GB_S4P_THREADS, GB_S4P_MINB) k_s4p_resample_pr
   if (tid < (int)(sizeof(gb_motion) / 4)) reinterpret_cast<uint32_t*>(&s_motion)[tid] = motion_word;
   if (propagate && tid < GB_MAX_OBS * 5) s_box[tid / 5][tid % 5] = (tid % 5 == 4) ? 0 : 0x7fffffff;
   if (tid >= 64 && tid < 70) s_refv[tid - 64] = ref_word;
-  if (tid >= 96 && tid < 96 + O) s_mask[tid - 96] = mask_byte;
+  if (tid >= 96 && tid < 96 + ns) s_mask[tid - 96] = mask_byte;
   if (tid >= 128 && tid < 134) s_pre6[tid - 128] = ref_word;
   __syncthreads();
   if (bulk) {
@@ -1391,9 +1400,9 @@ __global__ void __launch_bounds__(GB_S4P_THREADS, GB_S4P_MINB) k_s4p_resample_pr
     ibx[o][0] = ibx[o][1] = ibx[o][2] = ibx[o][3] = 0x7fffffff;
     ibx[o][4] = 0;
   }
-  unsigned obs_on = 0;  // observers that see this point at t + 1 (block-uniform)
+  unsigned obs_on = 0;  // slots of t + 1 whose observer sees this point (block-uniform)
   if (propagate)
-    for (int o = 0; o < O; ++o)
+    for (int o = 0; o < ns; ++o)
       if (nxt.img[o] >= 0 && s_mask[o]) obs_on |= 1u << o;
   int carry = 0;  // parent of the last child of the previous chunk
   for (int Jc = J0; Jc < J1; Jc += CAP) {
@@ -1479,17 +1488,17 @@ __global__ void __launch_bounds__(GB_S4P_THREADS, GB_S4P_MINB) k_s4p_resample_pr
         // the first two observers are unrolled: their camera operands come straight from the constant bank
 #pragma unroll
         for (int o = 0; o < 2; ++o) {
-          if (o >= O) break;
+          if (o >= ns) break;
           if (!(obs_on >> o & 1)) continue;
-          const int64_t po = p * O + o;
+          const int64_t po = p * prm.slot_stride + o;
           int e[5];
           s4p_project_child(nxt.cam[o], s, prm.s_uv + po * 2 * (int64_t)N, N, j, hw, hh, e);
 #pragma unroll
           for (int k = 0; k < 5; ++k) ibx[o][k] = min(ibx[o][k], e[k]);
         }
-        for (int o = 2; o < O; ++o) {
+        for (int o = 2; o < ns; ++o) {
           if (!(obs_on >> o & 1)) continue;
-          const int64_t po = p * O + o;
+          const int64_t po = p * prm.slot_stride + o;
           int e[5];
           s4p_project_child(nxt.cam[o], s, prm.s_uv + po * 2 * (int64_t)N, N, j, hw, hh, e);
 #pragma unroll
@@ -1503,7 +1512,7 @@ __global__ void __launch_bounds__(GB_S4P_THREADS, GB_S4P_MINB) k_s4p_resample_pr
     // cloud boxes of time t + 1: registers -> warp -> shared -> global
 #pragma unroll
     for (int o = 0; o < 2; ++o) {
-      if (o >= O) break;
+      if (o >= ns) break;
       int mine = 0x7fffffff;
 #pragma unroll
       for (int k = 0; k < 5; ++k) {
@@ -1514,9 +1523,9 @@ __global__ void __launch_bounds__(GB_S4P_THREADS, GB_S4P_MINB) k_s4p_resample_pr
     }
     const int any = (int)block_or(flags, &s_or);  // also orders the shared-memory atomics above
     if (any && tid == 0) atomicOr(&prm.s_pflags_next[p], any);
-    if (tid < O * 5) {
+    if (tid < ns * 5) {
       const int o = tid / 5, k = tid - o * 5;
-      const int64_t po = p * O + o;
+      const int64_t po = p * prm.slot_stride + o;
       if (obs_on >> o & 1) atomicMin(&prm.s_ibox[po * 5 + k], s_box[o][k]);
     }
   }

@@ -249,18 +249,41 @@ def lower_models(models, viewshed=None):
     return table_m, table, view
 
 
+def observer_slots(image_index: np.ndarray) -> int:
+    """Most observers with a matched image at one time in a (T, O) grid of image indices (-1 = no match).  A time step's
+    cameras are kernel launch parameters, so this count, not the number of observers, is bounded by ``GB_MAX_OBS``."""
+    return int((np.asarray(image_index) >= 0).sum(axis=1).max(initial=0))
+
+
+def check_observer_slots(image_index: np.ndarray) -> None:
+    """Raise ``NotImplementedError`` at the first time with more than ``GB_MAX_OBS`` observers with a matched image."""
+    active = (np.asarray(image_index) >= 0).sum(axis=1)
+    if active.max(initial=0) > _lib.GB_MAX_OBS:
+        t = int(np.argmax(active > _lib.GB_MAX_OBS))
+        raise NotImplementedError(f"{int(active[t])} observers have an image at time index {t}: the device kernels take at most "
+                                  f"{_lib.GB_MAX_OBS} observers with a frame at the same time")
+
+
+def plan_slots(image_index: np.ndarray) -> int:
+    """Observer slots of a launch plan: one per observer in a call of up to ``GB_MAX_OBS`` observers, otherwise one per
+    observer with a frame at the same time (at least one)."""
+    O = np.shape(image_index)[1]
+    return O if O <= _lib.GB_MAX_OBS else max(observer_slots(image_index), 1)
+
+
 def plan_template_flags(tw: int, th: int) -> int:
     """The plan flag a ``tw`` x ``th`` template needs: templates above 1024 pixels are planned with their own organisation."""
     return _lib.GB_PLAN_LARGE_TEMPLATES if tw * th > _lib.GB_MAX_TEMPLATE else 0
 
 
 def session_bytes(lib, mode: int, cluster: int, P: int, N: int, T: int, O: int, tw: int, th: int, return_covariances: bool,
-                  return_particles: bool, window_margin: int = _lib.GB_WINDOW_MARGIN) -> int:
+                  return_particles: bool, window_margin: int = _lib.GB_WINDOW_MARGIN, slots: Optional[int] = None) -> int:
     """Device memory one :class:`Session` of ``P`` points allocates (the frames excluded): two particle-state buffers,
-    the weights, the launch plan's scratch, templates and result blocks."""
+    the weights, the launch plan's scratch, templates and result blocks.  ``slots``: the plan's observer slots
+    (:func:`plan_slots`; default ``O``), which size the scratch; templates and results are sized by ``O``."""
     plan = _lib.gb_plan()
     flags = int(cluster) | plan_template_flags(tw, th)
-    _lib.check(lib.gb_step_plan_ex(N, tw, th, P, O, flags, mode, int(window_margin), C.byref(plan)))
+    _lib.check(lib.gb_step_plan_ex(N, tw, th, P, O if slots is None else int(slots), flags, mode, int(window_margin), C.byref(plan)))
     per_point = 2 * 48 * N + 8 * N                      # state_a, state_b, weight_state
     per_point += 3 * O * tw * th * 8 + O * 40           # templates
     per_point += T * ((36 if return_covariances else 6) + 6) * 8 + T * O * 9 + 16  # moments, flags, window sizes, status
@@ -298,8 +321,7 @@ class Session:
         N = self.N = int(models[0].n)
         if any(int(m.n) != N for m in models):
             raise ValueError("one device session holds models with the same number of particles (Tracker.track groups them)")
-        if O > _lib.GB_MAX_OBS:
-            raise NotImplementedError(f"at most {_lib.GB_MAX_OBS} observers per track() call (GB_MAX_OBS, include/glimpse_b200.h)")
+        check_observer_slots(image_index)
         self.tw, self.th = (int(v) for v in tile_size)
         self.return_covariances, self.return_particles = return_covariances, return_particles
         self.image_index = np.ascontiguousarray(image_index, dtype=np.int32)
@@ -315,7 +337,7 @@ class Session:
                 window_margin = getattr(tracker, "window_margin", _lib.GB_WINDOW_MARGIN)
             flags = _lib.GB_PLAN_RANKED_FRAMES if frames_need_ranks(tracker.observers, self.image_index) else 0
             flags |= plan_template_flags(self.tw, self.th)
-            _lib.check(self.lib.gb_step_plan_ex(N, self.tw, self.th, P, O, flags, mode, int(window_margin),
+            _lib.check(self.lib.gb_step_plan_ex(N, self.tw, self.th, P, plan_slots(self.image_index), flags, mode, int(window_margin),
                                                 C.byref(self.plan)))
             self.h2d = 0
             # the first two frames' uploads start right away (the first kernels wait for them); the other big copies are

@@ -50,7 +50,7 @@ def pairwise_distance_datetimes(x, y) -> np.ndarray:
     return np.abs(xs[:, None] - ys[None, :])
 
 
-from .session import point_span  # noqa: E402,F401  (re-exported)
+from .session import check_observer_slots, point_span  # noqa: E402,F401  (point_span: re-exported)
 
 
 def highpass_params(highpass: dict):
@@ -127,7 +127,11 @@ def shard_bounds(n_items: int, world_size: int, rank: int):
 
 
 class Tracker:
-    """Estimate the trajectory of world points through time (reference ``tracker.py:21-70``)."""
+    """Estimate the trajectory of world points through time (reference ``tracker.py:21-70``).
+
+    ``observers`` may be any number of stations (a station that was moved or re-calibrated is a new one), with at most eight
+    observers with a frame at the same time: ``track`` raises ``NotImplementedError`` naming the first time index with more,
+    before any device work (a time step's cameras are kernel launch parameters)."""
 
     def __init__(
         self,
@@ -277,6 +281,7 @@ class Tracker:
         observer_mask = np.asarray(observer_mask, dtype=bool).reshape(ntracks, len(self.observers))
         matching_images = self.match_datetimes(datetimes=datetimes, maxdt=maxdt)
         image_index = np.array([[-1 if v is None else int(v) for v in row] for row in matching_images], dtype=np.int32)
+        check_observer_slots(image_index)
         unit = time_unit.total_seconds()
         taus = np.array([dt.total_seconds() / unit for dt in np.diff(datetimes)], dtype=float)
 
@@ -544,7 +549,8 @@ class Tracker:
                         pass  # size unknown before the frame is read: the 10 % margin has to cover it
         mode = _lib.GB_MODE_STREAM
         shape = dict(N=int(models[0].n), T=image_index.shape[0], O=image_index.shape[1], tw=tile_size[0], th=tile_size[1],
-                     return_covariances=return_covariances, return_particles=return_particles, window_margin=int(self.window_margin))
+                     return_covariances=return_covariances, return_particles=return_particles, window_margin=int(self.window_margin),
+                     slots=_session.plan_slots(image_index))
         lib = _lib.load()
         # the common case costs no driver call: a track needing less than a quarter of the device is not measured against
         # the free memory (cudaMemGetInfo takes from a fraction of a millisecond to several)

@@ -231,8 +231,9 @@ typedef struct gb_plan {
   int32_t mode;             /* GB_MODE_* */
   int32_t stream_block;     /* GB_MODE_STREAM: particles per CTA of the per-particle kernels (even, <= 768) */
   int32_t stream_nblk;      /* GB_MODE_STREAM: CTAs per point */
-  int32_t n_observers;
-  int64_t surf_bytes;       /* GB_MODE_STREAM: bytes of the per-(point, observer) surface region */
+  int32_t n_observers;      /* observer slots (1-8): one per observer in a call of up to GB_MAX_OBSERVERS observers, otherwise
+                             * at least the most observers with a frame at the same time */
+  int64_t surf_bytes;       /* GB_MODE_STREAM: bytes of the per-(point, slot) surface region */
   int32_t stream_batch;     /* GB_MODE_STREAM: points per batch (<= 65535) */
   int32_t stream_slots;     /* GB_MODE_STREAM: batches in flight (side streams / scratch slots) */
 } gb_plan;
@@ -244,11 +245,16 @@ typedef struct gb_plan {
 #define GB_HP_MIRROR 3
 #define GB_HP_WRAP 4
 
-/* Observers per gb_track call: the cameras of one time step travel as kernel launch parameters (operands straight from the
- * constant bank), which bounds their number.  (The reference has no limit; its use cases have one to three stations.) */
+/* Observers with a frame at the same time: the cameras of one time step travel as kernel launch parameters (operands straight
+ * from the constant bank), which bounds their number.  A call may have any number of observers (d.O).  Up to
+ * GB_MAX_OBSERVERS observers, every observer has a slot of its own (plan n_observers = O); beyond, each time step gives its
+ * observers with a frame (image_index_host >= 0) the slots in ascending observer order, and the plan needs as many slots as
+ * the most such observers at one time.  gb_track* return GB_E_RESOURCE when more than GB_MAX_OBSERVERS observers have a frame
+ * at one time, GB_E_INVALID for a plan with fewer slots than that.  Templates, masks, obs_flags, window_stats and the
+ * gb_stage_io dumps stay indexed by observer. */
 #define GB_MAX_OBSERVERS 8
 
-/* Size a launch plan for N particles per point, a w x h template, P points and O observers.
+/* Size a launch plan for N particles per point, a w x h template, P points and n_observers observer slots (see GB_MAX_OBSERVERS).
  * `flags`: GB_PLAN_RANKED_FRAMES = some frame is not uint8 (the surface regions are sized for rank histograms of the largest window);
  * GB_PLAN_LARGE_TEMPLATES = admit templates above 1024 pixels, up to 128 pixels a side (without it they return GB_E_RESOURCE;
  * with it a template above 1024 pixels and above 128 pixels a side still does).  The kernels choose their path from the template
