@@ -1814,18 +1814,30 @@ int gb_viewshed(const double* z, int32_t nx, int32_t ny, const double* x_centres
     q.corr_c2 = 2.0 * corr[0];
   }
   q.visible = visible;
+  // GB_VS_RING_CAP (test hook): a lower ring capacity sends small rasters through the large-ring sort, merge and search; the
+  // result is the same
+  q.cap = GB_VS_MAX_RING;
+  if (const char* e = getenv("GB_VS_RING_CAP")) {
+    const int c = atoi(e);
+    q.cap = c < 1 ? 1 : c > GB_VS_MAX_RING ? GB_VS_MAX_RING : c;
+  }
   cudaStream_t s = (cudaStream_t)stream;
   const int sort_smem = GB_VS_MAX_RING * 12, sweep_smem = (GB_VS_MAX_RING + 2) * 8;
   // (per device and cheap: set on every call rather than remembered per process)
   GB_CUDA(cudaFuncSetAttribute(k_vs_sort, cudaFuncAttributeMaxDynamicSharedMemorySize, sort_smem));
-  GB_CUDA(cudaFuncSetAttribute(k_vs_sweep, cudaFuncAttributeMaxDynamicSharedMemorySize, sweep_smem));
+  GB_CUDA(cudaFuncSetAttribute(k_vs_sweep<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, sweep_smem));
+  GB_CUDA(cudaFuncSetAttribute(k_vs_sweep<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, sweep_smem));
   k_vs_init<<<grid_for(max_rings + 1, 256), 256, 0, s>>>(q);
   k_vs_cells<<<grid_for(n, 256), 256, 0, s>>>(q);
   k_vs_count<<<grid_for(n, 256), 256, 0, s>>>(q);
   k_vs_scan<<<1, 1024, 0, s>>>(q);
   k_vs_scatter<<<grid_for(n, 256), 256, 0, s>>>(q);
   k_vs_sort<<<max_rings, GB_VS_SORT_THREADS, sort_smem, s>>>(q);
-  k_vs_sweep<<<1, GB_VS_SWEEP_THREADS, sweep_smem, s>>>(q);
+  // enough passes for a ring of all n cells; a pass no ring needs returns at once (the ring sizes stay on the device)
+  for (int pass = 0, passes = vs_merge_passes((int)n, q.cap); pass < passes; ++pass)
+    k_vs_merge<<<grid_for(n, 256), 256, 0, s>>>(q, pass);
+  k_vs_sweep<false><<<1, GB_VS_SWEEP_THREADS, sweep_smem, s>>>(q);  // (one of the two returns at once)
+  k_vs_sweep<true><<<1, GB_VS_SWEEP_THREADS, sweep_smem, s>>>(q);
   GB_CUDA(cudaGetLastError());
   return GB_OK;
 }

@@ -7,31 +7,38 @@
 //   k_vs_cells    one thread per cell: ring, heading, ratio; range of the ring numbers
 //   k_vs_count    cells per ring          k_vs_scan   ring offsets (one CTA)
 //   k_vs_scatter  cells into their ring's bucket (any order)
-//   k_vs_sort     one CTA per ring: bitonic sort of (heading, cell index) in shared memory = np.lexsort((heading, ring))
+//   k_vs_sort     one CTA per ring: bitonic sort of (heading, cell index) in shared memory = np.lexsort((heading, ring)); a
+//                 ring of more than C cells (the capacity, GB_VS_MAX_RING) is sorted in chunks of C cells
+//   k_vs_merge    rings of more than C cells only: pass p merges the sorted runs of C * 2^p cells pairwise, between the bucket
+//                 arrays (b_head, b_idx) and the dead heading / ring arrays; a ring of m cells takes ceil(log2(m / C)) passes
+//                 and ends in the second pair when that count is odd
 //   k_vs_sweep    one CTA walks the rings in order; its threads share a ring's cells; the horizon of the previous ring =
 //                 headings modulo 2 pi in increasing order with the two wrap-around entries np.interp adds (in shared memory:
-//                 the binary search reads them ~14 times per cell) and the running maxima (double-buffered in global memory)
+//                 the binary search reads them ~14 times per cell; after a ring of more than C cells only every k-th of them,
+//                 and the search ends in a k-entry segment of the global copy) and the running maxima (double-buffered in global
+//                 memory)
 // Everything but the heading (atan2) is IEEE-exact arithmetic in the reference's order, so the result equals the reference's
 // unless a ratio sits within rounding of the interpolated horizon.
 // (included by glimpse_b200.cu inside namespace gb, after common.cuh)
 #pragma once
 
-#define GB_VS_MAX_RING 16384  // cells per ring the sort holds in shared memory (a full circle of radius ~2 600 cells)
+#define GB_VS_MAX_RING 16384  // C: cells per ring the sort holds in shared memory (a full circle of radius ~2 600 cells)
 #define GB_VS_SORT_THREADS 1024
 #define GB_VS_SWEEP_THREADS 1024
 
+// Work buffer: 64 bytes per cell + 12 per ring + 2 KB of alignment and header (viewshed_layout).
 struct ViewshedWork {
-  int32_t* head;     // [8] status, rmin, rmax, -, ...
-  int32_t* ring;     // [n]
-  double* heading;   // [n]
+  int32_t* head;     // [8] status, rmin, rmax, largest ring over C cells (0: none), ...
+  int32_t* ring;     // [n]  (after the scatter: the merge passes' second index buffer)
+  double* heading;   // [n]  (after the sort: the merge passes' second heading buffer)
   double* ratio;     // [n]
   int32_t* count;    // [R + 1]
   int32_t* start;    // [R + 1]
   int32_t* fill;     // [R + 1]
   double* b_head;    // [n] bucketed, then sorted, headings
   int32_t* b_idx;    // [n] ... and their cells
-  double* hx[2];     // [0]: a ring's abscissae (headings mod 2 pi, wrapped) before they are copied into the sweep's shared memory
-  double* hf[2];     // [GB_VS_MAX_RING + 2] horizon ordinates (running maximum of the ratio)
+  double* hx[2];     // [n + 2] a ring's abscissae (headings mod 2 pi, wrapped), double-buffered: the previous ring's stay readable
+  double* hf[2];     // [n + 2] horizon ordinates (running maximum of the ratio)
 };
 
 __host__ __device__ inline int64_t vs_align(int64_t b) { return (b + 255) / 256 * 256; }
@@ -53,9 +60,9 @@ __host__ inline int64_t viewshed_layout(int64_t n, int64_t R, unsigned char* bas
   p = take((R + 1) * 4); if (w) w->fill = reinterpret_cast<int32_t*>(p);
   p = take(n * 8); if (w) w->b_head = reinterpret_cast<double*>(p);
   p = take(n * 4); if (w) w->b_idx = reinterpret_cast<int32_t*>(p);
-  for (int k = 0; k < 2; ++k) {
-    p = take((GB_VS_MAX_RING + 2) * 8); if (w) w->hx[k] = reinterpret_cast<double*>(p);
-    p = take((GB_VS_MAX_RING + 2) * 8); if (w) w->hf[k] = reinterpret_cast<double*>(p);
+  for (int k = 0; k < 2; ++k) {  // (a ring holds at most n cells)
+    p = take((n + 2) * 8); if (w) w->hx[k] = reinterpret_cast<double*>(p);
+    p = take((n + 2) * 8); if (w) w->hf[k] = reinterpret_cast<double*>(p);
   }
   return off;
 }
@@ -65,6 +72,7 @@ struct ViewshedParams {
   const double* xc;  // [nx] cell-centre x in array order
   const double* yc;  // [ny]
   int32_t nx, ny, R, has_corr;
+  int32_t cap;       // C, 1..GB_VS_MAX_RING: rings of more cells take the chunked sort, the merge and the sampled search
   double ox, oy, oz, inv_cell, corr_c1, corr_c2;
   ViewshedWork w;
   uint8_t* visible;
@@ -76,6 +84,7 @@ __global__ void k_vs_init(const __grid_constant__ ViewshedParams q) {
     q.w.head[0] = 0;
     q.w.head[1] = 0x7fffffff;
     q.w.head[2] = -1;
+    q.w.head[3] = 0;
   }
   if (i <= q.R) {
     q.w.count[i] = 0;
@@ -146,7 +155,7 @@ __global__ void k_vs_scan(const __grid_constant__ ViewshedParams q) {
     for (int k = 0; k < warp; ++k) off += s_warp[k];
     if (i < span) {
       q.w.start[i] = off + incl - v;
-      if (v > GB_VS_MAX_RING) q.w.head[0] = 3;  // a ring larger than the sort's shared memory
+      if (v > q.cap) atomicMax(&q.w.head[3], v);  // a ring for the merge passes
     }
     __syncthreads();
     if (tid == blockDim.x - 1) s_carry = off + incl;
@@ -172,65 +181,158 @@ __device__ __forceinline__ uint64_t vs_orderable(double v) {
   return (b >> 63) ? ~b : (b | 0x8000000000000000ull);
 }
 
-// One CTA per ring: (heading, cell) ascending — np.lexsort((heading, ring)) is stable, so equal headings keep cell order.
+// One CTA per ring: (heading, cell) ascending — np.lexsort((heading, ring)) is stable, so equal headings keep cell order.  A
+// ring of more than q.cap cells is sorted in runs of q.cap cells, which k_vs_merge joins.
 __global__ void __launch_bounds__(GB_VS_SORT_THREADS) k_vs_sort(const __grid_constant__ ViewshedParams q) {
   extern __shared__ __align__(16) unsigned char vs_raw[];
   if (q.w.head[0] != 0) return;
   const int b = blockIdx.x;
   if (b > q.w.head[2] - q.w.head[1]) return;
-  const int m = q.w.count[b];
-  const int s0 = q.w.start[b];
-  if (m <= 1 || m > GB_VS_MAX_RING) {
+  const int m_ring = q.w.count[b];
+  if (m_ring <= 1) {
     // (the sweep wants the number of negative headings of every ring: they follow the others modulo 2 pi)
-    if (threadIdx.x == 0) q.w.fill[b] = (m == 1 && q.w.b_head[s0] < 0.0) ? 1 : 0;
+    if (threadIdx.x == 0) q.w.fill[b] = (m_ring == 1 && q.w.b_head[q.w.start[b]] < 0.0) ? 1 : 0;
     return;
   }
-  int cap = 1;
-  while (cap < m) cap <<= 1;
-  uint64_t* key = reinterpret_cast<uint64_t*>(vs_raw);
-  uint32_t* idx = reinterpret_cast<uint32_t*>(key + cap);
-  for (int i = threadIdx.x; i < cap; i += blockDim.x) {
-    key[i] = i < m ? vs_orderable(q.w.b_head[s0 + i]) : ~0ull;
-    idx[i] = i < m ? (uint32_t)q.w.b_idx[s0 + i] : 0xffffffffu;
-  }
-  __syncthreads();
-  for (int k = 2; k <= cap; k <<= 1) {
-    for (int j = k >> 1; j > 0; j >>= 1) {
-      for (int i = threadIdx.x; i < cap; i += blockDim.x) {
-        const int l = i ^ j;
-        if (l > i) {
-          const bool up = (i & k) == 0;
-          const uint64_t ka = key[i], kb = key[l];
-          const uint32_t ia = idx[i], ib = idx[l];
-          const bool greater = ka > kb || (ka == kb && ia > ib);
-          if (greater == up) {
-            key[i] = kb;
-            key[l] = ka;
-            idx[i] = ib;
-            idx[l] = ia;
+  int n_neg = 0;  // (thread 0's)
+  for (int c0 = 0; c0 < m_ring; c0 += q.cap) {
+    const int m = min(m_ring - c0, q.cap);
+    const int s0 = q.w.start[b] + c0;
+    int cap = 1;
+    while (cap < m) cap <<= 1;
+    uint64_t* key = reinterpret_cast<uint64_t*>(vs_raw);
+    uint32_t* idx = reinterpret_cast<uint32_t*>(key + cap);
+    if (c0 > 0) __syncthreads();  // the previous run's keys are read
+    for (int i = threadIdx.x; i < cap; i += blockDim.x) {
+      key[i] = i < m ? vs_orderable(q.w.b_head[s0 + i]) : ~0ull;
+      idx[i] = i < m ? (uint32_t)q.w.b_idx[s0 + i] : 0xffffffffu;
+    }
+    __syncthreads();
+    for (int k = 2; k <= cap; k <<= 1) {
+      for (int j = k >> 1; j > 0; j >>= 1) {
+        for (int i = threadIdx.x; i < cap; i += blockDim.x) {
+          const int l = i ^ j;
+          if (l > i) {
+            const bool up = (i & k) == 0;
+            const uint64_t ka = key[i], kb = key[l];
+            const uint32_t ia = idx[i], ib = idx[l];
+            const bool greater = ka > kb || (ka == kb && ia > ib);
+            if (greater == up) {
+              key[i] = kb;
+              key[l] = ka;
+              idx[i] = ib;
+              idx[l] = ia;
+            }
           }
         }
+        __syncthreads();
       }
-      __syncthreads();
+    }
+    for (int i = threadIdx.x; i < m; i += blockDim.x) {
+      const uint32_t c = idx[i];
+      q.w.b_idx[s0 + i] = (int)c;
+      q.w.b_head[s0 + i] = q.w.heading[c];
+    }
+    if (threadIdx.x == 0) {
+      // negative headings come first: their orderable keys have the top bit clear
+      int lo = 0, hi = m;  // first i with the top bit set
+      while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (key[mid] >> 63) hi = mid; else lo = mid + 1;
+      }
+      n_neg += lo;
     }
   }
-  for (int i = threadIdx.x; i < m; i += blockDim.x) {
-    const uint32_t c = idx[i];
-    q.w.b_idx[s0 + i] = (int)c;
-    q.w.b_head[s0 + i] = q.w.heading[c];
-  }
-  if (threadIdx.x == 0) {
-    // negative headings come first: their orderable keys have the top bit clear
-    int lo = 0, hi = m;  // first i with the top bit set
-    while (lo < hi) {
+  if (threadIdx.x == 0) q.w.fill[b] = n_neg;
+}
+
+// Merge passes of the rings of more than q.cap cells: k_vs_sort left runs of q.cap cells; pass p merges the runs of
+// q.cap * 2^p cells pairwise.  Even passes read (b_head, b_idx) and write (heading, ring), odd passes the other way round, so a
+// ring ends in the second pair when its number of passes (vs_merge_passes) is odd.  The keys (heading, cell) are all distinct,
+// so a cell's place is its place in its run plus the number of cells of the partner run with a smaller key.
+__host__ __device__ __forceinline__ int vs_merge_passes(int m, int cap) {
+  int p = 0;
+  for (int64_t run = cap; run < m; run <<= 1) ++p;
+  return p;
+}
+
+__global__ void k_vs_merge(const __grid_constant__ ViewshedParams q, int pass) {
+  if (q.w.head[0] != 0) return;
+  const int64_t run = (int64_t)q.cap << pass;
+  if (q.w.head[3] <= run) return;  // no ring needs this pass
+  const int span = q.w.head[2] - q.w.head[1] + 1;
+  const int total = q.w.start[span];
+  const double* sh = (pass & 1) ? q.w.heading : q.w.b_head;
+  const int32_t* si = (pass & 1) ? q.w.ring : q.w.b_idx;
+  double* dh = (pass & 1) ? q.w.b_head : q.w.heading;
+  int32_t* di = (pass & 1) ? q.w.b_idx : q.w.ring;
+  for (int64_t pos = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; pos < total; pos += (int64_t)gridDim.x * blockDim.x) {
+    int lo = 0, hi = span;  // the ring of pos: the last b with start[b] <= pos (empty rings share their successor's start)
+    while (hi - lo > 1) {
       const int mid = (lo + hi) >> 1;
-      if (key[mid] >> 63) hi = mid; else lo = mid + 1;
+      if (q.w.start[mid] <= pos) lo = mid; else hi = mid;
     }
-    q.w.fill[b] = lo;
+    const int m = q.w.count[lo];
+    if (m <= run) continue;
+    const int64_t s0 = q.w.start[lo], e = pos - s0;
+    const double h = sh[pos];
+    const int32_t c = si[pos];
+    const uint64_t key = vs_orderable(h);
+    const int64_t r = e / run, left = (r & ~1ll) * run;  // first cell of the pair
+    const bool in_left = (r & 1) == 0;
+    int64_t p0 = in_left ? left + run : left, p1 = in_left ? min(left + 2 * run, (int64_t)m) : left + run;  // the partner run
+    int64_t out = in_left ? e : e - run;
+    if (p0 < p1) {  // cells of the partner run below (h, c)
+      int64_t a = p0, z = p1;
+      while (a < z) {
+        const int64_t mid = (a + z) >> 1;
+        const uint64_t km = vs_orderable(sh[s0 + mid]);
+        if (km < key || (km == key && si[s0 + mid] < c)) a = mid + 1; else z = mid;
+      }
+      out += a - p0;
+    }
+    dh[s0 + out] = h;
+    di[s0 + out] = c;
   }
 }
 
-// np.interp's compiled loop for one abscissa (numpy compiled_base.c arr_interp): xp increasing, n >= 1.
+// np.interp's compiled loop for one abscissa (numpy compiled_base.c arr_interp): xp increasing, n >= 1.  vs_interp_at: from
+// the j the search found.
+template <typename XP>
+__device__ __forceinline__ double vs_interp_at(double x, int j, XP xp, const double* __restrict__ fp, int n) {
+  if (j == n - 1 || xp(j) == x) return fp[j];
+  const double slope = quo(sub(fp[j + 1], fp[j]), sub(xp(j + 1), xp(j)));
+  double r = add(mul(slope, sub(x, xp(j))), fp[j]);
+  if (isnan(r)) {  // "if we get nan in one direction, try the other"
+    r = add(mul(slope, sub(x, xp(j + 1))), fp[j + 1]);
+    if (isnan(r) && fp[j] == fp[j + 1]) r = fp[j];
+  }
+  return r;
+}
+
+// The same for a horizon of more entries than shared memory holds: xs = xp[0], xp[k], xp[2k], ... in shared memory, xp and fp
+// in global memory (xp written by this CTA: read through L2).  The search ends in the k-entry segment xs brackets, so j is again
+// the largest with xp[j] <= x.
+__device__ inline double vs_interp_sampled(double x, const double* __restrict__ xs, int k, const double* xp,
+                                           const double* __restrict__ fp, int n) {
+  const auto xg = [xp](int i) { return __ldcg(xp + i); };
+  if (isnan(x)) return x;
+  if (x < xs[0]) return fp[0];
+  if (x > xg(n - 1)) return fp[n - 1];
+  int lo = 0, hi = (n - 1) / k + 1;  // largest t with xs[t] <= x
+  while (hi - lo > 1) {
+    const int mid = (lo + hi) >> 1;
+    if (xs[mid] <= x) lo = mid; else hi = mid;
+  }
+  lo *= k;
+  hi = min(lo + k, n);
+  while (hi - lo > 1) {
+    const int mid = (lo + hi) >> 1;
+    if (xg(mid) <= x) lo = mid; else hi = mid;
+  }
+  return vs_interp_at(x, lo, xg, fp, n);
+}
+
 __device__ inline double vs_interp(double x, const double* __restrict__ xp, const double* __restrict__ fp, int n) {
   if (isnan(x)) return x;
   if (x < xp[0]) return fp[0];
@@ -240,15 +342,7 @@ __device__ inline double vs_interp(double x, const double* __restrict__ xp, cons
     const int mid = (lo + hi) >> 1;
     if (xp[mid] <= x) lo = mid; else hi = mid;
   }
-  const int j = lo;
-  if (j == n - 1 || xp[j] == x) return fp[j];
-  const double slope = quo(sub(fp[j + 1], fp[j]), sub(xp[j + 1], xp[j]));
-  double r = add(mul(slope, sub(x, xp[j])), fp[j]);
-  if (isnan(r)) {  // "if we get nan in one direction, try the other"
-    r = add(mul(slope, sub(x, xp[j + 1])), fp[j + 1]);
-    if (isnan(r) && fp[j] == fp[j + 1]) r = fp[j];
-  }
-  return r;
+  return vs_interp_at(x, lo, [xp](int i) { return xp[i]; }, fp, n);
 }
 
 #define GB_VS_TWO_PI 6.283185307179586
@@ -258,33 +352,48 @@ __device__ __forceinline__ double vs_mod_period(double h) {  // np.remainder(h, 
   return h == 0.0 ? 0.0 : h;
 }
 
+// LARGE = false: every ring has at most q.cap cells (head[3] == 0); LARGE = true: some ring has more, so a ring may sit in the
+// merge passes' second buffer pair, and the ring after one searches the sampled horizon.  Both are launched; the one that does
+// not apply returns at once, so the common case keeps a kernel of its own registers.
+template <bool LARGE>
 __global__ void __launch_bounds__(GB_VS_SWEEP_THREADS) k_vs_sweep(const __grid_constant__ ViewshedParams q) {
   extern __shared__ __align__(16) unsigned char vs_sweep_raw[];
-  double* xp_s = reinterpret_cast<double*>(vs_sweep_raw);  // [prev_m + 2] abscissae of the previous ring's horizon
+  // [prev_m + 2] abscissae of the previous ring's horizon; after a ring of more than q.cap cells every prev_k-th of them
+  double* xp_s = reinterpret_cast<double*>(vs_sweep_raw);
   __shared__ int s_cnt[2];  // unknown horizons, newly opened cells (only while the horizon still has NaN)
   constexpr int VS_BATCH = 4;
   const int64_t n = (int64_t)q.nx * q.ny;
   const int tid = threadIdx.x, nthr = GB_VS_SWEEP_THREADS;
-  if (q.w.head[0] != 0) return;
+  if (q.w.head[0] != 0 || (q.w.head[3] != 0) != LARGE) return;
   const int rmin = q.w.head[1], span = q.w.head[2] - rmin + 1;
   // a raster that is one ring: all visible if that ring is ring 0 (raster.py:1343-1345), otherwise that ring is the first
-  int rings_with_cells = 0;
-  for (int b = 0; b < span; ++b) rings_with_cells += q.w.count[b] > 0;  // (every thread counts: span is a few thousand at most)
-  if (rings_with_cells == 1 && rmin == 0) {
+  int rings_with_cells = 0;  // (of this thread's rings: there are ~15 000 rings in a DEM of 10^8 cells)
+  for (int b = tid; b < span; b += nthr) rings_with_cells += q.w.count[b] > 0;
+  const bool one_ring = __syncthreads_count(rings_with_cells > 0) == 1 && !__syncthreads_or(rings_with_cells > 1);
+  if (one_ring && rmin == 0) {
     for (int64_t i = tid; i < n; i += nthr) q.visible[i] = 1;
     return;
   }
   for (int64_t i = tid; i < n; i += nthr) q.visible[i] = 0;
   bool first = true, has_nan = false;
-  int prev_m = 0, cur = 0;
+  int prev_m = 0, prev_k = 1, cur = 0;
   for (int b = 0; b < span; ++b) {
     const int m = q.w.count[b];
     if (m == 0) continue;
     if (b == 0 && rmin == 0) continue;  // the cells within half a cell of the origin are not visited (raster.py:1336-1338)
     const int s0 = q.w.start[b], n_neg = q.w.fill[b];
+    const double* r_head = q.w.b_head;
+    const int32_t* r_idx = q.w.b_idx;
+    if constexpr (LARGE) {
+      if (vs_merge_passes(m, q.cap) & 1) {  // k_vs_merge left the ring in its second buffer pair
+        r_head = q.w.heading;
+        r_idx = q.w.ring;
+      }
+    }
     const double* pf = q.w.hf[cur ^ 1];
+    const double* px = q.w.hx[cur ^ 1];
     double* nf_ = q.w.hf[cur];
-    double* nx_ = q.w.hx[0];  // this ring's abscissae on their way to shared memory
+    double* nx_ = q.w.hx[LARGE ? cur : 0];  // this ring's abscissae on their way to shared memory
     if (has_nan) {
       if (tid < 2) s_cnt[tid] = 0;
       __syncthreads();
@@ -298,8 +407,8 @@ __global__ void __launch_bounds__(GB_VS_SWEEP_THREADS) k_vs_sweep(const __grid_c
       for (int k = 0; k < VS_BATCH; ++k) {
         const int j = tid + (k0 + k) * nthr;
         if (j < m) {
-          h[k] = q.w.b_head[s0 + j];
-          cell[k] = q.w.b_idx[s0 + j];
+          h[k] = r_head[s0 + j];
+          cell[k] = r_idx[s0 + j];
         }
       }
 #pragma unroll
@@ -317,7 +426,10 @@ __global__ void __launch_bounds__(GB_VS_SWEEP_THREADS) k_vs_sweep(const __grid_c
             hor = r[k];
             nans |= isnan(r[k]);
           } else {
-            hor = vs_interp(x, xp_s, pf, prev_m + 2);
+            if (LARGE && prev_k > 1)
+              hor = vs_interp_sampled(x, xp_s, prev_k, px, pf, prev_m + 2);
+            else
+              hor = vs_interp(x, xp_s, pf, prev_m + 2);
             seen = r[k] > hor;
             if (has_nan) {
               const bool unk = isnan(hor);
@@ -356,8 +468,15 @@ __global__ void __launch_bounds__(GB_VS_SWEEP_THREADS) k_vs_sweep(const __grid_c
     } else {
       __syncthreads();
     }
-    // everybody is done with the previous abscissae: this ring's take their place in shared memory
-    for (int i = tid; i < m + 2; i += nthr) xp_s[i] = __ldcg(nx_ + i);
+    // everybody is done with the previous abscissae: this ring's take their place in shared memory (every prev_k-th of them
+    // when there are more than q.cap + 2: then at most q.cap + 2 samples)
+    if (LARGE && m > q.cap) {
+      prev_k = (m + 2 + q.cap + 1) / (q.cap + 2);
+      for (int i = tid; i <= (m + 1) / prev_k; i += nthr) xp_s[i] = __ldcg(nx_ + (int64_t)i * prev_k);
+    } else {
+      prev_k = 1;
+      for (int i = tid; i < m + 2; i += nthr) xp_s[i] = __ldcg(nx_ + i);
+    }
     __syncthreads();
     first = false;
     prev_m = m;

@@ -267,8 +267,6 @@ class Raster:
         _lib.check(lib.gb_viewshed(z_d.data_ptr(), nx, ny, x_d.data_ptr(), y_d.data_ptr(), float(d[0]), (C.c_double * 3)(*origin[:3]),
                                    corr, max_rings, work.data_ptr(), nbytes, out.data_ptr(), torch.cuda.current_stream().cuda_stream))
         status = int(work[:4].cpu().numpy().view(np.int32)[0])  # (synchronises)
-        if status == 3:
-            raise NotImplementedError("viewshed: a ring of more than 16384 cells (rasters beyond ~2600 cells of radius)")
         if status != 0:
             raise RuntimeError(f"viewshed: device status {status}")
         return out.cpu().numpy().reshape(ny, nx).astype(bool)

@@ -188,9 +188,11 @@ int gb_decode_jpeg(const uint8_t* jpeg_host, int64_t nbytes, int32_t width, int3
  * origin_host = (x, y, z).  x_centres[nx] / y_centres[ny] (device) are the cell-centre coordinates in array order (Grid.x, Grid.y,
  * raster.py:139-174), cell = |d[0]|, corr_host = {radius, refraction} or NULL (helpers.elevation_corrections).  max_rings bounds
  * the number of distance rings between the nearest and the farthest cell (the host knows it from the raster's corners); work =
- * gb_viewshed_work_bytes(nx, ny, max_rings) bytes of device scratch whose first int32 is the status the caller reads back after
- * the stream: 0 ok, 2 more rings than max_rings, 3 a ring of more than 16 384 cells (rasters beyond ~2 600 cells of radius).
- * visible[ny * nx] = 1 / 0. */
+ * gb_viewshed_work_bytes(nx, ny, max_rings) bytes of device scratch (64 per cell, 12 per ring and 2 KB) whose first int32 is the
+ * status the caller reads back after the stream: 0 ok, 2 more rings than max_rings.  Rings of any size; GB_E_RESOURCE, before
+ * any device work, for more than 2^31 cells.  The call only enqueues work on `stream`.  visible[ny * nx] = 1 / 0.
+ * Test hook: the environment variable GB_VS_RING_CAP (1 up to the default capacity) lowers the number of cells a ring may have
+ * before it takes the large-ring sort and horizon search; the result is the same. */
 int64_t gb_viewshed_work_bytes(int32_t nx, int32_t ny, int32_t max_rings);
 int gb_viewshed(const double* z, int32_t nx, int32_t ny, const double* x_centres, const double* y_centres, double cell,
                 const double* origin_host, const double* corr_host, int32_t max_rings, void* work, int64_t work_bytes,
