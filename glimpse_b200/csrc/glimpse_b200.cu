@@ -45,9 +45,7 @@ struct StepParams {
   int64_t P, N;
   int T, O, S, t;
   int tile_w, tile_h;
-  int cluster, n_local, particles_in_smem, tile_bytes;
-  int n_slabs, hp_rows;       // hp_rows x hp_cols: size of the median high-pass (Tracker.highpass['size'], tracker.py:59, 530)
-  int64_t slab_bytes, particle_scratch_bytes;
+  int hp_rows;                // hp_rows x hp_cols: size of the median high-pass (Tracker.highpass['size'], tracker.py:59, 530)
   int skip_evolve, viewshed, rng_mode, hp_cols;
   int hp_mode, hp_org_r, hp_org_c;  // border mode (GB_HP_*) and origin of the median high-pass
   double hp_cval;
@@ -79,7 +77,6 @@ struct StepParams {
   double* state_a;
   double* state_b;
   double* weight_state;
-  double* scratch;
   double* tmpl_tile;
   double* tmpl_values;
   double* tmpl_quantiles;
@@ -790,28 +787,6 @@ __device__ __forceinline__ double warp_inclusive_scan(double v, int lane) {
 // ---------------------------------------------------------------------------------------------
 // Host side
 // ---------------------------------------------------------------------------------------------
-static std::once_flag g_tables_once[16];
-
-static int ensure_tables() {
-  int dev = 0;
-  GB_CUDA(cudaGetDevice(&dev));
-  if (dev < 0 || dev >= 16) return fail(GB_E_INVALID, "device index out of range%s");
-  cudaError_t err = cudaSuccess;
-  std::call_once(g_tables_once[dev], [&]() {
-    static double cp[GB_MAX_SURFACE], inv[GB_MAX_SURFACE];
-    cp[0] = 2.0;
-    inv[0] = 1.0;
-    for (int i = 1; i < GB_MAX_SURFACE; ++i) {
-      inv[i] = 1.0 / (4.0 - cp[i - 1]);
-      cp[i] = inv[i];
-    }
-    err = cudaMemcpyToSymbol(c_spline_cp, cp, sizeof(cp));
-    if (err == cudaSuccess) err = cudaMemcpyToSymbol(c_spline_inv, inv, sizeof(inv));
-  });
-  if (err != cudaSuccess) return fail(GB_E_CUDA, "spline tables: %s", cudaGetErrorString(err));
-  return GB_OK;
-}
-
 static int grid_for(int64_t n, int threads) {
   int64_t g = (n + threads - 1) / threads;
   if (g < 1) g = 1;
@@ -946,13 +921,6 @@ static void fill_params(const gb_track_desc& d, int t, StepParams& prm) {
   prm.hp_has_fp = d.highpass_footprint_host != nullptr;
   if (prm.hp_has_fp)
     for (int a = 0; a < GB_MAX_HIGHPASS; ++a) prm.hp_fp[a] = a < prm.hp_rows ? d.highpass_footprint_host[a] : 0u;
-  prm.cluster = d.plan.cluster;
-  prm.n_local = d.plan.n_local;
-  prm.particles_in_smem = d.plan.particles_in_smem;
-  prm.tile_bytes = d.plan.tile_bytes;
-  prm.n_slabs = d.plan.n_slabs;
-  prm.slab_bytes = d.plan.slab_bytes;
-  prm.particle_scratch_bytes = d.plan.particle_scratch_bytes;
   prm.viewshed = d.viewshed;
   prm.rng_mode = d.rng_mode;
   prm.seed = d.seed;
@@ -1001,7 +969,6 @@ static void fill_params(const gb_track_desc& d, int t, StepParams& prm) {
   prm.state_a = d.state_a;
   prm.state_b = d.state_b;
   prm.weight_state = d.weight_state;
-  prm.scratch = d.scratch;
   prm.tmpl_tile = d.tmpl_tile;
   prm.tmpl_values = d.tmpl_values;
   prm.tmpl_quantiles = d.tmpl_quantiles;
@@ -1077,6 +1044,8 @@ static int check_desc(const gb_track_desc& d) {
   if ((d.plan.stream_nblk < 1 || d.plan.surf_bytes <= 0 ||
                                         d.plan.stream_batch < 1 || d.plan.stream_slots < 1 || d.plan.stream_slots > kMaxSlots))
     return fail(GB_E_INVALID, "streaming plan does not match the descriptor (use gb_step_plan)%s");
+  if (d.plan.stream_block > GB_S4P_CAP || (d.plan.stream_block & 1)) return fail(GB_E_INVALID, "plan: stream_block must be even and <= 768%s");
+  if (d.plan.stream_batch > 65535) return fail(GB_E_INVALID, "plan: stream_batch must be <= 65535%s");
   if (d.plan.scratch_bytes > 0 && !d.scratch) return fail(GB_E_INVALID, "plan needs a scratch buffer%s");
   if ((int64_t)d.plan.n_local < d.N) return fail(GB_E_INVALID, "plan does not cover N particles%s");
   return GB_OK;
@@ -1163,7 +1132,7 @@ static void stream_bind(const gb_track_desc& d, StepParams& prm, int par, int64_
 
 // Side streams on which batches of points advance independently (points never interact).  One pool per device.
 struct StreamPool {
-  std::mutex busy;  // one streaming call at a time per device: the fork / join events are shared
+  std::mutex busy;  // one call at a time per device: the fork / join events are shared
   cudaStream_t side[kMaxSlots] = {};
   cudaEvent_t fork = nullptr, join[kMaxSlots] = {};
   bool ready = false;
@@ -1188,87 +1157,6 @@ static int get_pool(StreamPool** out) {
   *out = &pool;
   return GB_OK;
 }
-
-template <bool COV>
-static int launch_stream_batch(const StepParams& prm, cudaStream_t stream) {
-  const unsigned nb = (unsigned)(prm.pb * prm.s_nblk);
-  k_s0_reset<<<grid_for(prm.pb * prm.slot_stride * 5, 256), 256, 0, stream>>>(prm);
-  k_s1_propagate<<<nb, GB_SBLOCK_THREADS, 0, stream>>>(prm);
-  FrameMaps fm;
-  frame_maps(prm, fm);
-  if (prm.tile_w * prm.tile_h > GB_SMEM_TEMPLATE)
-    k_s2_surface<true><<<(unsigned)(prm.pb * prm.n_slots), GB_S2_THREADS, prm.s2_smem, stream>>>(prm, fm, prm.s2_budget);
-  else
-    k_s2_surface<false><<<(unsigned)(prm.pb * prm.n_slots), GB_S2_THREADS, prm.s2_smem, stream>>>(prm, fm, prm.s2_budget);
-  if (spline_is_hermite(prm.interp_cols, prm.interp_rows))
-    k_s3_weights<false><<<dim3((unsigned)prm.s_nblk, (unsigned)prm.pb), s3_threads(prm.s_block), 0, stream>>>(prm);
-  else
-    k_s3_weights<true><<<dim3((unsigned)prm.s_nblk, (unsigned)prm.pb), s3_threads(prm.s_block), 0, stream>>>(prm);
-  if (prm.resample_method == GB_RESAMPLE_CHOICE) {
-    k_s4c_scan<<<nb, GB_SBLOCK_THREADS, 0, stream>>>(prm);
-    k_s4c_gather<COV><<<nb, GB_SBLOCK_THREADS, 0, stream>>>(prm);
-  } else if (prm.resample_method == GB_RESAMPLE_RESIDUAL) {
-    k_s4r_residual<<<(unsigned)prm.pb, GB_SBLOCK_THREADS, 0, stream>>>(prm);
-    k_s4c_gather<COV><<<nb, GB_SBLOCK_THREADS, 0, stream>>>(prm);
-  } else {
-    k_s4_resample<COV><<<nb, GB_SBLOCK_THREADS, 0, stream>>>(prm);
-  }
-  k_s5_finalize<COV><<<(unsigned)((prm.pb + 3) / 4), 128, 0, stream>>>(prm);
-  GB_CUDA(cudaGetLastError());
-  return GB_OK;
-}
-
-// One update of all points in GB_MODE_STREAM: the points are cut into batches whose intermediates fit the
-// L2 cache; batch b runs on side stream b % slots with scratch slot b % slots.  `fork`: make the side streams
-// wait for everything enqueued on `stream` so far; `join`: make `stream` wait for the side streams.
-static int launch_stream_update(const gb_track_desc& d, StepParams& prm, cudaStream_t stream, bool fork, bool join,
-                                int64_t* launches) {
-  static std::once_flag attr_once[16];
-  int dev = 0;
-  GB_CUDA(cudaGetDevice(&dev));
-  cudaError_t aerr = cudaSuccess;
-  std::call_once(attr_once[dev & 15], [&]() {
-    aerr = cudaFuncSetAttribute(k_s2_surface<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSurfaceSmem);
-    if (aerr == cudaSuccess) aerr = cudaFuncSetAttribute(k_s2_surface<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSurfaceSmemLarge);
-  });
-  if (aerr != cudaSuccess) return fail(GB_E_CUDA, "k_s2_surface attributes: %s", cudaGetErrorString(aerr));
-  const bool cov = d.covariances != nullptr;
-  const int slots = d.plan.stream_slots;
-  const int64_t batch = d.plan.stream_batch;
-  const int64_t nbatch = (d.P + batch - 1) / batch;
-  StreamPool* pool = nullptr;
-  int rc = get_pool(&pool);
-  if (rc) return rc;
-  const int used = (int)(nbatch < slots ? nbatch : slots);
-  std::lock_guard<std::mutex> guard(pool->busy);
-  if (fork) {
-    GB_CUDA(cudaEventRecord(pool->fork, stream));
-    for (int k = 0; k < used; ++k) GB_CUDA(cudaStreamWaitEvent(pool->side[k], pool->fork, 0));
-  }
-  if (d.image_events_host)
-    for (int s = 0; s < prm.n_slots; ++s)
-      if (prm.img[s] >= 0 && d.image_events_host[prm.img[s]])
-        for (int k = 0; k < used; ++k)
-          GB_CUDA(cudaStreamWaitEvent(pool->side[k], (cudaEvent_t)d.image_events_host[prm.img[s]], 0));
-  for (int64_t b = 0; b < nbatch; ++b) {
-    const int slot = (int)(b % slots);
-    const int64_t p0 = b * batch, pb = (p0 + batch <= d.P) ? batch : d.P - p0;
-    stream_bind(d, prm, prm.t, p0, pb);
-    rc = cov ? launch_stream_batch<true>(prm, pool->side[slot]) : launch_stream_batch<false>(prm, pool->side[slot]);
-    if (rc) return rc;
-    if (launches) *launches += 6;
-  }
-  if (join) {
-    for (int k = 0; k < used; ++k) {
-      GB_CUDA(cudaEventRecord(pool->join[k], pool->side[k]));
-      GB_CUDA(cudaStreamWaitEvent(stream, pool->join[k], 0));
-    }
-  }
-  return GB_OK;
-}
-
-static int launch_init(const StepParams& prm, bool cov, cudaStream_t stream);
-static int launch_template(const gb_track_desc& d, StepParams prm, cudaStream_t stream);
 
 // Optional per-kernel timing of the pipelined flow (gb_kernel_timing): every launch is bracketed by CUDA events
 // on the stream it is launched on; durations are accumulated per kernel kind when the track has finished.
@@ -1313,217 +1201,115 @@ struct KernelTimer {
 };
 static KernelTimer g_ktimer;
 
-// gb_track in GB_MODE_STREAM: the pipelined flow of stream.cuh.  Points are cut into `slots` batches that
-// advance on their own side streams without meeting; the caller's stream runs the kernels that need all
-// batches to be at the same time (first-frame initialisation, template construction) between a join and a fork.
-static int track_streaming(const gb_track_desc& d, cudaStream_t stream, int64_t* launches) {
-  static std::once_flag attr_once[16];
+// Per-device set-up of the gb_track* entry points and gb_sample_surface: the spline tables, and the dynamic shared memory of
+// every kernel that may need more than 48 KB.  The outcome is kept, so a failure reaches every call, not only the first.
+static int ensure_device() {
+  static std::once_flag once[16];
+  static cudaError_t result[16];
   int dev = 0;
   GB_CUDA(cudaGetDevice(&dev));
-  cudaError_t aerr = cudaSuccess;
-  std::call_once(attr_once[dev & 15], [&]() {
-    aerr = cudaFuncSetAttribute(k_s2_surface<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSurfaceSmem);
-    if (aerr == cudaSuccess) aerr = cudaFuncSetAttribute(k_s2_surface<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSurfaceSmemLarge);
-    if (aerr == cudaSuccess) aerr = cudaFuncSetAttribute(k_s4p_resample_propagate<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kS4pSmem);
-    if (aerr == cudaSuccess) aerr = cudaFuncSetAttribute(k_s4p_resample_propagate<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kS4pSmem);
-    if (aerr == cudaSuccess) aerr = cudaFuncSetAttribute(k_s4p_resample_propagate<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kS4pSmem);
-    if (aerr == cudaSuccess) aerr = cudaFuncSetAttribute(k_s4p_resample_propagate<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kS4pSmem);
+  if (dev < 0 || dev >= 16) return fail(GB_E_INVALID, "device index out of range%s");
+  std::call_once(once[dev], [dev]() {
+    static double cp[GB_MAX_SURFACE], inv[GB_MAX_SURFACE];
+    cp[0] = 2.0;
+    inv[0] = 1.0;
+    for (int i = 1; i < GB_MAX_SURFACE; ++i) {
+      inv[i] = 1.0 / (4.0 - cp[i - 1]);
+      cp[i] = inv[i];
+    }
+    cudaError_t err = cudaMemcpyToSymbol(c_spline_cp, cp, sizeof(cp));
+    if (err == cudaSuccess) err = cudaMemcpyToSymbol(c_spline_inv, inv, sizeof(inv));
+    auto smem = [&err](const void* kernel, int bytes) {
+      if (err == cudaSuccess) err = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+    };
+    smem((const void*)k_s2_surface<false>, kSurfaceSmem);
+    smem((const void*)k_s2_surface<true>, kSurfaceSmemLarge);
+    smem((const void*)k_s4p_resample_propagate<true, true>, kS4pSmem);
+    smem((const void*)k_s4p_resample_propagate<false, true>, kS4pSmem);
+    smem((const void*)k_s4p_resample_propagate<true, false>, kS4pSmem);
+    smem((const void*)k_s4p_resample_propagate<false, false>, kS4pSmem);
+    smem((const void*)k_template<true>, template_smem_bytes(GB_MAX_TEMPLATE_SIDE * GB_MAX_TEMPLATE_SIDE));
+    result[dev] = err;
   });
-  if (aerr != cudaSuccess) return fail(GB_E_CUDA, "stream kernel attributes: %s", cudaGetErrorString(aerr));
-  if (d.plan.stream_block > GB_S4P_CAP || (d.plan.stream_block & 1)) return fail(GB_E_INVALID, "plan: stream_block must be even and <= 768%s");
-  if (d.plan.stream_batch > 65535) return fail(GB_E_INVALID, "plan: stream_batch must be <= 65535%s");
-  const bool cov = d.covariances != nullptr;
-  // kernels without the tangent models' DEM gathers when the caller says no point uses them (0 = unknown: assume any kind)
-  const bool tangent = d.motion_kinds == 0 || (d.motion_kinds & ((1 << GB_MOTION_TANGENT_CARTESIAN) | (1 << GB_MOTION_TANGENT_CYLINDRICAL))) != 0;
-  const int slots = d.plan.stream_slots;
-  const int64_t batch = d.plan.stream_batch;
-  const int64_t nbatch = (d.P + batch - 1) / batch;
-  const int used = (int)(nbatch < slots ? nbatch : slots);
+  if (result[dev] != cudaSuccess) return fail(GB_E_CUDA, "spline tables or kernel attributes: %s", cudaGetErrorString(result[dev]));
+  return GB_OK;
+}
+
+// `s` waits for the uploads of the frames of time prm.t (gb_track_desc.image_events_host).
+static int wait_frames(const gb_track_desc& d, const StepParams& prm, cudaStream_t s) {
+  if (!d.image_events_host) return GB_OK;
+  for (int k = 0; k < prm.n_slots; ++k)
+    if (prm.img[k] >= 0 && d.image_events_host[prm.img[k]])
+      GB_CUDA(cudaStreamWaitEvent(s, (cudaEvent_t)d.image_events_host[prm.img[k]], 0));
+  return GB_OK;
+}
+
+// The side streams of a call.  Points never interact, so batches of them advance on their own streams: batch b runs on side
+// stream b % slots with scratch slot b % slots.  The caller's stream forks them after its own kernels (first-frame
+// initialisation, templates) and joins them before the next such kernel and at the end.
+struct SideStreams {
+  const gb_track_desc& d;
+  cudaStream_t stream;  // the caller's
   StreamPool* pool = nullptr;
-  int rc = get_pool(&pool);
-  if (rc) return rc;
-  std::lock_guard<std::mutex> guard(pool->busy);
-  std::vector<int> tmpl_frame(d.O);
-  for (int o = 0; o < d.O; ++o) tmpl_frame[o] = template_frame(d, o);
-  // what happens at each time (host copies of first / last / mask)
-  const int T = d.T;
-  std::vector<uint8_t> has_init(T, 0), has_tmpl(T, 0), has_update(T, 0), has_prop(T, 0);
-  bool staggered_any = false;
-  for (int64_t p = 0; p < d.P; ++p) {
-    const int f = d.first_host[p], l = d.last_host[p];
-    if (f < 0 || f >= T || l < f) continue;
-    has_init[f] = 1;
-    for (int t = f; t <= l && t < T; ++t) {
-      if (t > f) has_update[t] = 1;
-      if (t < l) has_prop[t] = 1;
-    }
-    for (int o = 0; o < d.O; ++o) {
-      const int tf = tmpl_frame[o];
-      if (tf >= f && tf <= l && d.mask_host[p * d.O + o]) {
-        has_tmpl[tf] = 1;
-        if (tf > f) staggered_any = true;
-      }
-    }
-  }
-  if (staggered_any && !d.weight_state)
-    return fail(GB_E_INVALID, "weight_state is required when a template starts after a point's first frame%s");
-  auto wait_images = [&](cudaStream_t s, const StepParams& prm) -> int {
-    if (!d.image_events_host) return GB_OK;
-    for (int k = 0; k < prm.n_slots; ++k)
-      if (prm.img[k] >= 0 && d.image_events_host[prm.img[k]])
-        GB_CUDA(cudaStreamWaitEvent(s, (cudaEvent_t)d.image_events_host[prm.img[k]], 0));
+  std::unique_lock<std::mutex> busy;
+  int used = 0;  // side streams that receive a batch
+  bool forked = false;
+
+  SideStreams(const gb_track_desc& desc, cudaStream_t caller) : d(desc), stream(caller) {}
+  int open() {
+    if (int rc = get_pool(&pool)) return rc;
+    busy = std::unique_lock<std::mutex>(pool->busy);
+    const int64_t nbatch = (d.P + d.plan.stream_batch - 1) / d.plan.stream_batch;
+    used = (int)(nbatch < d.plan.stream_slots ? nbatch : d.plan.stream_slots);
     return GB_OK;
-  };
-  bool forked = false, need_fork = true;
-  auto join_sides = [&]() -> int {
+  }
+  // the side streams wait for what the caller's stream holds now (once until the next join)
+  int fork() {
+    if (forked) return GB_OK;
+    GB_CUDA(cudaEventRecord(pool->fork, stream));
+    for (int k = 0; k < used; ++k) GB_CUDA(cudaStreamWaitEvent(pool->side[k], pool->fork, 0));
+    forked = true;
+    return GB_OK;
+  }
+  // the caller's stream waits for what the side streams hold
+  int join() {
     if (!forked) return GB_OK;
     for (int k = 0; k < used; ++k) {
       GB_CUDA(cudaEventRecord(pool->join[k], pool->side[k]));
       GB_CUDA(cudaStreamWaitEvent(stream, pool->join[k], 0));
     }
     forked = false;
-    need_fork = true;
     return GB_OK;
-  };
-  {
-    StepParams prm;
-    fill_params(d, 0, prm);
-    stream_bind(d, prm, 0, 0, d.P);
-    k_s0p_reset<<<grid_for(d.P * prm.slot_stride * 5, 256), 256, 0, stream>>>(prm);
-    GB_CUDA(cudaGetLastError());
-    if (launches) ++*launches;
   }
-  bool have_activity = false;
-  for (int t = 0; t < T; ++t) {
-    if (!has_init[t] && !has_update[t] && !has_prop[t]) {
-      have_activity = false;  // a gap: the last k_s5p wrote the activity of a time that is not processed
-      continue;
-    }
-    StepParams prm;
-    fill_params(d, t, prm);
-    NextParams nxt;
-    memset(&nxt, 0, sizeof(nxt));
-    for (int o = 0; o < GB_MAX_OBS; ++o) nxt.img[o] = -1;
-    nxt.spec_update = has_init[t] ? 0 : 1;
-    if (const char* e = getenv("GB_S4P_SPEC")) nxt.spec_update = nxt.spec_update && atoi(e) != 0;
-    if (t + 1 < T) {
-      StepParams pn;
-      fill_params(d, t + 1, pn);
-      nxt.tau = pn.tau;
-      nxt.tau2 = pn.tau2;
-      nxt.n_slots = pn.n_slots;
-      for (int s = 0; s < pn.n_slots; ++s) {
-        nxt.obs[s] = pn.obs[s];
-        nxt.img[s] = pn.img[s];
-        nxt.cam[s] = pn.cam[s];
-      }
-    }
-    FrameMaps fm;
-    frame_maps(prm, fm);
-    if (has_init[t] || has_tmpl[t]) {
-      if ((rc = join_sides())) return rc;
-      if ((rc = wait_images(stream, prm))) return rc;
-      stream_bind(d, prm, t, 0, d.P);
-      prm.tmpl_from_ev = 1;
-      if (has_init[t]) {
-        g_ktimer.begin(GB_K_INIT, stream);
-        if ((rc = launch_init(prm, cov, stream))) return rc;
-        g_ktimer.end(stream);
-        if (launches) ++*launches;
-      }
-      if (has_tmpl[t]) {
-        g_ktimer.begin(GB_K_TEMPLATE, stream);
-        if ((rc = launch_template(d, prm, stream))) return rc;
-        g_ktimer.end(stream);
-        if (launches) ++*launches;
-      }
-    }
-    if (need_fork) {
-      GB_CUDA(cudaEventRecord(pool->fork, stream));
-      for (int k = 0; k < used; ++k) GB_CUDA(cudaStreamWaitEvent(pool->side[k], pool->fork, 0));
-      forked = true;
-      need_fork = false;
-    }
-    if (has_update[t])
-      for (int k = 0; k < used; ++k)
-        if ((rc = wait_images(pool->side[k], prm))) return rc;
-    // activity of time t: written by k_s5p of the previous processed time unless statuses may have changed since
-    const bool need_activity = !have_activity || has_init[t] || has_tmpl[t];
-    have_activity = true;
-    for (int64_t b = 0; b < nbatch; ++b) {
-      cudaStream_t ss = pool->side[b % slots];
-      const int64_t p0 = b * batch, pb = (p0 + batch <= d.P) ? batch : d.P - p0;
-      stream_bind(d, prm, t, p0, pb);
-      KernelTimer& kt = g_ktimer;
-      if (need_activity) {
-        kt.begin(GB_K_ACTIVITY, ss);
-        k_s0p_activity<<<grid_for(pb, 256), 256, 0, ss>>>(prm);
-        kt.end(ss);
-      }
-      if (has_update[t]) {
-        kt.begin(GB_K_SURFACE, ss);
-        if (prm.tile_w * prm.tile_h > GB_SMEM_TEMPLATE)
-          k_s2_surface<true><<<(unsigned)(pb * prm.n_slots), GB_S2_THREADS, prm.s2_smem, ss>>>(prm, fm, prm.s2_budget);
-        else
-          k_s2_surface<false><<<(unsigned)(pb * prm.n_slots), GB_S2_THREADS, prm.s2_smem, ss>>>(prm, fm, prm.s2_budget);
-        kt.end(ss);
-        kt.begin(GB_K_WEIGHTS, ss);
-        if (spline_is_hermite(prm.interp_cols, prm.interp_rows))
-          k_s3_weights<false><<<dim3((unsigned)prm.s_nblk, (unsigned)pb), s3_threads(prm.s_block), 0, ss>>>(prm);
-        else
-          k_s3_weights<true><<<dim3((unsigned)prm.s_nblk, (unsigned)pb), s3_threads(prm.s_block), 0, ss>>>(prm);
-        kt.end(ss);
-        kt.begin(GB_K_PUBLISH, ss);
-        k_s3b_publish<<<(unsigned)((pb + 7) / 8), 256, 0, ss>>>(prm);
-        kt.end(ss);
-      }
-      kt.begin(GB_K_RESAMPLE_PROPAGATE, ss);
-      {
-        const dim3 grid((unsigned)prm.s_nblk, (unsigned)pb);
-        if (cov && tangent)
-          k_s4p_resample_propagate<true, true><<<grid, GB_S4P_THREADS, kS4pSmem, ss>>>(prm, nxt);
-        else if (cov)
-          k_s4p_resample_propagate<true, false><<<grid, GB_S4P_THREADS, kS4pSmem, ss>>>(prm, nxt);
-        else if (tangent)
-          k_s4p_resample_propagate<false, true><<<grid, GB_S4P_THREADS, kS4pSmem, ss>>>(prm, nxt);
-        else
-          k_s4p_resample_propagate<false, false><<<grid, GB_S4P_THREADS, kS4pSmem, ss>>>(prm, nxt);
-      }
-      kt.end(ss);
-      kt.begin(GB_K_FINALIZE, ss);
-      if (cov)
-        k_s5p_finalize<true><<<(unsigned)((pb + 3) / 4), 128, 0, ss>>>(prm);
-      else
-        k_s5p_finalize<false><<<(unsigned)((pb + 3) / 4), 128, 0, ss>>>(prm);
-      kt.end(ss);
-      GB_CUDA(cudaGetLastError());
-      if (launches) *launches += (has_update[t] ? 5 : 2) + (need_activity ? 1 : 0);
-    }
+  int wait_frames(const StepParams& prm) {
+    for (int k = 0; k < used; ++k)
+      if (int rc = gb::wait_frames(d, prm, pool->side[k])) return rc;
+    return GB_OK;
   }
-  if ((rc = join_sides())) return rc;
-  if (g_ktimer.on) {
-    GB_CUDA(cudaStreamSynchronize(stream));
-    g_ktimer.collect();
+  // launch(prm bound to the batch, its side stream) for every batch of points
+  template <class Launch>
+  int each_batch(StepParams& prm, Launch&& launch) {
+    const int64_t batch = d.plan.stream_batch;
+    for (int64_t b = 0, p0 = 0; p0 < d.P; ++b, p0 += batch) {
+      stream_bind(d, prm, prm.t, p0, p0 + batch <= d.P ? batch : d.P - p0);
+      if (int rc = launch(prm, pool->side[b % d.plan.stream_slots])) return rc;
+    }
+    return GB_OK;
   }
-  return GB_OK;
-}
+};
 
-// One update for all points in the organisation the plan asks for.
-static int launch_update(const gb_track_desc& d, StepParams& prm, cudaStream_t stream, bool fork, bool join, int64_t* launches) {
-  return launch_stream_update(d, prm, stream, fork, join, launches);
-}
-
-static int launch_init(const StepParams& prm, bool cov, cudaStream_t stream) {
-  const int smem = kHeaderBytes;
+// Each launch helper below adds the kernels it enqueues to `launches`.
+static int launch_init(const StepParams& prm, bool cov, cudaStream_t stream, int64_t& launches) {
   if (cov)
-    k_init<true><<<(unsigned)prm.P, GB_THREADS, smem, stream>>>(prm);
+    k_init<true><<<(unsigned)prm.P, GB_THREADS, kHeaderBytes, stream>>>(prm);
   else
-    k_init<false><<<(unsigned)prm.P, GB_THREADS, smem, stream>>>(prm);
+    k_init<false><<<(unsigned)prm.P, GB_THREADS, kHeaderBytes, stream>>>(prm);
+  ++launches;
   GB_CUDA(cudaGetLastError());
   return GB_OK;
 }
 
-static int launch_template(const gb_track_desc& d, StepParams prm, cudaStream_t stream) {
+static int launch_template(const gb_track_desc& d, StepParams prm, cudaStream_t stream, int64_t& launches) {
   const int area = prm.tile_w * prm.tile_h;
   if (area <= GB_SMEM_TEMPLATE) {
     k_template<false><<<(unsigned)(prm.P * prm.n_slots), 256, 0, stream>>>(prm);
@@ -1531,18 +1317,243 @@ static int launch_template(const gb_track_desc& d, StepParams prm, cudaStream_t 
     // the work area of ranked frames: the surface regions (plan.surf_bytes >= 8 B a template pixel)
     prm.s_surf = reinterpret_cast<char*>(d.scratch) + stream_layout(d.P, d.N, d.plan.n_observers, d.plan.stream_nblk, d.plan.surf_bytes).surf;
     prm.surf_bytes = d.plan.surf_bytes;
-    const int smem = template_smem_bytes(area);
-    static std::once_flag once[16];
-    int dev = 0;
-    GB_CUDA(cudaGetDevice(&dev));
-    cudaError_t err = cudaSuccess;
-    std::call_once(once[dev & 15], [&]() {
-      err = cudaFuncSetAttribute(k_template<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, template_smem_bytes(GB_MAX_TEMPLATE_SIDE * GB_MAX_TEMPLATE_SIDE));
-    });
-    if (err != cudaSuccess) return fail(GB_E_CUDA, "k_template attributes: %s", cudaGetErrorString(err));
-    k_template<true><<<(unsigned)(prm.P * prm.n_slots), 256, smem, stream>>>(prm);
+    k_template<true><<<(unsigned)(prm.P * prm.n_slots), 256, template_smem_bytes(area), stream>>>(prm);
   }
+  ++launches;
   GB_CUDA(cudaGetLastError());
+  return GB_OK;
+}
+
+static void launch_surface(const StepParams& prm, const FrameMaps& fm, cudaStream_t s, int64_t& launches) {
+  if (prm.tile_w * prm.tile_h > GB_SMEM_TEMPLATE)
+    k_s2_surface<true><<<(unsigned)(prm.pb * prm.n_slots), GB_S2_THREADS, prm.s2_smem, s>>>(prm, fm, prm.s2_budget);
+  else
+    k_s2_surface<false><<<(unsigned)(prm.pb * prm.n_slots), GB_S2_THREADS, prm.s2_smem, s>>>(prm, fm, prm.s2_budget);
+  ++launches;
+}
+
+static void launch_weights(const StepParams& prm, cudaStream_t s, int64_t& launches) {
+  if (spline_is_hermite(prm.interp_cols, prm.interp_rows))
+    k_s3_weights<false><<<dim3((unsigned)prm.s_nblk, (unsigned)prm.pb), s3_threads(prm.s_block), 0, s>>>(prm);
+  else
+    k_s3_weights<true><<<dim3((unsigned)prm.s_nblk, (unsigned)prm.pb), s3_threads(prm.s_block), 0, s>>>(prm);
+  ++launches;
+}
+
+// One batch of the step-by-step flow: k_s0 k_s1 k_s2 k_s3 k_s4* k_s5 (gb_track for choice / residual, gb_track_step).
+template <bool COV>
+static int step_batch(const StepParams& prm, const FrameMaps& fm, cudaStream_t s, int64_t& launches) {
+  const unsigned nb = (unsigned)(prm.pb * prm.s_nblk);
+  k_s0_reset<<<grid_for(prm.pb * prm.slot_stride * 5, 256), 256, 0, s>>>(prm);
+  ++launches;
+  k_s1_propagate<<<nb, GB_SBLOCK_THREADS, 0, s>>>(prm);
+  ++launches;
+  launch_surface(prm, fm, s, launches);
+  launch_weights(prm, s, launches);
+  if (prm.resample_method == GB_RESAMPLE_CHOICE || prm.resample_method == GB_RESAMPLE_RESIDUAL) {
+    if (prm.resample_method == GB_RESAMPLE_CHOICE)
+      k_s4c_scan<<<nb, GB_SBLOCK_THREADS, 0, s>>>(prm);
+    else
+      k_s4r_residual<<<(unsigned)prm.pb, GB_SBLOCK_THREADS, 0, s>>>(prm);
+    ++launches;
+    k_s4c_gather<COV><<<nb, GB_SBLOCK_THREADS, 0, s>>>(prm);
+  } else {
+    k_s4_resample<COV><<<nb, GB_SBLOCK_THREADS, 0, s>>>(prm);
+  }
+  ++launches;
+  k_s5_finalize<COV><<<(unsigned)((prm.pb + 3) / 4), 128, 0, s>>>(prm);
+  ++launches;
+  GB_CUDA(cudaGetLastError());
+  return GB_OK;
+}
+
+// One batch of the pipelined flow: [k_s0p] k_s2 k_s3 k_s3b k_s4p k_s5p, k_s4p advancing the particles to the time `nxt`
+// describes.  `activity`: k_s0p writes the activity of this time; `update`: some point of the call is updated at it.
+static int pipelined_batch(const StepParams& prm, const FrameMaps& fm, const NextParams& nxt, bool activity, bool update, bool cov,
+                           bool tangent, cudaStream_t s, int64_t& launches) {
+  KernelTimer& kt = g_ktimer;
+  if (activity) {
+    kt.begin(GB_K_ACTIVITY, s);
+    k_s0p_activity<<<grid_for(prm.pb, 256), 256, 0, s>>>(prm);
+    kt.end(s);
+    ++launches;
+  }
+  if (update) {
+    kt.begin(GB_K_SURFACE, s);
+    launch_surface(prm, fm, s, launches);
+    kt.end(s);
+    kt.begin(GB_K_WEIGHTS, s);
+    launch_weights(prm, s, launches);
+    kt.end(s);
+    kt.begin(GB_K_PUBLISH, s);
+    k_s3b_publish<<<(unsigned)((prm.pb + 7) / 8), 256, 0, s>>>(prm);
+    kt.end(s);
+    ++launches;
+  }
+  kt.begin(GB_K_RESAMPLE_PROPAGATE, s);
+  const dim3 grid((unsigned)prm.s_nblk, (unsigned)prm.pb);
+  if (cov && tangent)
+    k_s4p_resample_propagate<true, true><<<grid, GB_S4P_THREADS, kS4pSmem, s>>>(prm, nxt);
+  else if (cov)
+    k_s4p_resample_propagate<true, false><<<grid, GB_S4P_THREADS, kS4pSmem, s>>>(prm, nxt);
+  else if (tangent)
+    k_s4p_resample_propagate<false, true><<<grid, GB_S4P_THREADS, kS4pSmem, s>>>(prm, nxt);
+  else
+    k_s4p_resample_propagate<false, false><<<grid, GB_S4P_THREADS, kS4pSmem, s>>>(prm, nxt);
+  kt.end(s);
+  ++launches;
+  kt.begin(GB_K_FINALIZE, s);
+  if (cov)
+    k_s5p_finalize<true><<<(unsigned)((prm.pb + 3) / 4), 128, 0, s>>>(prm);
+  else
+    k_s5p_finalize<false><<<(unsigned)((prm.pb + 3) / 4), 128, 0, s>>>(prm);
+  kt.end(s);
+  ++launches;
+  GB_CUDA(cudaGetLastError());
+  return GB_OK;
+}
+
+// What k_s4p needs of time t + 1 (no slots after the last time).  `spec_update`: no point starts at t.
+static NextParams next_params(const gb_track_desc& d, int t, bool spec_update) {
+  NextParams nxt;
+  memset(&nxt, 0, sizeof(nxt));
+  for (int o = 0; o < GB_MAX_OBS; ++o) nxt.img[o] = -1;
+  nxt.spec_update = spec_update;
+  if (t + 1 < d.T) {
+    StepParams pn;
+    fill_params(d, t + 1, pn);
+    nxt.tau = pn.tau;
+    nxt.tau2 = pn.tau2;
+    nxt.n_slots = pn.n_slots;
+    for (int s = 0; s < pn.n_slots; ++s) {
+      nxt.obs[s] = pn.obs[s];
+      nxt.img[s] = pn.img[s];
+      nxt.cam[s] = pn.cam[s];
+    }
+  }
+  return nxt;
+}
+
+// What gb_track does at each time, from the host copies of first / last / mask (tracker.py:321-347).  A time without init
+// or update work is idle: a point is advanced from t to t + 1 only at times it starts or is updated at.
+struct TimeWork {
+  bool init;       // a point starts (k_init)
+  bool tmpl;       // an observer's template is cut (k_template)
+  bool update;     // a point that started earlier is updated
+  bool staggered;  // a template is cut after its point's first frame
+};
+struct Schedule {
+  std::vector<TimeWork> at;
+  bool staggered = false;  // at any time
+};
+
+static Schedule schedule(const gb_track_desc& d) {
+  Schedule s;
+  s.at.assign(d.T, TimeWork{});
+  std::vector<int> tmpl_frame(d.O);
+  for (int o = 0; o < d.O; ++o) tmpl_frame[o] = template_frame(d, o);
+  for (int64_t p = 0; p < d.P; ++p) {
+    const int f = d.first_host[p], l = d.last_host[p] < d.T ? d.last_host[p] : d.T - 1;
+    if (f < 0 || f >= d.T || l < f) continue;
+    s.at[f].init = true;
+    for (int t = f + 1; t <= l; ++t) s.at[t].update = true;
+    for (int o = 0; o < d.O; ++o) {
+      const int tf = tmpl_frame[o];
+      if (tf >= f && tf <= l && d.mask_host[p * d.O + o]) {
+        s.at[tf].tmpl = true;
+        if (tf > f) s.at[tf].staggered = s.staggered = true;
+      }
+    }
+  }
+  return s;
+}
+
+// gb_track.  The pipelined flow (systematic / stratified resampling) advances the particles to the next time in k_s4p of
+// this one; the step-by-step flow (choice / residual) moves them in k_s1 of the next update, or on the caller's stream
+// ahead of a template that is cut after a point's first frame.  The flows differ only in what the caller's stream runs at
+// a time and in the kernels of one batch.
+static int track(const gb_track_desc& d, cudaStream_t stream, int64_t& launches) {
+  const bool pipelined = d.resample_method != GB_RESAMPLE_CHOICE && d.resample_method != GB_RESAMPLE_RESIDUAL;
+  const bool cov = d.covariances != nullptr;
+  // kernels without the tangent models' DEM gathers when the caller says no point uses them (0 = unknown: assume any kind)
+  const bool tangent = d.motion_kinds == 0 || (d.motion_kinds & ((1 << GB_MOTION_TANGENT_CARTESIAN) | (1 << GB_MOTION_TANGENT_CYLINDRICAL))) != 0;
+  const Schedule work = schedule(d);
+  if (work.staggered && !d.weight_state)
+    return fail(GB_E_INVALID, "weight_state is required when a template starts after a point's first frame%s");
+  SideStreams sides(d, stream);
+  int rc = sides.open();
+  if (rc) return rc;
+  if (pipelined) {
+    StepParams prm;
+    fill_params(d, 0, prm);
+    stream_bind(d, prm, 0, 0, d.P);
+    k_s0p_reset<<<grid_for(d.P * prm.slot_stride * 5, 256), 256, 0, stream>>>(prm);
+    ++launches;
+    GB_CUDA(cudaGetLastError());
+  }
+  bool have_activity = false;
+  for (int t = 0; t < d.T; ++t) {
+    const TimeWork& w = work.at[t];
+    if (!w.init && !w.update) {
+      have_activity = false;  // a gap: the last k_s5p wrote the activity of a time that is not processed
+      continue;
+    }
+    StepParams prm;
+    fill_params(d, t, prm);
+    FrameMaps fm;
+    frame_maps(prm, fm);
+    if (w.init || w.tmpl) {
+      if ((rc = sides.join()) || (rc = wait_frames(d, prm, stream))) return rc;
+      if (pipelined) {
+        stream_bind(d, prm, t, 0, d.P);
+        prm.tmpl_from_ev = 1;
+        if (w.init) {
+          g_ktimer.begin(GB_K_INIT, stream);
+          if ((rc = launch_init(prm, cov, stream, launches))) return rc;
+          g_ktimer.end(stream);
+        }
+        if (w.tmpl) {
+          g_ktimer.begin(GB_K_TEMPLATE, stream);
+          if ((rc = launch_template(d, prm, stream, launches))) return rc;
+          g_ktimer.end(stream);
+        }
+      } else {
+        if (w.init && (rc = launch_init(prm, cov, stream, launches))) return rc;
+        if (w.staggered) {
+          dim3 grid((unsigned)grid_for(d.N, 256), (unsigned)d.P, 1);
+          k_evolve<<<grid, 256, 0, stream>>>(d.motion, d.surfaces, d.P, d.N, prm.tau, prm.tau2, d.step_normals,
+                                             (int64_t)(d.T - 1) * d.N * 3, ((t - 1) & 1) ? d.state_b : d.state_a, d.first, d.last,
+                                             d.status, d.status_time, t, d.rng_mode, d.seed, d.T - 1, d.point_offset);
+          ++launches;
+          GB_CUDA(cudaGetLastError());
+          prm.skip_evolve = 1;
+        }
+        if (w.tmpl && (rc = launch_template(d, prm, stream, launches))) return rc;
+      }
+    }
+    if (!pipelined && !w.update) continue;  // (that flow's batches only update)
+    if ((rc = sides.fork())) return rc;
+    if (w.update && (rc = sides.wait_frames(prm))) return rc;
+    if (pipelined) {
+      const NextParams nxt = next_params(d, t, !w.init);
+      // activity of time t: written by k_s5p of the previous processed time unless statuses may have changed since
+      const bool activity = !have_activity || w.init || w.tmpl;
+      have_activity = true;
+      rc = sides.each_batch(prm, [&](const StepParams& b, cudaStream_t s) {
+        return pipelined_batch(b, fm, nxt, activity, w.update, cov, tangent, s, launches);
+      });
+    } else {
+      rc = sides.each_batch(prm, [&](const StepParams& b, cudaStream_t s) {
+        return cov ? step_batch<true>(b, fm, s, launches) : step_batch<false>(b, fm, s, launches);
+      });
+    }
+    if (rc) return rc;
+  }
+  if ((rc = sides.join())) return rc;
+  if (g_ktimer.on) {
+    GB_CUDA(cudaStreamSynchronize(stream));
+    g_ktimer.collect();
+  }
   return GB_OK;
 }
 
@@ -1952,11 +1963,12 @@ int gb_track_init(const gb_track_desc* d, int32_t t, void* stream) {
   int rc = check_desc(*d);
   if (rc) return rc;
   if (t < 0 || t >= d->T) return fail(GB_E_INVALID, "time index out of range%s");
-  if ((rc = ensure_tables())) return rc;
+  if ((rc = ensure_device())) return rc;
   StepParams prm;
   fill_params(*d, t, prm);
-  if ((rc = launch_init(prm, d->covariances != nullptr, (cudaStream_t)stream))) return rc;
-  return launch_template(*d, prm, (cudaStream_t)stream);
+  int64_t launches = 0;
+  if ((rc = launch_init(prm, d->covariances != nullptr, (cudaStream_t)stream, launches))) return rc;
+  return launch_template(*d, prm, (cudaStream_t)stream, launches);
 }
 
 int gb_track_step(const gb_track_desc* d, int32_t t, const gb_stage_io* io, void* stream) {
@@ -1964,102 +1976,32 @@ int gb_track_step(const gb_track_desc* d, int32_t t, const gb_stage_io* io, void
   int rc = check_desc(*d);
   if (rc) return rc;
   if (t < 1 || t >= d->T) return fail(GB_E_INVALID, "time index out of range%s");
-  if ((rc = ensure_tables())) return rc;
+  if ((rc = ensure_device())) return rc;
   if ((rc = ensure_tensor_maps(*d))) return rc;
   StepParams prm;
   fill_params(*d, t, prm);
   if (io) prm.io = *io;
-  return launch_update(*d, prm, (cudaStream_t)stream, true, true, nullptr);
+  FrameMaps fm;
+  frame_maps(prm, fm);
+  const bool cov = d->covariances != nullptr;
+  int64_t launches = 0;
+  SideStreams sides(*d, (cudaStream_t)stream);
+  if ((rc = sides.open()) || (rc = sides.fork()) || (rc = sides.wait_frames(prm))) return rc;
+  rc = sides.each_batch(prm, [&](const StepParams& b, cudaStream_t s) {
+    return cov ? step_batch<true>(b, fm, s, launches) : step_batch<false>(b, fm, s, launches);
+  });
+  return rc ? rc : sides.join();
 }
 
-int gb_track(const gb_track_desc* d, void* stream_, int64_t* launches_out) {
+int gb_track(const gb_track_desc* d, void* stream, int64_t* launches_out) {
   if (!d) return fail(GB_E_INVALID, "null descriptor%s");
   int rc = check_desc(*d);
   if (rc) return rc;
   if (!d->mask_host || !d->first_host || !d->last_host) return fail(GB_E_INVALID, "host copies of mask/first/last required%s");
-  if ((rc = ensure_tables())) return rc;
-  cudaStream_t stream = (cudaStream_t)stream_;
+  if ((rc = ensure_device())) return rc;
   if ((rc = ensure_tensor_maps(*d))) return rc;
-  const bool cov = d->covariances != nullptr;
   int64_t launches = 0;
-  if (d->resample_method != GB_RESAMPLE_CHOICE && d->resample_method != GB_RESAMPLE_RESIDUAL) {  // (those two: step-by-step flow below)
-    if ((rc = track_streaming(*d, stream, &launches))) return rc;
-    if (launches_out) *launches_out = launches;
-    return GB_OK;
-  }
-  // per-time work flags from the host copies (tracker.py:321-347)
-  std::vector<int> tmpl_frame(d->O);
-  for (int o = 0; o < d->O; ++o) tmpl_frame[o] = template_frame(*d, o);
-  // In GB_MODE_STREAM the updates run on side streams that advance batch by batch without meeting; the
-  // caller's stream forks them after its own kernels (init, templates, in-place evolve) and joins them
-  // before the next such kernel and at the end.
-  bool forked = false, need_fork = true;
-  const bool streaming = true;
-  auto join_sides = [&]() -> int {
-    if (!streaming || !forked) return GB_OK;
-    StreamPool* pool = nullptr;
-    int rcj = get_pool(&pool);
-    if (rcj) return rcj;
-    for (int k = 0; k < d->plan.stream_slots; ++k) {
-      GB_CUDA(cudaEventRecord(pool->join[k], pool->side[k]));
-      GB_CUDA(cudaStreamWaitEvent(stream, pool->join[k], 0));
-    }
-    forked = false;
-    need_fork = true;
-    return GB_OK;
-  };
-  for (int t = 0; t < d->T; ++t) {
-    bool any_init = false, any_step = false, any_tmpl = false, staggered = false;
-    for (int64_t p = 0; p < d->P; ++p) {
-      const int f = d->first_host[p], l = d->last_host[p];
-      if (f == t && l >= t) any_init = true;
-      if (f < t && t <= l) any_step = true;
-      if (f <= t && t <= l)
-        for (int o = 0; o < d->O; ++o)
-          if (tmpl_frame[o] == t && d->mask_host[p * d->O + o]) {
-            any_tmpl = true;
-            if (f < t) staggered = true;
-          }
-    }
-    if (!any_init && !any_step) continue;
-    StepParams prm;
-    fill_params(*d, t, prm);
-    if (any_init || staggered || any_tmpl) {
-      if ((rc = join_sides())) return rc;
-      if (d->image_events_host)
-        for (int s = 0; s < prm.n_slots; ++s)
-          if (prm.img[s] >= 0 && d->image_events_host[prm.img[s]])
-            GB_CUDA(cudaStreamWaitEvent(stream, (cudaEvent_t)d->image_events_host[prm.img[s]], 0));
-    }
-    if (any_init) {
-      if ((rc = launch_init(prm, cov, stream))) return rc;
-      ++launches;
-    }
-    if (staggered) {
-      if (!d->weight_state) return fail(GB_E_INVALID, "weight_state is required when a template starts after a point's first frame%s");
-      dim3 grid((unsigned)grid_for(d->N, 256), (unsigned)d->P, 1);
-      k_evolve<<<grid, 256, 0, stream>>>(d->motion, d->surfaces, d->P, d->N, prm.tau, prm.tau2, d->step_normals,
-                                         (int64_t)(d->T - 1) * d->N * 3, ((t - 1) & 1) ? d->state_b : d->state_a, d->first, d->last,
-                                         d->status, d->status_time, t, d->rng_mode, d->seed, d->T - 1, d->point_offset);
-      GB_CUDA(cudaGetLastError());
-      ++launches;
-      prm.skip_evolve = 1;
-    }
-    if (any_tmpl) {
-      if ((rc = launch_template(*d, prm, stream))) return rc;
-      ++launches;
-    }
-    if (any_step) {
-      if (!streaming && d->image_events_host)
-        for (int s = 0; s < prm.n_slots; ++s)
-          if (prm.img[s] >= 0 && d->image_events_host[prm.img[s]])
-            GB_CUDA(cudaStreamWaitEvent(stream, (cudaEvent_t)d->image_events_host[prm.img[s]], 0));
-      if ((rc = launch_update(*d, prm, stream, need_fork, false, &launches))) return rc;
-      forked = true;
-      need_fork = false;
-    }
-  }
-  if ((rc = join_sides())) return rc;
+  if ((rc = track(*d, (cudaStream_t)stream, launches))) return rc;
   if (launches_out) *launches_out = launches;
   return GB_OK;
 }
@@ -2098,7 +2040,7 @@ int gb_sample_surface(const double* tile, int32_t rows, int32_t cols, int32_t kx
   if (kx < 1 || kx > 5 || ky < 1 || ky > 5) return fail(GB_E_INVALID, "spline degrees 1 to 5 are supported%s");
   if (rows < kx + 1 || cols < ky + 1 || rows > GB_MAX_SURFACE || cols > GB_MAX_SURFACE)
     return fail(GB_E_INVALID, "tile must have between degree + 1 and 1024 cells per axis%s");
-  int rc = ensure_tables();
+  int rc = ensure_device();
   if (rc) return rc;
   k_sample_surface<<<1, 256, 0, (cudaStream_t)stream>>>(tile, cols, rows, ky, kx, xy, n, reinterpret_cast<float4*>(work), out);
   GB_CUDA(cudaGetLastError());

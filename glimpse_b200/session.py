@@ -276,14 +276,22 @@ def plan_template_flags(tw: int, th: int) -> int:
     return _lib.GB_PLAN_LARGE_TEMPLATES if tw * th > _lib.GB_MAX_TEMPLATE else 0
 
 
-def session_bytes(lib, mode: int, cluster: int, P: int, N: int, T: int, O: int, tw: int, th: int, return_covariances: bool,
+def plan_flags(observers, image_index, tw: int, th: int) -> int:
+    """The flags of a track's launch plan: ranked frames when some frame it reads is not uint8, and the flag of its template size."""
+    ranked = _lib.GB_PLAN_RANKED_FRAMES if frames_need_ranks(observers, image_index) else 0
+    return ranked | plan_template_flags(tw, th)
+
+
+def session_bytes(lib, observers, image_index, P: int, N: int, T: int, O: int, tw: int, th: int, return_covariances: bool,
                   return_particles: bool, window_margin: int = _lib.GB_WINDOW_MARGIN, slots: Optional[int] = None) -> int:
     """Device memory one :class:`Session` of ``P`` points allocates (the frames excluded): two particle-state buffers,
-    the weights, the launch plan's scratch, templates and result blocks.  ``slots``: the plan's observer slots
+    the weights, the launch plan's scratch, templates and result blocks.  ``observers`` / ``image_index``: the frames the
+    track reads, which decide the plan's flags (:func:`plan_flags`).  ``slots``: the plan's observer slots
     (:func:`plan_slots`; default ``O``), which size the scratch; templates and results are sized by ``O``."""
     plan = _lib.gb_plan()
-    flags = int(cluster) | plan_template_flags(tw, th)
-    _lib.check(lib.gb_step_plan_ex(N, tw, th, P, O if slots is None else int(slots), flags, mode, int(window_margin), C.byref(plan)))
+    flags = plan_flags(observers, image_index, tw, th)
+    _lib.check(lib.gb_step_plan_ex(N, tw, th, P, O if slots is None else int(slots), flags, _lib.GB_MODE_STREAM, int(window_margin),
+                                   C.byref(plan)))
     per_point = 2 * 48 * N + 8 * N                      # state_a, state_b, weight_state
     per_point += 3 * O * tw * th * 8 + O * 40           # templates
     per_point += T * ((36 if return_covariances else 6) + 6) * 8 + T * O * 9 + 16  # moments, flags, window sizes, status
@@ -292,15 +300,15 @@ def session_bytes(lib, mode: int, cluster: int, P: int, N: int, T: int, O: int, 
     return int(plan.scratch_bytes) + P * per_point
 
 
-def points_per_session(lib, mode: int, cluster: int, P: int, budget: int, **shape) -> int:
+def points_per_session(lib, observers, image_index, P: int, budget: int, **shape) -> int:
     """Largest number of points (<= P) whose session fits ``budget`` bytes (at least 1): points are independent, so a
     track that does not fit the device runs as consecutive sessions of this many points."""
-    if session_bytes(lib, mode, cluster, P, **shape) <= budget:
+    if session_bytes(lib, observers, image_index, P, **shape) <= budget:
         return P
     lo, hi = 1, P  # session_bytes grows with the number of points
     while hi - lo > 1:
         mid = (lo + hi) // 2
-        if session_bytes(lib, mode, cluster, mid, **shape) <= budget:
+        if session_bytes(lib, observers, image_index, mid, **shape) <= budget:
             lo = mid
         else:
             hi = mid
@@ -332,13 +340,11 @@ class Session:
         with torch.cuda.device(device):
             self.stream = torch.cuda.current_stream().cuda_stream
             self.plan = _lib.gb_plan()
-            mode = _lib.GB_MODE_STREAM
             if window_margin is None:
                 window_margin = getattr(tracker, "window_margin", _lib.GB_WINDOW_MARGIN)
-            flags = _lib.GB_PLAN_RANKED_FRAMES if frames_need_ranks(tracker.observers, self.image_index) else 0
-            flags |= plan_template_flags(self.tw, self.th)
-            _lib.check(self.lib.gb_step_plan_ex(N, self.tw, self.th, P, plan_slots(self.image_index), flags, mode, int(window_margin),
-                                                C.byref(self.plan)))
+            flags = plan_flags(tracker.observers, self.image_index, self.tw, self.th)
+            _lib.check(self.lib.gb_step_plan_ex(N, self.tw, self.th, P, plan_slots(self.image_index), flags, _lib.GB_MODE_STREAM,
+                                                int(window_margin), C.byref(self.plan)))
             self.h2d = 0
             # the first two frames' uploads start right away (the first kernels wait for them); the other big copies are
             # queued after the small tables, which they would otherwise hold up on the copy engine for tens of ms

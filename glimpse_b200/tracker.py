@@ -547,7 +547,6 @@ class Tracker:
                         frames += int(array.nbytes) if array is not None else 3 * int(np.prod(obs.images[i].size))
                     except (AttributeError, TypeError):
                         pass  # size unknown before the frame is read: the 10 % margin has to cover it
-        mode = _lib.GB_MODE_STREAM
         shape = dict(N=int(models[0].n), T=image_index.shape[0], O=image_index.shape[1], tw=tile_size[0], th=tile_size[1],
                      return_covariances=return_covariances, return_particles=return_particles, window_margin=int(self.window_margin),
                      slots=_session.plan_slots(image_index))
@@ -555,11 +554,11 @@ class Tracker:
         # the common case costs no driver call: a track needing less than a quarter of the device is not measured against
         # the free memory (cudaMemGetInfo takes from a fraction of a millisecond to several)
         total = torch.cuda.get_device_properties(device).total_memory
-        if _session.session_bytes(lib, mode, 0, cap, **shape) + frames <= total // 4:
+        if _session.session_bytes(lib, self.observers, image_index, cap, **shape) + frames <= total // 4:
             return cap
         free, _total = torch.cuda.mem_get_info(device)
         free += torch.cuda.memory_reserved(device) - torch.cuda.memory_allocated(device)
-        return _session.points_per_session(lib, mode, 0, cap, int(0.9 * max(free - frames, 0)), **shape)
+        return _session.points_per_session(lib, self.observers, image_index, cap, int(0.9 * max(free - frames, 0)), **shape)
 
     # ------------------------------------------------------------------ multi-GPU: one final gather
     @staticmethod

@@ -357,11 +357,13 @@ def test_blocks_of_points_give_the_same_track(cuda, rng):
     assert len(runs[1][1].last_run["window_width"]) == len(runs[0][1].last_run["window_width"])
 
 
+@pytest.mark.parametrize("method", ["systematic", "choice", "residual"])
 @pytest.mark.parametrize("slots,batch", [(1, 7), (4, 2), (4, 1), (2, 5)])
-def test_the_batch_plan_does_not_change_the_track(cuda, monkeypatch, slots, batch):
+def test_the_batch_plan_does_not_change_the_track(cuda, monkeypatch, slots, batch, method):
     """gb_track cuts the points into batches that advance on their own streams (one batch for few points, up to four): points are
     independent and Philox counters are global, so every plan gives bit-identical results — also with an observer that starts
-    later (templates join the batches) and a point that fails on the way."""
+    later (templates join the batches) and a point that fails on the way.  'systematic' runs the pipelined flow, 'choice' and
+    'residual' the step-by-step one."""
     import glimpse_b200 as gb
 
     scene = synthetic.nadir_scene(seed=31, n_points=7, n_particles=700, n_frames=7, imgsz=(400, 300), margin_px=100)
@@ -370,10 +372,11 @@ def test_the_batch_plan_does_not_change_the_track(cuda, monkeypatch, slots, batc
     observers, models = synthetic.build(scene, gb)
     with warnings.catch_warnings():
         warnings.simplefilter("ignore")
-        base = gb.Tracker(observers, seed=9).track(models, tile_size=scene.tile_size, return_covariances=True, return_particles=True)
+        base = gb.Tracker(observers, seed=9, resample_method=method).track(models, tile_size=scene.tile_size, return_covariances=True,
+                                                                         return_particles=True)
         monkeypatch.setenv("GB_STREAM_SLOTS", str(slots))
         monkeypatch.setenv("GB_STREAM_BATCH", str(batch))
-        tracker = gb.Tracker(observers, seed=9)
+        tracker = gb.Tracker(observers, seed=9, resample_method=method)
         other = tracker.track(models, tile_size=scene.tile_size, return_covariances=True, return_particles=True)
     plan = tracker.last_run["plan"]
     assert plan["stream_slots"] == slots and plan["stream_batch"] == batch
@@ -382,6 +385,22 @@ def test_the_batch_plan_does_not_change_the_track(cuda, monkeypatch, slots, batc
     np.testing.assert_array_equal(other.means, base.means)
     np.testing.assert_array_equal(other.covariances, base.covariances)
     np.testing.assert_array_equal(other.particles, base.particles)
+
+
+def test_kernel_launches_of_the_step_by_step_flow(cuda, monkeypatch):
+    """Tracker.last_run['kernel_launches'] of a 'choice' track counts what gb_track launched: per batch of points and update
+    k_s0 k_s1 k_s2 k_s3 k_s4c_scan k_s4c_gather k_s5, and k_init and k_template at the first time."""
+    import glimpse_b200 as gb
+
+    scene = synthetic.nadir_scene(seed=2, n_points=3, n_particles=500, n_frames=4, imgsz=(320, 240), margin_px=90)
+    observers, models = synthetic.build(scene, gb)
+    monkeypatch.setenv("GB_STREAM_SLOTS", "2")
+    monkeypatch.setenv("GB_STREAM_BATCH", "2")
+    tracker = gb.Tracker(observers, seed=3, resample_method="choice")
+    tracks = tracker.track(models, tile_size=scene.tile_size)
+    assert all(e is None for e in tracks.errors)
+    batches, updates = 2, 3
+    assert tracker.last_run["kernel_launches"] == 7 * batches * updates + 1 + 1
 
 
 @pytest.mark.parametrize("kind", ["cartesian", "cylindrical", "tangent_cartesian", "tangent_cylindrical"])

@@ -368,15 +368,45 @@ def test_points_are_blocked_by_device_memory():
 
     build.build()
     lib = _lib.load()
+    frames = ([], None)  # no frame to read: the plan of uint8 frames
     shape = dict(N=10000, T=365, O=1, tw=15, th=15, return_covariances=False, return_particles=False)
-    whole = session_bytes(lib, _lib.GB_MODE_STREAM, 0, 100000, **shape)
+    whole = session_bytes(lib, *frames, 100000, **shape)
     assert 250e9 < whole < 350e9
-    assert session_bytes(lib, _lib.GB_MODE_STREAM, 0, 12500, **shape) < 45e9
-    block = points_per_session(lib, _lib.GB_MODE_STREAM, 0, 100000, int(160e9), **shape)
+    assert session_bytes(lib, *frames, 12500, **shape) < 45e9
+    block = points_per_session(lib, *frames, 100000, int(160e9), **shape)
     assert 45000 < block < 65000
-    assert session_bytes(lib, _lib.GB_MODE_STREAM, 0, block, **shape) <= 160e9 < session_bytes(lib, _lib.GB_MODE_STREAM, 0, block + 1, **shape)
-    assert points_per_session(lib, _lib.GB_MODE_STREAM, 0, 1000, int(160e9), **shape) == 1000
-    assert points_per_session(lib, _lib.GB_MODE_STREAM, 0, 1000, 1, **shape) == 1  # never less than one point
+    assert session_bytes(lib, *frames, block, **shape) <= 160e9 < session_bytes(lib, *frames, block + 1, **shape)
+    assert points_per_session(lib, *frames, 1000, int(160e9), **shape) == 1000
+    assert points_per_session(lib, *frames, 1000, 1, **shape) == 1  # never less than one point
+
+
+def test_session_bytes_plan_ranked_frames_as_the_session_does():
+    """A uint16 observer makes Session plan ranked frames, whose surface regions hold a rank histogram of the largest window
+    (twice the bytes at 15 x 15 and 10 000 particles).  session_bytes plans the same, so the blocks Tracker cuts a large
+    track into fit the device."""
+    from glimpse_b200 import _lib
+    from glimpse_b200.session import session_bytes
+
+    lib = _lib.load()
+    P, N, T, O, tw, th = 1000, 10000, 4, 2, 15, 15
+    observers = [_observers(T), _observers(T)]
+    index = np.array([[0, 0], [1, -1], [2, 1], [3, 2]])
+    shape = dict(N=N, T=T, O=O, tw=tw, th=th, return_covariances=False, return_particles=False)
+    uint8 = session_bytes(lib, observers, index, P, **shape)
+    for image in observers[1].images:
+        image.array = np.zeros((10, 20), dtype=np.uint16)
+    uint16 = session_bytes(lib, observers, index, P, **shape)
+    plans = {}
+    for flags in (0, _lib.GB_PLAN_RANKED_FRAMES):
+        plans[flags] = _lib.gb_plan()
+        assert lib.gb_step_plan_ex(N, tw, th, P, O, flags, _lib.GB_MODE_STREAM, _lib.GB_WINDOW_MARGIN, C.byref(plans[flags])) == 0
+    ranked = plans[_lib.GB_PLAN_RANKED_FRAMES]
+    # per point: particle states and weights, three template arrays and 40 B of template scalars per observer, moments and
+    # sigmas, flag bytes and window sizes per time and observer, status
+    per_point = 2 * 48 * N + 8 * N + O * (3 * tw * th * 8 + 40) + T * 12 * 8 + T * O * 9 + 16
+    assert uint16 == ranked.scratch_bytes + P * per_point
+    assert ranked.surf_bytes > plans[0].surf_bytes
+    assert uint16 - uint8 == P * O * (ranked.surf_bytes - plans[0].surf_bytes)
 
 
 def test_blocks_and_second_runs_are_assembled_on_the_host(monkeypatch):

@@ -54,8 +54,8 @@ def test_session_bytes_large_template():
 
     lib = _lib.load()
     shape = dict(N=1000, T=5, O=1, return_covariances=False, return_particles=False)
-    small = session_bytes(lib, _lib.GB_MODE_STREAM, 0, 10, tw=32, th=32, **shape)
-    large = session_bytes(lib, _lib.GB_MODE_STREAM, 0, 10, tw=64, th=64, **shape)
+    small = session_bytes(lib, [], None, 10, tw=32, th=32, **shape)
+    large = session_bytes(lib, [], None, 10, tw=64, th=64, **shape)
     assert large > small > 0
 
 

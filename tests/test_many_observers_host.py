@@ -58,17 +58,17 @@ def test_session_bytes_size_the_scratch_by_slots_and_the_templates_by_observers(
     from glimpse_b200.session import session_bytes
 
     lib = _lib.load()
-    S = _lib.GB_MODE_STREAM
+    frames = ([], None)  # no frame to read: the plan of uint8 frames
     shape = dict(N=1000, T=40, tw=15, th=15, return_covariances=False, return_particles=False)
-    twelve = session_bytes(lib, S, 0, 50, O=12, slots=3, **shape)
-    three = session_bytes(lib, S, 0, 50, O=3, **shape)
+    twelve = session_bytes(lib, *frames, 50, O=12, slots=3, **shape)
+    three = session_bytes(lib, *frames, 50, O=3, **shape)
     # per point and observer: three template arrays of w x h doubles and 40 B of template scalars; T flag bytes and window sizes
     per_observer = 3 * 15 * 15 * 8 + 40 + 40 * 9
     assert twelve - three == 50 * 9 * per_observer
-    assert three - 50 * 3 * per_observer == session_bytes(lib, S, 0, 50, O=1, slots=3, **shape) - 50 * per_observer
-    assert session_bytes(lib, S, 0, 50, O=3, slots=3, **shape) == three
+    assert three - 50 * 3 * per_observer == session_bytes(lib, *frames, 50, O=1, slots=3, **shape) - 50 * per_observer
+    assert session_bytes(lib, *frames, 50, O=3, slots=3, **shape) == three
     with pytest.raises(RuntimeError):  # twelve observers cannot have a slot each
-        session_bytes(lib, S, 0, 50, O=12, **shape)
+        session_bytes(lib, *frames, 50, O=12, **shape)
 
 
 def desc_with(O, T, index, plan_slots, N=4):
