@@ -1532,7 +1532,7 @@ __global__ void __launch_bounds__(GB_S4P_THREADS, GB_S4P_MINB) k_s4p_resample_pr
 }
 
 // s5 of the pipelined flow: moments and status of time t, then the failure flags of this parity are cleared
-// for time t + 2.  Also stores the moment origin of the next time (the first resampled particle).
+// for time t + 2.  The moments are taken about the point's moment origin, which k_init fixes from the prior.
 template <bool COV>
 __global__ void k_s5p_finalize(const __grid_constant__ StepParams prm) {
   const int64_t p = prm.p0 + ((blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5);
