@@ -5,19 +5,24 @@ A ``gb_track`` run with ``return_particles=True`` returns, for every point p and
 realised search-window sizes.  Given the outputs at t - 1 and the draws of t, update t is determined: the replay evolves
 ``particles[p, t - 1]`` with the oracle's motion step, computes the pre-resample weights (carried, uniform, DEM-only or
 through the oracle's closed-form tile pipeline), resamples with the oracle's ``systematic_indices`` /
-``stratified_indices``, and checks the device's update against it.  Each update starts from the device's own previous
+``stratified_indices`` (the pipelined flow) or ``choice_indices`` / ``residual_indices`` (the step-by-step flow), and checks
+the device's update against it.  Each update starts from the device's own previous
 outputs, so one flipped ancestor does not make the rest of the track diverge: every update is checked on its own.
 
 What ``replay_track`` asserts, per update:
 * propagation: every child row equals exactly one row of the evolved particles (rtol = atol = 1e-13, the tolerance of
   ``test_stand_alone_evolve_particles_matches_the_oracle``; the second nearest row is far outside it), which recovers the
   device's ancestors; at the first time the particles equal ``init_particles`` of the init draws and the weights are 1;
-* structure: ancestors non-decreasing, children of one parent bitwise-equal rows with bitwise-equal weights;
+* structure: children of one parent bitwise-equal rows with bitwise-equal weights; ancestors non-decreasing (systematic,
+  stratified; choice children are in draw order, residual ones repetitions first);
 * weights: carried and uniform updates bit for bit (``w_pre[k]``); DEM-only within ``DEM_REL`` (the ``exp_neg_fast``
   bound); observed within ``WEIGHT_REL``;
 * ancestors: equal to the reference's, or a near-tie: moved across one boundary b of the cumulative weights C (by one
   parent, or over parents whose weights add up to no more than the band) with |pos - C[b]| <= delta min(C[b], 1 - C[b]) + 1e-12, delta = 0 at carried / uniform updates, 2 DEM_REL at DEM-only ones,
-  2 WEIGHT_REL at observed ones;
+  2 WEIGHT_REL at observed ones; choice: the position is the child's uniform, C is normalised by C[-1];
+  residual (``check_residual``): bit-equal at carried / uniform updates; elsewhere the device's repetitions within the weight
+  noise of floor(N wn) and every additional child an answer NumPy's search can reach, comparisons within the noise going
+  either way;
 * moments: means, sigmas or covariances against a long-double reference of the device's own particles and weights, taken
   about particle 0 (means 1e-9 sigma, variances 2e-7 relative, covariances 1e-7 sqrt(c_ii c_jj), plus two float64 ulps of
   the value for the rounding of the stored result).  The device sums one pass of first and second moments about the
@@ -41,6 +46,8 @@ PROP_TOL = 1e-13   # motion step: rtol = atol
 SEED = 0x5EED_0F_A11  # the philox key of the GPU replay (the host coverage test restates its draws)
 KINDS = ("carried", "uniform", "dem", "observed")
 CHUNK = 768        # children per k_s4p chunk / particles per block at most
+EPS = np.finfo(float).eps
+STEP_METHODS = ("choice", "residual")  # resamplers of the step-by-step flow
 
 
 # ------------------------------------------------------------------------------------------------ scenes
@@ -69,17 +76,23 @@ def fine_dem_sigma(scene, cells=(140, 180), lo=0.01, hi=0.05):
     return scene
 
 
-def case(name, n_particles=None):
+def stream_block(N):
+    """gb_step_plan's particles per block for N particles: CHUNK at most, even, as equal as possible."""
+    nblk = -(-N // CHUNK)
+    return (-(-N // nblk) + 1) // 2 * 2
+
+
+def case(name, n_particles=None, method=None):
     """(scene, observer mask, resample method, covariances) of a replay case: every case has an interleaved observer (the
     last one) that the mask takes away from some points, so that they take updates without any image.  ``n_particles``
-    overrides the case's particle count (host tests of the replay itself).  ``scene.meta["kinds"]`` = the motion kind of
+    overrides the case's particle count (host tests of the replay itself), ``method`` its resampler.  ``scene.meta["kinds"]`` = the motion kind of
     every point where they differ, ``scene.meta["reverse"]`` = the track runs its datetimes backwards (``build``,
     ``inputs``, ``datetimes``)."""
     import scenes
     from glimpse_b200 import synthetic
 
     small = dict(imgsz=(320, 240), margin_px=100)
-    method, cov, later, kinds, reverse = "systematic", False, None, None, False
+    case_method, cov, later, kinds, reverse = "systematic", False, None, None, False
     if name == "tan_carried_collapse":
         scene = synthetic.nadir_scene(seed=61, n_points=1, n_particles=100000, n_frames=3, kind="tangent_cartesian", **small)
         scenes.add_gridded_dem(scene)
@@ -89,7 +102,7 @@ def case(name, n_particles=None):
         scene = synthetic.nadir_scene(seed=62, n_points=2, n_particles=9999, n_frames=3, kind="tangent_cylindrical",
                                       velocity_sigma=0.2, **small)
         scenes.add_gridded_dem(scene)
-        method, cov, masked = "stratified", True, [0]
+        case_method, cov, masked = "stratified", True, [0]
         later = 1  # sees the interleaved observer only: starts half a time unit after point 0
     elif name == "cart_dem_floor":
         scene = synthetic.nadir_scene(seed=63, n_points=2, n_particles=10000, n_frames=3, **small)
@@ -124,6 +137,7 @@ def case(name, n_particles=None):
         raise KeyError(name)
     if n_particles is not None:
         scene.n_particles = int(n_particles)
+    method = method or case_method
     scene.meta.update(kinds=kinds, reverse=reverse)
     interleave(scene)
     P, O = len(scene.points), len(scene.observers)
@@ -136,6 +150,10 @@ def case(name, n_particles=None):
 
 CASES = ["tan_carried_collapse", "tan_cyl_stratified_odd", "cart_dem_floor", "shape_c2_interleaved", "mixed_three_obs", "million",
          "small_2", "small_37", "small_769"]
+# the step-by-step flow (k_s1_propagate -> k_s2 -> k_s3 -> k_s4c_scan or k_s4r_residual -> k_s4c_gather -> k_s5_finalize):
+# (case, resampler); small_99005 takes uniform updates at N (1 / N) < 1, where the residual resampler has no repetitions
+STEP_CASES = [("tan_carried_collapse", "choice"), ("million", "choice"), ("mixed_three_obs", "choice"),
+              ("tan_cyl_stratified_odd", "residual"), ("cart_dem_floor", "residual"), ("small_99005", "residual")]
 
 
 def _kind_scene(scene, kind):
@@ -289,7 +307,10 @@ def moment_origin(spec):
     return np.array([xy[0], xy[1], 0.0 if np.isnan(z) else z, vxy[0], vxy[1], v[2]])
 
 
-def check_moments(rep, res, p, t, cov, tag, origin):
+def check_moments(rep, res, p, t, cov, tag, origin, terms=None):
+    """``terms``: a one-pass allowance of terms eps D on the means and terms eps D_i D_j on the (co)variances, for sums over a
+    chain of up to ``terms`` additions taken far from a collapsed cloud (test_gpu_resample_step).  None: the replay's own
+    allowance, 16 eps D_i D_j on the (co)variances and none on the means."""
     ps, w = res["particles"][p, t], res["weights"][p, t]
     mean, sig = moments_ref(ps, w, cov)
     got_m, got_s = res["means"][p, t], res["sigmas"][p, t]
@@ -297,22 +318,134 @@ def check_moments(rep, res, p, t, cov, tag, origin):
     mean = mean.astype(float)
     dm = np.abs(got_m - mean)
     ulp = lambda x: 2 * np.spacing(np.abs(x))  # noqa: E731
-    assert (dm <= 1e-9 * s + ulp(mean)).all(), f"{tag}: means {got_m} against {mean} (sigma {s})"
-    rep.worst("mean/sigma", np.max(np.where(s > 0, dm / np.where(s > 0, s, 1), 0)))
     step = np.abs(ps - origin).max(axis=0)
-    one_pass = 16 * np.finfo(float).eps * np.outer(step, step)
+    # the mean is r + E[d]: where the spread has collapsed the rounding of E[d], terms eps D, is all that is left
+    mean_pass = 0.0 if terms is None else terms * EPS * step
+    assert (dm <= 1e-9 * s + ulp(mean) + mean_pass).all(), f"{tag}: means {got_m} against {mean} (sigma {s})"
+    spread = s > 1e-7 * step  # (relative errors are reported where the spread has not collapsed)
+    rep.worst("mean/sigma", np.max(np.where(spread, dm / np.where(spread, s, 1), 0)))
+    rep.worst("mean abs where the spread collapsed", np.max(np.where(spread, 0, dm)))
+    one_pass = (16 if terms is None else terms) * EPS * np.outer(step, step)
     if cov:
         c = sig.astype(float)
         scale = np.sqrt(np.outer(s, s))
         dc = np.abs(got_s - c)
         assert (dc <= 1e-7 * scale + one_pass + ulp(c)).all(), \
             f"{tag}: covariances off by {np.max(dc / np.maximum(scale, 1e-300))} of sqrt(c_ii c_jj)"
-        rep.worst("cov rel", np.max(np.where(scale > 0, dc / np.where(scale > 0, scale, 1), 0)))
+        both = np.outer(spread, spread)
+        rep.worst("cov rel", np.max(np.where(both, dc / np.where(both, scale, 1), 0)))
     else:
         dv = np.abs(got_s ** 2 - s ** 2)
         assert (dv <= 2e-7 * s ** 2 + np.diagonal(one_pass) + ulp(s ** 2)).all(), f"{tag}: sigmas {got_s} against {s}"
-        rep.worst("sigma rel", np.max(np.where(s > 0, np.abs(got_s - s) / np.where(s > 0, s, 1), 0)))
-        rep.worst("sigma abs where the spread collapsed", np.max(np.where(s <= 1e-7 * step, np.abs(got_s - s), 0)))
+        rep.worst("sigma rel", np.max(np.where(spread, np.abs(got_s - s) / np.where(spread, s, 1), 0)))
+        rep.worst("sigma abs where the spread collapsed", np.max(np.where(spread, 0, np.abs(got_s - s))))
+
+
+def check_near_ties(rep, anc, idx, w_pre, pos, delta, kind, tag, choice=False):
+    """The device's ancestors ``anc`` against the reference's ``idx``: equal, or a near-tie — moved across one boundary b of
+    the normalised cumulative weights C (by one parent, or over parents whose weights add up to no more than the band), the
+    child's position ``pos`` within delta min(C[b], 1 - C[b]) of C[b], plus the rounding of two summation orders of C (1e-12;
+    choice: C is normalised by C[-1] and divides the device's block-wise sums by their total, (N + 2) eps C at least).
+    Returns the differing children."""
+    flipped = np.nonzero(anc != idx)[0]
+    if len(flipped):
+        N = len(w_pre)
+        C = np.cumsum(w_pre / w_pre.sum())
+        if choice:
+            C /= C[-1]
+        a, b = np.minimum(anc[flipped], idx[flipped]), np.maximum(anc[flipped], idx[flipped])
+        slack = np.maximum(1e-12, (N + 2) * EPS * C[b - 1]) if choice else 1e-12
+        band = delta * np.minimum(C[a], 1 - C[a]) + slack
+        between = C[b - 1] - C[a]  # weight of the parents strictly between the two: inside the weight noise
+        assert (between <= band).all(), \
+            f"{tag}: children {flipped[:5].tolist()} have ancestors {anc[flipped[:5]].tolist()}, reference {idx[flipped[:5]].tolist()}"
+        pos = pos[flipped] if np.ndim(pos) else pos
+        gap = np.abs(pos - C[a])
+        assert (gap <= band).all(), \
+            f"{tag}: ancestors of children {flipped[:5].tolist()} differ beyond a near-tie (gaps {gap[:5].tolist()})"
+        print(f"{tag}: {len(flipped)} near-ties at a {kind} update, |position - boundary| {gap.max():.3g}, "
+              f"most parents crossed {int((b - a).max())}")
+    return flipped
+
+
+def searchsorted_reachable(cs, key, lo, hi, band):
+    """The answers np.searchsorted's binary search (side 'left', from the bounds [lo, hi)) can reach on ``cs`` when every
+    comparison with |cs[mid] - key| <= band may go either way."""
+    out, todo, seen = set(), [(lo, hi)], set()
+    while todo:
+        lo, hi = todo.pop()
+        if (lo, hi) in seen:
+            continue
+        seen.add((lo, hi))
+        if lo >= hi:
+            out.add(lo)
+            continue
+        mid = lo + ((hi - lo) >> 1)
+        d = cs[mid] - key
+        if d < 0 or abs(d) <= band:
+            todo.append((mid + 1, hi))
+        if d >= 0 or abs(d) <= band:
+            todo.append((lo, mid))
+    return out
+
+
+def carried_bounds(keys, prev, N):
+    """NumPy's search bounds (numpy/_core/src/npysort/binsearch.cpp) for each key after the previous key's search ended at
+    ``prev`` (its state is its answer): [prev, N) after a smaller key, else [0, min(prev + 1, N)).  The first key: [0, N)."""
+    lo, hi = np.zeros(len(keys), dtype=np.int64), np.full(len(keys), N, dtype=np.int64)
+    if len(keys) > 1:
+        up = keys[:-1] < keys[1:]
+        lo[1:] = np.where(up, prev, 0)
+        hi[1:] = np.where(up, N, np.minimum(prev + 1, N))
+    return lo, hi
+
+
+def check_residual(rep, anc, w_pre, row, delta, kind, tag):
+    """The residual resampler's ancestors (oracle.residual_indices: repetitions of floor(N wn), then np.searchsorted of the
+    uniforms ``row[:N - K]`` on the cumulative sum of wn - repetitions).  Exact weights (delta = 0): bit-equal to the
+    reference's.  Otherwise the repetitions may differ where the weight noise moves N wn across an integer: the device's K is
+    found among the last few children of the ancestors' longest non-decreasing prefix, its repetitions bincount(anc[:K]) must
+    lie within floor(N wn (1 -+ delta)), and every additional child must be an answer NumPy's search can reach on the
+    cumulative sum rebuilt from the reference's wn and those repetitions, starting from the device's previous answer, when
+    comparisons within the noise of that sum may go either way."""
+    N = len(w_pre)
+    if delta == 0:
+        ref, used = orc.residual_indices(w_pre, lambda m: row[:m])
+        bad = np.nonzero(anc != ref)[0]
+        assert len(bad) == 0, \
+            f"{tag}: K {N - len(used)}, children {bad[:5].tolist()} have ancestors {anc[bad[:5]].tolist()}, reference {ref[bad[:5]].tolist()}"
+        rep.count(f"residual K = 0 ({kind})", len(used) == N)
+        return
+    wn = w_pre / w_pre.sum()
+    reps_lo, reps_hi = np.floor(N * wn * (1 - delta)), np.floor(N * wn * (1 + delta))
+    dec = np.nonzero(np.diff(anc) < 0)[0]
+    prefix = int(dec[0]) + 1 if len(dec) else N
+    why = "no K satisfies the repetition bounds"
+    for K in range(prefix, max(prefix - 8, 0) - 1, -1):
+        reps = np.bincount(anc[:K], minlength=N)
+        if not ((reps_lo <= reps) & (reps <= reps_hi)).all():
+            continue
+        residuals = wn - reps
+        residuals *= 1 / residuals.sum()
+        cs = np.cumsum(residuals)
+        cs[-1] = 1.0
+        keys, got = row[:N - K], anc[K:]
+        # wn carries up to delta of relative error (tol in the weights, tol in their sum), so |d cs| <= delta (1 + |cs|) / |1 - K|
+        # (the residuals sum to 1 - K), plus the rounding of the sums
+        band = delta * (1 + np.abs(cs).max()) / max(abs(1 - K), 1) + (N + 2) * EPS * np.abs(cs).max()
+        lo, hi = carried_bounds(keys, got[:-1], N)
+        lo0, hi0 = lo.copy(), hi.copy()
+        while (lo < hi).any():  # the exact search from the device's state, every key at once
+            mid = lo + ((hi - lo) >> 1)
+            go = cs[np.minimum(mid, N - 1)] < keys
+            lo, hi = np.where((lo < hi) & go, mid + 1, lo), np.where((lo < hi) & ~go, mid, hi)
+        off = np.nonzero(lo != got)[0]
+        if all(int(got[i]) in searchsorted_reachable(cs, keys[i], int(lo0[i]), int(hi0[i]), band) for i in off):
+            rep.worst(f"residual repetitions off floor(N wn) ({kind})", np.abs(reps - np.floor(N * wn)).max(initial=0))
+            rep.count(f"residual searches within the noise ({kind})", len(off))
+            return
+        why = f"K {K}: additional children {off[:5].tolist()} unreachable"
+    raise AssertionError(f"{tag}: residual ancestors: {why} (non-decreasing prefix {prefix})")
 
 
 def replay_track(res, draws, scene_inputs, method, mask, tile_size, cov=False, windows=None, highpass_size=(5, 5), kx=3, ky=3):
@@ -409,14 +542,15 @@ def replay_track(res, draws, scene_inputs, method, mask, tile_size, cov=False, w
                 kind, w_pre = "dem", orc.weights_from_log_likelihoods([ll])
             rep.count(f"{kind} updates")
             u = unif[p, k]
-            idx = orc.stratified_indices(w_pre, u) if method == "stratified" else orc.systematic_indices(w_pre, u)
             children, w_got = res["particles"][p, t], res["weights"][p, t]
             anc, err = recover_ancestors(children, evolved)
             rep.worst(f"propagation ({kind})", err)
-            assert (np.diff(anc) >= 0).all(), f"{tag}: ancestors decrease at child {int(np.argmax(np.diff(anc) < 0))}"
-            same = anc[1:] == anc[:-1]
-            assert (children[1:][same] == children[:-1][same]).all(), f"{tag}: children of one parent differ"
-            assert (w_got[1:][same] == w_got[:-1][same]).all(), f"{tag}: weights of one parent's children differ"
+            if method in ("systematic", "stratified"):
+                assert (np.diff(anc) >= 0).all(), f"{tag}: ancestors decrease at child {int(np.argmax(np.diff(anc) < 0))}"
+            order = np.argsort(anc, kind="stable")  # (the identity where the ancestors are sorted)
+            same = anc[order][1:] == anc[order][:-1]
+            assert (children[order][1:][same] == children[order][:-1][same]).all(), f"{tag}: children of one parent differ"
+            assert (w_got[order][1:][same] == w_got[order][:-1][same]).all(), f"{tag}: weights of one parent's children differ"
             ref_w = w_pre[anc]
             if kind in ("carried", "uniform"):
                 bad = np.nonzero(w_got != ref_w)[0]
@@ -428,25 +562,21 @@ def replay_track(res, draws, scene_inputs, method, mask, tile_size, cov=False, w
                 assert rel <= tol, f"{tag}: {kind} weights {rel} from the reference's"
                 rep.worst(f"weight rel ({kind})", rel)
                 delta = 2 * tol
-            flipped = np.nonzero(anc != idx)[0]
-            if len(flipped):
-                C = np.cumsum(w_pre / w_pre.sum())
-                a, b = np.minimum(anc[flipped], idx[flipped]), np.maximum(anc[flipped], idx[flipped])
-                band = delta * np.minimum(C[a], 1 - C[a]) + 1e-12
-                between = C[b - 1] - C[a]  # weight of the parents strictly between the two: inside the weight noise
-                assert (between <= band).all(), \
-                    f"{tag}: children {flipped[:5].tolist()} have ancestors {anc[flipped[:5]].tolist()}, reference {idx[flipped[:5]].tolist()}"
+            if method == "residual":
+                check_residual(rep, anc, w_pre, u, delta, kind, tag)
+                flipped = ()
+            elif method == "choice":
+                flipped = check_near_ties(rep, anc, orc.choice_indices(w_pre, u), w_pre, u, delta, kind, tag, choice=True)
+            else:
+                idx = orc.stratified_indices(w_pre, u) if method == "stratified" else orc.systematic_indices(w_pre, u)
                 pos = (np.arange(len(w_pre)) + np.asarray(u)) * (1 / len(w_pre))
-                pos = pos[flipped] if pos.ndim else pos
-                gap = np.abs(pos - C[a])
-                assert (gap <= band).all(), \
-                    f"{tag}: ancestors of children {flipped[:5].tolist()} differ beyond a near-tie (gaps {gap[:5].tolist()})"
-                print(f"{tag}: {len(flipped)} near-ties at a {kind} update, |position - boundary| {gap.max():.3g}, "
-                      f"most parents crossed {int((b - a).max())}")
+                flipped = check_near_ties(rep, anc, idx, w_pre, pos, delta, kind, tag)
             rep.count(f"near-ties ({kind})", len(flipped))
             rep.worst("children of one parent", np.bincount(anc).max())
             rep.worst(f"children of one parent ({kind})", np.bincount(anc).max())
-            check_moments(rep, res, p, t, cov, tag, origin)
+            # the step-by-step flow sums the moments about particle 0 of the previous resampled particles (k_s4c_gather and
+            # k_s5_finalize read state_buffer(t - 1)); the pipelined flow about k_init's moment origin
+            check_moments(rep, res, p, t, cov, tag, prev[0] if method in STEP_METHODS else origin)
     return rep
 
 

@@ -3,7 +3,8 @@ k_s4p_resample_propagate -> k_s5p_finalize) replayed in float64 from the track's
 1 000 001 particles: 1 to 1 303 blocks per point, odd N, stratified resampling, carried, uniform, DEM-only and observed
 updates, a late-starting point, a failed point in a batch of active points, a call mixing cartesian, cylindrical and
 tangent points over three observers with its datetimes backwards, batches of points running concurrently on up to four side
-streams.  And the resampler at the
+streams.  The same for the step-by-step flow (k_s1_propagate -> k_s2_surface -> k_s3_weights -> k_s4c_scan or
+k_s4r_residual -> k_s4c_gather -> k_s5_finalize) that runs the choice and residual resamplers.  And the resampler at the
 edge uniforms 0, 2^-30, 1/2 and 1 - 2^-53, supplied as draws."""
 import numpy as np
 import pytest
@@ -41,8 +42,9 @@ def check_final_state(tracker, res):
     assert np.array_equal(tracker.weights, res["weights"][P - 1, last])
 
 
-@pytest.mark.parametrize("name", replay.CASES)
-def test_every_update_replays(cuda, monkeypatch, name):
+def track_and_replay(monkeypatch, name, method=None):
+    """Tracker.track of a replay case (``method``: another resampler) and the replay of every update; returns (report,
+    tracks)."""
     import glimpse_b200 as gb
     from glimpse_b200.session import point_span
 
@@ -51,7 +53,7 @@ def test_every_update_replays(cuda, monkeypatch, name):
     monkeypatch.setenv("GB_STREAM_BATCH", "2" if name == "mixed_three_obs" else "1")
     monkeypatch.setenv("GB_STREAM_SLOTS", "4")
     kept = record_sessions(monkeypatch)
-    scene, mask, method, cov = replay.case(name)
+    scene, mask, method, cov = replay.case(name, method=method)
     observers, models = replay.build(scene, gb)
     tracker = gb.Tracker(observers, seed=SEED, resample_method=method)
     tracks = tracker.track(models, datetimes=replay.datetimes(scene), tile_size=scene.tile_size, observer_mask=mask,
@@ -64,17 +66,35 @@ def test_every_update_replays(cuda, monkeypatch, name):
     P = len(models)
     draws = philox.device_draws(SEED, range(P), first, last, scene.n_particles, [m.tangent for m in inputs[1]], method)
     rep = replay.replay_track(res, draws, inputs, method, mask, scene.tile_size, cov=cov, windows=windows)
-    print(replay.summary(name, rep))
+    print(replay.summary(f"{name} ({method})", rep))
     check_final_state(tracker, res)
     assert rep["windows"] > 0
     if name.startswith("small_") or name == "mixed_three_obs":
         assert rep["failed points"] == 1 and tracks.errors[1] is not None
-    if name == "tan_carried_collapse":
-        assert rep["children of one parent (observed)"] > 3 * replay.CHUNK and rep["carried updates"] == 2
     if name == "mixed_three_obs":
         assert all(rep[f"{k} updates"] > 0 for k in replay.KINDS)
     if name == "cart_dem_floor":
         assert rep["dem updates"] == 4
+    return rep, tracks
+
+
+@pytest.mark.parametrize("name", replay.CASES)
+def test_every_update_replays(cuda, monkeypatch, name):
+    rep, _ = track_and_replay(monkeypatch, name)
+    if name == "tan_carried_collapse":
+        assert rep["children of one parent (observed)"] > 3 * replay.CHUNK and rep["carried updates"] == 2
+
+
+@pytest.mark.parametrize("name,method", replay.STEP_CASES)
+def test_every_step_flow_update_replays(cuda, monkeypatch, name, method):
+    """The step-by-step flow of gb_track (choice, residual) replayed: k_s1_propagate for every particle (the pipelined cases'
+    draws), k_s4c_scan's cumulative weights across up to 1 303 blocks, k_s4r_residual at up to 10^5 particles (every child
+    searched at small_99005's uniform updates), k_s4c_gather and k_s5_finalize combining the moment partials."""
+    rep, _ = track_and_replay(monkeypatch, name, method)
+    if name == "tan_carried_collapse":  # a parent with more than three blocks of children, drawn in any order
+        assert rep["children of one parent (observed)"] > 3 * replay.CHUNK and rep["carried updates"] == 2
+    if name == "small_99005":
+        assert rep["residual K = 0 (uniform)"] == rep["uniform updates"] > 0
 
 
 EDGE_U = [0.0, 1 - 2.0 ** -53, 2.0 ** -30, 0.5]

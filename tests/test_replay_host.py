@@ -44,9 +44,10 @@ def host_draws(specs, first, last, method, seed):
     return init, step, unif
 
 
-def oracle_track(name, n_particles=None, seed=7):
-    """(replay inputs, oracle result, draws) of a replay case run by the oracle with closed-form kernels."""
-    scene, mask, method, cov = replay.case(name, n_particles)
+def oracle_track(name, n_particles=None, seed=7, method=None):
+    """(replay inputs, oracle result, draws) of a replay case run by the oracle with closed-form kernels (``method``: another
+    resampler)."""
+    scene, mask, method, cov = replay.case(name, n_particles, method)
     inputs = replay.inputs(scene)
     obs, specs, taus, idx = inputs
     first, last = span(idx, mask)
@@ -242,4 +243,119 @@ def test_scenes_contain_what_the_gpu_test_claims():
     out, args, res = oracle_track("tan_carried_collapse", seed=("philox", replay.SEED))
     most = {s["t"]: int(np.bincount(np.asarray(s["indices"])).max()) for s in res.trace if "indices" in s}
     print("tan_carried_collapse: most children of one parent per time", most)
+    assert max(most.values()) > 3 * replay.CHUNK
+
+
+@pytest.mark.parametrize("name,n,method", [("tan_carried_collapse", 10000, "choice"), ("mixed_three_obs", None, "choice"),
+                                           ("tan_cyl_stratified_odd", 999, "residual"), ("cart_dem_floor", 2000, "residual"),
+                                           ("small_99005", 2000, "residual")])
+def test_replay_accepts_oracle_step_flow_tracks(name, n, method):
+    out, args, _ = oracle_track(name, n, method=method)
+    rep = replay.replay_track(out, **args)
+    print(replay.summary(f"{name} ({method})", rep))
+    for kind in replay.KINDS:
+        assert rep.get(f"near-ties ({kind})", 0) == 0
+        assert rep.get(f"propagation ({kind})", 0.0) == 0.0
+        assert rep.get(f"weight rel ({kind})", 0.0) == 0.0
+        assert rep.get(f"residual searches within the noise ({kind})", 0) == 0
+        assert rep.get(f"residual repetitions off floor(N wn) ({kind})", 0.0) == 0.0
+    if name == "mixed_three_obs":
+        assert rep["failed points"] == 1
+
+
+def step_update(steps, t):
+    s = steps[(0, t)]
+    return np.asarray(s["indices"]), s["evolved"], s["u"]
+
+
+def test_step_flow_mutations_are_rejected():
+    """Choice on the collapse case (N = 10 000, 14 blocks), residual on the odd tangent case (N = 999)."""
+    cases = {}
+    out, args, res = oracle_track("tan_carried_collapse", 10000, method="choice")
+    steps = {(s["p"], s["t"]): s for s in res.trace if "indices" in s}
+    carried, observed = carried_and_observed(args)
+    t_c, t_o = carried[0], observed[0]
+    anc, evolved, _ = step_update(steps, t_c)
+    i = 100
+    j = next(j for j in range(len(anc) - 1, 0, -1) if anc[j] != anc[i])
+
+    def swap(a):
+        a[0, t_c, [i, j]] = a[0, t_c, [j, i]]
+
+    N = len(anc)
+    B = replay.stream_block(N)  # the moment partials of the second block
+
+    def drop_block(m):
+        ps, w = out["particles"][0, t_o], out["weights"][0, t_o]
+        keep = np.ones(N, dtype=bool)
+        keep[B:2 * B] = False
+        m[0, t_o] = orc.weighted_mean(ps[keep], w[keep])
+
+    cases["choice: two children given each other's parents"] = (mutated(out, particles=swap, weights=swap), args)
+    cases["choice: one block's moments dropped"] = (mutated(out, means=drop_block), args)
+
+    out_r, args_r, res_r = oracle_track("tan_cyl_stratified_odd", 999, method="residual")
+    steps_r = {(s["p"], s["t"]): s for s in res_r.trace if "indices" in s}
+    carried_r, observed_r = carried_and_observed(args_r)
+    carried_r = [t for t in carried_r if t > observed_r[0]]  # carried weights of an observed update: uneven
+    anc, evolved, u = step_update(steps_r, carried_r[0])
+    K = len(anc) - len(u)
+    assert 0 < K < len(anc) - 1
+    run_end = next(k for k in range(1, K) if anc[k] != anc[k - 1])  # the first parent's repetitions end here
+
+    w_c = steps_r[(0, carried_r[0])]["weights"]
+
+    def shift(ps):  # the first parent gets one more repetition, the next one fewer
+        ps[0, carried_r[0], run_end] = evolved[anc[run_end - 1]]
+
+    def shift_w(ws):
+        ws[0, carried_r[0], run_end] = w_c[anc[run_end - 1]]
+
+    cases["residual: initial segment shifted by one child"] = (mutated(out_r, particles=shift, weights=shift_w), args_r)
+    # an additional child (at an observed update: the noisy path) moved to the next parent, its key far from that parent's and
+    # its neighbours' cumulative residuals
+    t_o = observed_r[0]
+    anc, evolved, u = step_update(steps_r, t_o)
+    N = len(anc)
+    K = N - len(u)
+    w = steps_r[(0, t_o)]["weights"]
+    wn = w / w.sum()
+    reps = np.bincount(anc[:K], minlength=N)
+    cs = np.cumsum((wn - reps) * (1 / (wn - reps).sum()))
+    far = [k for k in range(len(u)) if anc[K + k] + 1 < N
+           and np.abs(cs[max(anc[K + k] - 1, 0):anc[K + k] + 2] - u[k]).min() > 1e-3]
+    k = far[len(far) // 2]
+
+    def move(ps):
+        ps[0, t_o, K + k] = evolved[anc[K + k] + 1]
+
+    def move_w(ws):
+        ws[0, t_o, K + k] = w[anc[K + k] + 1]
+
+    cases["residual: an additional child moved to the next parent"] = (mutated(out_r, particles=move, weights=move_w), args_r)
+    for label, (bad, kw) in cases.items():
+        with pytest.raises(AssertionError) as info:
+            replay.replay_track(bad, **kw)
+        print(label, "->", str(info.value).splitlines()[0][:160])
+
+
+def test_step_scenes_contain_what_the_gpu_test_claims():
+    """The step-flow cases of tests/test_gpu_replay.py: small_99005's uniform updates leave the residual resampler no
+    repetitions (N (1 / N) < 1: every child searched), the choice collapse gives a parent more than three blocks of
+    children with the philox draws of the GPU test, and the cases keep the kinds of update of their pipelined versions."""
+    for name, method in replay.STEP_CASES:
+        scene, mask, m, cov = replay.case(name, method=method)
+        assert m == method
+        _, specs, taus, idx = replay.inputs(scene)
+        kinds = replay.update_kinds(specs, idx, mask)
+        counts = {k: sum(1 for v in kinds.values() if v == k) for k in replay.KINDS}
+        print(name, method, "N", scene.n_particles, "blocks", -(-scene.n_particles // replay.CHUNK), "updates", counts)
+        if name == "small_99005":
+            N = scene.n_particles
+            assert N * (1 / N) < 1 and counts["uniform"] > 0
+            assert len(orc.residual_indices(np.ones(N), np.random.random)[1]) == N  # K = 0
+    assert replay.case("million", method="choice")[0].n_particles == 1000001
+    out, args, res = oracle_track("tan_carried_collapse", seed=("philox", replay.SEED), method="choice")
+    most = {s["t"]: int(np.bincount(np.asarray(s["indices"])).max()) for s in res.trace if "indices" in s}
+    print("tan_carried_collapse (choice): most children of one parent per time", most)
     assert max(most.values()) > 3 * replay.CHUNK
